@@ -4,7 +4,7 @@
 Workload: Sentinel-3 OLCI-shaped swath (4865 x 4091 lon/lat float64, 21 float32 bands) rectified to
 a regular 0.0027 deg (~300 m) EPSG:4326 grid with nearest AND bilinear interpolation.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A *scene pass* is ONE ``rectify_dataset`` call that produces the 21 bands with both methods (the
 band stack enters the dataset under two variable names with ``interp_methods`` per variable): as in
@@ -69,7 +69,14 @@ def parse_args():
     ap.add_argument("--no-graph", action="store_true", help="take `value` from the eager, sequential region")
     ap.add_argument("--cpu-kind", default="auto", choices=["auto", "reference", "port"],
                     help="CPU baseline: the reference's own numba kernels (oracle/_ref) or the C restatement")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of the last step's outputs as DIR/<name>.npy "
+                         "(float32, every band at the same seeded target pixels; with N > 1 GPUs rank 0's row band) "
+                         "to compare two builds; --impl reference writes nothing and says so in its result line")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ---------------------------------------------------------------------------
@@ -324,6 +331,8 @@ def reference_arm(args):
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
+    if args.dump_outputs:  # the CPU arm times a sample of target tiles; it has no whole outputs to write
+        line["notes"] = ["--dump-outputs: nothing written; it writes the outputs of the GPU path (--impl ours)"]
     print(json.dumps(line), flush=True)
 
 
@@ -408,7 +417,7 @@ def ours(args):
         lat_p[...] = lat
         bands_p = _dev.pinned_empty(bands.shape, np.float32)
         bands_p[...] = bands
-        e2e_steps = max(1, min(args.steps, 10))
+        e2e_steps = args.steps
         interp = {"bands_nearest": "nearest", "bands_bilinear": "bilinear"}
         if world == 1:
             ds = xrs.Dataset(data_vars=dict(bands_nearest=(("band", "y", "x"), bands_p),
@@ -690,10 +699,19 @@ def ours(args):
     # ---- parity spot-check of the timed outputs against the oracle (rank 0) ----------------
     parity = None
     if rank == 0:
+        ij_ref = None
         try:
-            parity = spot_check(lon, lat, bands, size, xy_min, res, outs, rows, plans[0] if not args.fused else None)
+            ij_ref = oracle_ij(lon, lat, size, xy_min, res)
+            parity = spot_check(bands, ij_ref, outs, rows, plans[0] if not args.fused else None)
         except Exception as e:
             parity = {"error": f"{type(e).__name__}: {e}"}
+        if args.dump_outputs:
+            try:
+                if ij_ref is None:
+                    ij_ref = oracle_ij(lon, lat, size, xy_min, res)
+                dump_outputs(outs, args.dump_outputs, np.isfinite(ij_ref[0, rows[0]:rows[1]]))
+            except Exception as e:  # the result line below still goes out, saying so
+                notes.append(f"--dump-outputs failed ({type(e).__name__}: {e})")
 
     # ---- roofline of the dominant kernel (largest share of the timed region) ------------
     peaks = {}
@@ -865,17 +883,22 @@ def ours(args):
             killer.cancel()
 
 
-def spot_check(lon, lat, bands, size, xy_min, res, outs, rows, plan, strip=48):
-    """The timed region's own outputs against the oracle on a strip of target rows in the middle of
-    this rank's band: ij image (when the two-step path ran) and both gathers of all bands, bit for bit."""
+def oracle_ij(lon, lat, size, xy_min, res):
+    """The oracle's ij image of the whole target (C restatement on all host threads, ~1 s at full size)."""
     import oracle
     from oracle import grid as ogrid
     from oracle import rectify as orect
 
     oracle.build()
     oracle.lib().xrso_set_num_threads(host_threads())
-    g = ogrid.regular_grid(size, xy_min, res, tile_size=TILE)
-    ij = orect.rectify_ij(lon, lat, g)
+    return orect.rectify_ij(lon, lat, ogrid.regular_grid(size, xy_min, res, tile_size=TILE))
+
+
+def spot_check(bands, ij, outs, rows, plan, strip=48):
+    """The timed region's own outputs against the oracle (its ij image ``ij``) on a strip of target rows in the
+    middle of this rank's band: ij image (when the two-step path ran) and both gathers of all bands, bit for bit."""
+    from oracle import rectify as orect
+
     mid = (rows[0] + rows[1]) // 2
     a = max(rows[0], mid - strip // 2)
     b = min(rows[1], a + strip)
@@ -891,6 +914,45 @@ def spot_check(lon, lat, bands, size, xy_min, res, outs, rows, plan, strip=48):
         out[f"{m}_bit_exact"] = bool(np.array_equal(got, want, equal_nan=True))
         out[f"{m}_mismatch_fraction"] = float(np.mean(~((got == want) | (np.isnan(got) & np.isnan(want)))))
     return out
+
+
+DUMP_PIXELS = 1 << 18  # covered pixels per method: 21 bands x 2^18 x 4 B = 22 MB
+DUMP_FILL_PIXELS = 1 << 15  # uncovered pixels per method: 21 bands x 2^15 x 4 B = 2.8 MB
+
+
+def _seeded_sample(mask, n, seed):
+    """Flat indices of ``n`` pixels drawn with a seeded generator from those ``mask`` marks (all of them when
+    there are fewer), in raster order."""
+    idx = np.flatnonzero(mask)
+    if idx.size > n:
+        idx = np.sort(np.random.default_rng(seed).choice(idx, size=n, replace=False))
+    return idx
+
+
+def dump_outputs(outs, out_dir, covered, n_pixels=DUMP_PIXELS, n_fill=DUMP_FILL_PIXELS, seed=0):
+    """What the timed step hands back -- one (bands, rows, cols) float32 image per method with the NaN fill
+    where no source pixel lands -- as a fixed, finite sample.  ``covered`` is where the oracle finds a source
+    pixel; it depends on the inputs alone, never on the build that computed ``outs``.
+
+    * ``out_dir/bands_<method>.npy`` (bands, n): every band at ``n_pixels`` covered pixels, the values;
+    * ``out_dir/fill_<method>.npy`` (bands, n): every band at ``n_fill`` uncovered pixels, 1.0 where the output
+      holds the NaN fill and 0.0 where it holds anything else (a build that writes outside the swath).
+
+    Both sets are drawn with seeded generators and kept in raster order."""
+    import torch
+
+    covered = np.asarray(covered, dtype=bool)
+    idx = _seeded_sample(covered.ravel(), n_pixels, seed)
+    idx_fill = _seeded_sample(~covered.ravel(), n_fill, seed + 1)
+    os.makedirs(out_dir, exist_ok=True)
+    for m, img in outs.items():
+        nb, h, w = img.shape
+        assert covered.shape == (h, w), f"coverage {covered.shape} does not match the output {(h, w)}"
+        flat = img.reshape(nb, h * w)
+        sample = flat[:, torch.from_numpy(idx).to(img.device)]
+        np.save(os.path.join(out_dir, f"bands_{m}.npy"), sample.cpu().numpy())
+        is_fill = torch.isnan(flat[:, torch.from_numpy(idx_fill).to(img.device)])
+        np.save(os.path.join(out_dir, f"fill_{m}.npy"), is_fill.to(torch.float32).cpu().numpy())
 
 
 def main():

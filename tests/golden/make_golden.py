@@ -1,6 +1,7 @@
 """Generate tests/golden/*.npz by running the REFERENCE's own kernels.
 
-Runs only in the build container, where ``/root/reference`` exists: the
+Runs only where the reference package is installed (the directories of
+``oracle/refkernels.py``'s ``REF_DIRS``, ``oracle/_ref`` first): the
 reference's numba / numpy kernels are imported from there (third-party packages
 that are not installed -- dask, xarray, pyproj, affine, zarr, dask_image -- are
 replaced by inert stub modules, numba JIT stays on) and executed on small seeded
@@ -23,7 +24,7 @@ sys.dont_write_bytecode = True
 import numpy as np  # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = "/root/reference"
+ROOT = os.path.dirname(os.path.dirname(HERE))
 
 
 class _Any:
@@ -58,6 +59,18 @@ class _Stub(types.ModuleType):
         return _Any()
 
 
+def reference_dir():
+    """The first directory of ``oracle.refkernels.REF_DIRS`` that holds the reference package."""
+    if ROOT not in sys.path:
+        sys.path.insert(0, ROOT)
+    from oracle.refkernels import REF_DIRS
+
+    where = next((d for d in REF_DIRS if os.path.isdir(os.path.join(d, "xcube_resampling"))), None)
+    if where is None:
+        raise SystemExit(f"the reference package (xcube_resampling) is in none of {list(REF_DIRS)}")
+    return where
+
+
 def install_reference():
     for name in ["dask", "dask.array", "dask.array.core", "xarray", "pyproj", "pyproj.crs", "pyproj.transformer",
                  "dask_image", "dask_image.ndinterp", "affine", "zarr", "zarr.convenience"]:
@@ -65,8 +78,9 @@ def install_reference():
             m = _Stub(name)
             m.__path__ = []
             sys.modules[name] = m
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
+    where = reference_dir()
+    if where not in sys.path:
+        sys.path.insert(0, where)
 
 
 # ---------------------------------------------------------------------------
@@ -245,9 +259,25 @@ def make_ij_bboxes(B):
     print("ij_bboxes.npz:", k, "cases")
 
 
+def make_dual_swath():
+    """Digests of the reference's three gathers, tile by tile, of the swath tests/test_oracle_dual.py holds
+    the two-method gather against (too large to commit as arrays)."""
+    import json
+
+    from oracle import refkernels
+    from tests.helpers import digest, dual_swath
+
+    x, y, g, data = dual_swath()
+    methods = ("nearest", "bilinear", "triangular")
+    _, ref = refkernels.rectify_pass(x, y, data, g, methods, n_threads=4, keep_outputs=True)
+    out = {m: digest(ref[m]) for m in methods}
+    out["source"] = "the reference's own kernels (tests/golden/make_golden.py)"
+    with open(os.path.join(HERE, "dual_swath_digests.json"), "w") as fh:
+        json.dump(out, fh, indent=0, sort_keys=True)
+    print("dual_swath_digests.json")
+
+
 def main():
-    if not os.path.isdir(REF):
-        raise SystemExit("make_golden.py needs /root/reference (build container only)")
     install_reference()
     import xcube_resampling.gridmapping.bboxes as B
     import xcube_resampling.rectify as R
@@ -255,6 +285,7 @@ def main():
     make_rectify(R, B)
     make_rectify_f32_coords(R, B)
     make_ij_bboxes(B)
+    make_dual_swath()
     try:
         from make_golden_resample import make_all as make_resample  # added with the affine/coarsen/reproject paths
     except ImportError:

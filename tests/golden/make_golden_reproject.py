@@ -1,6 +1,6 @@
 """Generate tests/golden/reproject.npz by running the REFERENCE's ``_reproject_block``.
 
-Build container only (needs ``/root/reference``); see make_golden.py for the stub recipe.
+Needs the reference package where make_golden.py's ``reference_dir`` finds it; see make_golden.py for the stub recipe.
 Inputs are seeded source-CRS coordinates of the target pixels of one tile plus a source window;
 outputs are what ``xcube_resampling.reproject._reproject_block`` (reproject.py:268-335) returns,
 for every interpolation method and a spread of dtypes.

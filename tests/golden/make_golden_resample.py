@@ -1,5 +1,5 @@
 """Coarsen goldens: the reference's own reducers (xcube_resampling/coarsen.py, imported from
-/root/reference by make_golden.py's stub recipe) on seeded windows.  Run through make_golden.py."""
+where make_golden.py's ``reference_dir`` finds it, with its stub recipe) on seeded windows.  Run through make_golden.py."""
 
 import os
 

@@ -1,5 +1,6 @@
 """Shared test helpers: golden loading, synthetic swaths, oracle grids."""
 
+import hashlib
 import os
 
 import numpy as np
@@ -32,6 +33,29 @@ def assert_same(a, b, what=""):
         idx = np.argwhere(bad)[:5]
         raise AssertionError(f"{what}: {bad.sum()} of {a.size} elements differ, first at {idx.tolist()}: "
                              f"{a[bad][:5]} vs {b[bad][:5]}")
+
+
+def digest(a) -> str:
+    """64-bit SHA-256 prefix of dtype, shape and values; every NaN hashes as one NaN and -0.0 as 0.0, so
+    equal digests stand for ``assert_same``: equal dtypes, shapes and ``np.array_equal(..., equal_nan=True)``."""
+    a = np.ascontiguousarray(a)
+    if a.dtype.kind == "f":
+        a = np.where(np.isnan(a), np.nan, a + 0).astype(a.dtype, copy=False)
+    h = hashlib.sha256(f"{a.dtype.str}{a.shape}".encode())
+    h.update(a.tobytes())
+    return h.hexdigest()[:16]
+
+
+def dual_swath():
+    """(x, y, grid, bands) on which tests/test_oracle_dual.py holds the two-method gather against the
+    reference's kernels (tests/golden/dual_swath_digests.json, written by make_golden.py)."""
+    x, y = swath(220, 180, theta=20.0, seed=5)
+    res = 0.0027
+    size, xy_min = covering_grid_args(x, y, res)
+    g = ogrid.regular_grid(size, xy_min, res, tile_size=64)
+    data = np.random.default_rng(5).random((3, 180, 220)).astype(np.float32)
+    data[1, 60:70, 80:120] = np.nan
+    return x, y, g, data
 
 
 INT32_MAX = np.iinfo(np.int32).max

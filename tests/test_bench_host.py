@@ -48,6 +48,52 @@ def test_reference_arm_only_rank_zero_works():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_argument_checks(tmp_path):
+    r = _run(["--steps", "0"])
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr
+    # the CPU arm has no whole outputs: nothing written, and its result line says so
+    r = _run(["--impl", "reference", "--scale", "0.05", "--steps", "1", "--warmup", "0", "--cpu-kind", "port",
+              "--dump-outputs", str(tmp_path / "dump")])
+    assert r.returncode == 0, r.stderr
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert "--dump-outputs: nothing written" in line["notes"][0] and not (tmp_path / "dump").exists()
+
+
+def test_dump_outputs_is_a_fixed_sample_of_every_band(tmp_path):
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    j, i = np.mgrid[:40, :50]
+    covered = np.abs(i - 25 - 0.4 * (j - 20)) < 15  # a slanted swath; the NaN fill outside it
+    imgs = {}
+    for k, m in enumerate(bench.METHODS):
+        img = torch.rand((3, 40, 50), generator=torch.Generator().manual_seed(k))
+        img[:, torch.from_numpy(~covered)] = float("nan")
+        imgs[m] = img
+    bench.dump_outputs(imgs, str(tmp_path / "a"), covered, n_pixels=300, n_fill=100)
+    bench.dump_outputs({m: img.clone() for m, img in imgs.items()}, str(tmp_path / "b"), covered, n_pixels=300,
+                       n_fill=100)
+    for m, img in imgs.items():
+        a, b = np.load(tmp_path / "a" / f"bands_{m}.npy"), np.load(tmp_path / "b" / f"bands_{m}.npy")
+        assert a.dtype == np.float32 and a.shape == (3, 300) and np.array_equal(a, b) and np.isfinite(a).all()
+        flat = img.numpy().reshape(3, -1)
+        cols = [int(np.flatnonzero(flat[0] == v)[0]) for v in a[0]]  # the sampled pixels, in raster order
+        assert cols == sorted(set(cols)) and covered.ravel()[cols].all() and np.array_equal(a, flat[:, cols])
+        fa, fb = np.load(tmp_path / "a" / f"fill_{m}.npy"), np.load(tmp_path / "b" / f"fill_{m}.npy")
+        assert fa.dtype == np.float32 and fa.shape == (3, 100) and np.array_equal(fa, fb) and (fa == 1.0).all()
+    # a build that writes values outside the swath, where the NaN fill belongs, shows in the fill sample
+    wrong = {m: torch.nan_to_num(img, nan=0.5) for m, img in imgs.items()}
+    bench.dump_outputs(wrong, str(tmp_path / "w"), covered, n_pixels=300, n_fill=100)
+    assert np.array_equal(np.load(tmp_path / "w" / "bands_nearest.npy"), np.load(tmp_path / "a" / "bands_nearest.npy"))
+    assert (np.load(tmp_path / "w" / "fill_nearest.npy") == 0.0).all()
+    bench.dump_outputs(imgs, str(tmp_path / "c"), covered, n_pixels=10 ** 6)  # fewer covered pixels: all of them
+    want = imgs["nearest"].numpy().reshape(3, -1)[:, covered.ravel()]
+    assert np.array_equal(np.load(tmp_path / "c" / "bands_nearest.npy"), want)
+
+
 def test_helpers_without_nvml():
     sys.path.insert(0, ROOT)
     import bench

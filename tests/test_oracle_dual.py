@@ -1,8 +1,11 @@
 """CPU pin of the two-method gather's algorithm (``k2_gather_dual`` / ``xrs_gather_ij2``): "the
 nearest-neighbour sample is one of the four taps of the bilinear / triangular one" is checked, without a
 GPU, against the oracle's ``_compute_var_image`` restatement and against the REFERENCE's own numba kernel
-(``rectify.py:640-734`` through ``oracle/refkernels.py``).  The GPU tests then only have to show that the
-CUDA kernel equals the oracle."""
+(``rectify.py:640-734``: through ``oracle/refkernels.py`` where it is installed, its golden outputs, stored
+digests).  The GPU tests then only have to show that the CUDA kernel equals the oracle."""
+
+import json
+import os
 
 import numpy as np
 import pytest
@@ -10,7 +13,8 @@ import pytest
 from oracle import grid as ogrid
 from oracle import rectify as orect
 
-from .helpers import assert_same, covering_grid_args, hand_made_ij, swath, two_method_gather_np
+from .helpers import (GOLDEN, assert_same, covering_grid_args, digest, dual_swath, hand_made_ij, swath,
+                      two_method_gather_np)
 
 nan = np.nan
 
@@ -53,26 +57,31 @@ def test_picked_tap_equals_oracle_on_swaths(theta, seed):
 
 def test_picked_tap_equals_the_reference_kernels():
     """The same against the reference's own ``_compute_var_image_sequential`` (tile by tile, as the
-    reference runs it), when the reference package and numba are available."""
+    reference runs it): against its outputs where the reference package and numba load (whose digests must
+    then equal the stored ones), and everywhere against tests/golden/dual_swath_digests.json (its ``source``
+    says what produced it)."""
     from oracle import refkernels
 
+    x, y, g, data = dual_swath()
+    with open(os.path.join(GOLDEN, "dual_swath_digests.json")) as fh:
+        stored = json.load(fh)
     try:
         refkernels.load()
-    except ImportError as e:
-        pytest.skip(f"reference kernels not available: {e}")
-    x, y = swath(220, 180, theta=20.0, seed=5)
-    res = 0.0027
-    size, xy_min = covering_grid_args(x, y, res)
-    g = ogrid.regular_grid(size, xy_min, res, tile_size=64)
-    data = np.random.default_rng(5).random((3, 180, 220)).astype(np.float32)
-    data[1, 60:70, 80:120] = nan
-    methods = ("nearest", "bilinear", "triangular")
-    _, ref = refkernels.rectify_pass(x, y, data, g, methods, n_threads=4, keep_outputs=True)
+    except ImportError:
+        ref = None
+    else:
+        _, ref = refkernels.rectify_pass(x, y, data, g, ("nearest", "bilinear", "triangular"), n_threads=4,
+                                         keep_outputs=True)
+        assert {m: digest(out) for m, out in ref.items()} == {m: stored[m] for m in ref}, "stored digests"
     ij = orect.rectify_ij(x, y, g)
     for method in ("bilinear", "triangular"):
         interp, near, valid = two_method_gather_np(data, ij, method)
-        assert_same(_apply_fill(interp, valid, nan), ref[method], f"{method} vs reference kernel")
-        assert_same(_apply_fill(near, valid, nan), ref["nearest"], "nearest vs reference kernel")
+        interp, near = _apply_fill(interp, valid, nan), _apply_fill(near, valid, nan)
+        if ref is not None:
+            assert_same(interp, ref[method], f"{method} vs reference kernel")
+            assert_same(near, ref["nearest"], "nearest vs reference kernel")
+        assert digest(interp) == stored[method], f"{method} vs stored digest"
+        assert digest(near) == stored["nearest"], "nearest vs stored digest"
     assert valid.mean() > 0.3
 
 
