@@ -297,7 +297,11 @@ int xrs_reproject(const void *const *src_planes_host, void *const *dst_planes_ho
  *   order      0 nearest, 1 linear; anything else fails like affine.py:329-335
  *   agg, f_j, f_i  reducer (enum xrs_agg) over f_j x f_i intermediate samples; f_j = f_i = 1: none
  *   slice_blend  1 reproduces scipy's zero-weight read of the neighbouring slice for 3-D float
- *              arrays with order 1 (non-finite values there make the sample NaN)  */
+ *              arrays with order 1 (non-finite values there make the sample NaN; one slice reads itself)
+ * Every sample takes scipy's float64 round trip, order 0 included: int64 values beyond 2^53 come back
+ * rounded as scipy rounds them (2^52 + 1 -> 2^52 + 2, 2^62 + 1 -> 2^62), -0.0 as +0.0; NaN / out-of-range
+ * results and cval in integer outputs convert as scipy's do on x86 (NaN -> INT32_MIN / INT64_MIN for 32- and
+ * 64-bit signed types, 0 for the others; 2^63 -> INT64_MIN, above -> INT64_MAX).  */
 int xrs_affine(const void *src, void *dst, int32_t dtype, int64_t n_slices, int64_t src_h, int64_t src_w,
                int64_t src_pitch, int64_t src_slice_stride, int64_t dst_h, int64_t dst_w, double j_scale, double j_off,
                double i_scale, double i_off, int32_t order, double cval, int32_t agg, int32_t f_j, int32_t f_i,
@@ -317,7 +321,8 @@ int xrs_affine_recover(const void *src, double *dst, int32_t dtype, int64_t n_sl
                        int32_t slice_blend, void *stream);
 
 /* K5 alone -- dask.array.coarsen(agg, array, {y: f_j, x: f_i}) with the same reducers
- * (coarsen.py:50-155); f_j, f_i must divide src_h, src_w.  dst as for xrs_affine. */
+ * (coarsen.py:50-155); f_j, f_i must divide src_h, src_w.  dst as for xrs_affine.  Unlike xrs_affine the
+ * values are aggregated as stored (dask never converts them): int64 beyond 2^53 stays exact, -0.0 stays -0.0. */
 int xrs_coarsen(const void *src, void *dst, int32_t dtype, int64_t n_slices, int64_t src_h, int64_t src_w,
                 int64_t src_pitch, int64_t src_slice_stride, int32_t agg, int32_t f_j, int32_t f_i, void *stream);
 

@@ -35,6 +35,25 @@ def assert_same(a, b, what=""):
                              f"{a[bad][:5]} vs {b[bad][:5]}")
 
 
+def assert_bits(a, b, what="", skip=None):
+    """Equal dtypes, shapes and bit patterns, every NaN taken as one NaN: unlike ``assert_same`` the sign of zero
+    counts.  ``skip``: boolean mask of elements left out (only for documented deviations)."""
+    a, b = np.asarray(a), np.asarray(b)
+    assert a.shape == b.shape, f"{what}: shape {a.shape} != {b.shape}"
+    assert a.dtype == b.dtype, f"{what}: dtype {a.dtype} != {b.dtype}"
+    ua, ub = (np.ascontiguousarray(x).view(f"u{a.dtype.itemsize}") for x in (a, b))
+    if a.dtype.kind == "f":
+        canon = np.array([np.nan], dtype=a.dtype).view(ua.dtype)[0]
+        ua, ub = np.where(np.isnan(a), canon, ua), np.where(np.isnan(b), canon, ub)
+    bad = ua != ub
+    if skip is not None:
+        bad &= ~np.asarray(skip, dtype=bool)
+    if bad.any():
+        idx = np.argwhere(bad)[:5]
+        raise AssertionError(f"{what}: {bad.sum()} of {a.size} elements differ, first at {idx.tolist()}: "
+                             f"{a[bad][:5]} vs {b[bad][:5]}")
+
+
 def digest(a) -> str:
     """64-bit SHA-256 prefix of dtype, shape and values; every NaN hashes as one NaN and -0.0 as 0.0, so
     equal digests stand for ``assert_same``: equal dtypes, shapes and ``np.array_equal(..., equal_nan=True)``."""

@@ -419,12 +419,19 @@ static void window_sums(const A *win, int f_j, int f_i, long n, A *out) {
 }
 extern "C" void xrsh_window_sums_f32(const float *win, int f_j, int f_i, long n, float *out) { window_sums<float>(win, f_j, f_i, n, out); }
 extern "C" void xrsh_window_sums_f64(const double *win, int f_j, int f_i, long n, double *out) { window_sums<double>(win, f_j, f_i, n, out); }
-extern "C" void xrsh_scipy_cast(const double *v, long n, uint8_t *u8, int16_t *i16, int32_t *i32, uint16_t *u16) {
+// out: 9 rows of n values, in the order float32, float64, uint8, int8, uint16, int16, int32, uint32, int64
+extern "C" void xrsh_scipy_cast(const double *v, long n, void *out) {
+    char *o = static_cast<char *>(out);
     for (long k = 0; k < n; ++k) {
-        u8[k] = xrs::scipy_cast<uint8_t>(v[k]);
-        i16[k] = xrs::scipy_cast<int16_t>(v[k]);
-        i32[k] = xrs::scipy_cast<int32_t>(v[k]);
-        u16[k] = xrs::scipy_cast<uint16_t>(v[k]);
+        reinterpret_cast<float *>(o)[k] = xrs::scipy_cast<float>(v[k]);
+        reinterpret_cast<double *>(o + 4 * n)[k] = xrs::scipy_cast<double>(v[k]);
+        reinterpret_cast<uint8_t *>(o + 12 * n)[k] = xrs::scipy_cast<uint8_t>(v[k]);
+        reinterpret_cast<int8_t *>(o + 13 * n)[k] = xrs::scipy_cast<int8_t>(v[k]);
+        reinterpret_cast<uint16_t *>(o + 14 * n)[k] = xrs::scipy_cast<uint16_t>(v[k]);
+        reinterpret_cast<int16_t *>(o + 16 * n)[k] = xrs::scipy_cast<int16_t>(v[k]);
+        reinterpret_cast<int32_t *>(o + 18 * n)[k] = xrs::scipy_cast<int32_t>(v[k]);
+        reinterpret_cast<uint32_t *>(o + 22 * n)[k] = xrs::scipy_cast<uint32_t>(v[k]);
+        reinterpret_cast<int64_t *>(o + 26 * n)[k] = xrs::scipy_cast<int64_t>(v[k]);
     }
 }
 extern "C" void xrsh_axis_order1(const double *c, long n, long len, long *k0, long *k1, double *w0, double *w1,
@@ -2056,3 +2063,354 @@ def k3_reproject(so_path: str, src, src_gm, tgt_gm, windows, method: str, fill, 
     if rc != 0:
         raise RuntimeError(f"xrsh_reproject failed ({rc})")
     return out, (int(stats[0]), bool(stats[1]), bool(stats[2]))
+
+
+# ---------------------------------------------------------------------------
+# K4 / K5 as kernels (csrc/resample.cu + csrc/resample_fast.cu, launch code and C ABI included)
+# ---------------------------------------------------------------------------
+# Both files are compiled unchanged apart from one rewrite: every `NAME<<<grid, block, shm, st>>>(args)` becomes
+# `xrsh_launch(grid, block, shm, st, &NAME, args)`.  The launcher runs the grid on 32 host threads, one per lane:
+# each walks every (block, warp) in the same order, with threadIdx / blockIdx thread-local, so the lanes of a warp
+# meet __any_sync together (exchanged through a shared array between two barrier waits).  These kernels have no
+# shared memory and no block barriers.  The rest of the shim:
+#   * XRS_TIMED records the kernel name (the list `xrsh_take_log` returns), so tests see which kernel ran;
+#   * __ldcs / __ldg count every load whose address is not aligned to the loaded type (uint4: 16, uint2: 8, else
+#     its size) -- x86 forgives what faults on the GPU, so this count is how the dispatch rules are checked;
+#   * the SIMD-in-a-word intrinsics are written per lane from the CUDA Math API definitions (xrsh_simd exports
+#     them for their own test).
+RSK_SHIM = r"""
+#define _GNU_SOURCE 1
+#include <pthread.h>
+#include <algorithm>
+#include <cassert>
+#include <climits>
+#include <cmath>
+#include <cstdint>
+#include <cstring>
+#include <limits>
+#include <math.h>
+#include <string>
+#include <thread>
+#include <tuple>
+#include <type_traits>
+#include <vector>
+#include "xrs.h"
+#define __device__
+#define __host__
+#define __global__
+#define __forceinline__ inline
+#define __launch_bounds__(...)
+typedef void *cudaStream_t;
+using std::isfinite; using std::floor; using std::fabs; using std::sqrt; using std::rint; using std::fmin; using std::fmax;
+struct dim3 {
+    unsigned x, y, z;
+    dim3(unsigned x_ = 1, unsigned y_ = 1, unsigned z_ = 1) : x(x_), y(y_), z(z_) {}
+};
+static thread_local dim3 threadIdx, blockIdx, blockDim, gridDim;
+struct uint4 { unsigned x, y, z, w; };
+struct uint2 { unsigned x, y; };
+template <typename T> struct xrsh_align { static constexpr uintptr_t value = sizeof(T); };
+template <> struct xrsh_align<uint4> { static constexpr uintptr_t value = 16; };
+template <> struct xrsh_align<uint2> { static constexpr uintptr_t value = 8; };
+static long xrsh_misaligned = 0;
+static std::vector<std::string> xrsh_log;
+static std::string xrsh_error;
+template <typename T> static inline T xrsh_load(const T *p) {
+    if (reinterpret_cast<uintptr_t>(p) % xrsh_align<T>::value) __atomic_fetch_add(&xrsh_misaligned, 1, __ATOMIC_RELAXED);
+    T v;
+    std::memcpy(&v, p, sizeof(T));
+    return v;
+}
+template <typename T> static inline T __ldg(const T *p) { return xrsh_load(p); }
+template <typename T> static inline T __ldcs(const T *p) { return xrsh_load(p); }
+static inline int atomicOr(int *p, int v) { return __atomic_fetch_or(p, v, __ATOMIC_RELAXED); }
+static inline int cudaMemsetAsync(void *p, int v, size_t n, cudaStream_t) { std::memset(p, v, n); return 0; }
+// one warp = 32 host threads in lock step at its collectives
+static pthread_barrier_t xrsh_warp_bar;
+static int xrsh_warp_vote[32];
+static thread_local int xrsh_lane = 0;
+static inline bool __any_sync(unsigned, bool p) {
+    xrsh_warp_vote[xrsh_lane] = p ? 1 : 0;
+    pthread_barrier_wait(&xrsh_warp_bar);
+    bool any = false;
+    for (int k = 0; k < 32; ++k) any = any || xrsh_warp_vote[k] != 0;
+    pthread_barrier_wait(&xrsh_warp_bar);
+    return any;
+}
+// SIMD-in-a-word intrinsics (CUDA Math API, integer intrinsics / SIMD intrinsics), lane by lane
+static inline uint32_t xrsh_lane_of(uint32_t v, int bits, int k) { return (v >> (bits * k)) & ((1u << bits) - 1u); }
+template <typename Op> static inline uint32_t xrsh_per_lane(uint32_t a, uint32_t b, int bits, Op op) {
+    uint32_t r = 0;
+    for (int k = 0; k < 32 / bits; ++k)
+        r |= (op(xrsh_lane_of(a, bits, k), xrsh_lane_of(b, bits, k)) & ((1u << bits) - 1u)) << (bits * k);
+    return r;
+}
+static inline uint32_t __byte_perm(uint32_t x, uint32_t y, uint32_t s) {
+    const uint64_t v = (static_cast<uint64_t>(y) << 32) | x;
+    uint32_t r = 0;
+    for (int k = 0; k < 4; ++k) {
+        const uint32_t sel = (s >> (4 * k)) & 0xfu;
+        assert((sel & 8u) == 0 && "__byte_perm: only the default mode is emulated");
+        r |= static_cast<uint32_t>((v >> (8 * sel)) & 0xffu) << (8 * k);
+    }
+    return r;
+}
+static inline uint32_t __vminu4(uint32_t a, uint32_t b) { return xrsh_per_lane(a, b, 8, [](uint32_t x, uint32_t y) { return x < y ? x : y; }); }
+static inline uint32_t __vmaxu4(uint32_t a, uint32_t b) { return xrsh_per_lane(a, b, 8, [](uint32_t x, uint32_t y) { return x > y ? x : y; }); }
+static inline uint32_t __vminu2(uint32_t a, uint32_t b) { return xrsh_per_lane(a, b, 16, [](uint32_t x, uint32_t y) { return x < y ? x : y; }); }
+static inline uint32_t __vmaxu2(uint32_t a, uint32_t b) { return xrsh_per_lane(a, b, 16, [](uint32_t x, uint32_t y) { return x > y ? x : y; }); }
+static inline uint32_t __vhaddu4(uint32_t a, uint32_t b) { return xrsh_per_lane(a, b, 8, [](uint32_t x, uint32_t y) { return (x + y) >> 1; }); }
+static inline uint32_t __vadd4(uint32_t a, uint32_t b) { return xrsh_per_lane(a, b, 8, [](uint32_t x, uint32_t y) { return x + y; }); }
+static inline uint32_t __vcmpeq4(uint32_t a, uint32_t b) { return xrsh_per_lane(a, b, 8, [](uint32_t x, uint32_t y) { return x == y ? 0xffu : 0u; }); }
+static inline uint32_t __vcmpne4(uint32_t a, uint32_t b) { return xrsh_per_lane(a, b, 8, [](uint32_t x, uint32_t y) { return x != y ? 0xffu : 0u; }); }
+static inline uint32_t __vcmpgtu4(uint32_t a, uint32_t b) { return xrsh_per_lane(a, b, 8, [](uint32_t x, uint32_t y) { return x > y ? 0xffu : 0u; }); }
+static inline uint32_t __dp4a(uint32_t a, uint32_t b, uint32_t c) {
+    for (int k = 0; k < 4; ++k) c += xrsh_lane_of(a, 8, k) * xrsh_lane_of(b, 8, k);
+    return c;
+}
+namespace xrs {
+static inline int fail(const std::string &msg) { xrsh_error = msg; return 1; }
+static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
+static inline double dadd(double a, double b) { return a + b; }
+static inline double dsub(double a, double b) { return a - b; }
+static inline double dmul(double a, double b) { return a * b; }
+static inline double ddiv(double a, double b) { return a / b; }
+}
+#define XRS_CUDA(expr) do { int _rc = (expr); if (_rc) return _rc; } while (0)
+#define XRS_LAUNCH_CHECK(name) do { } while (0)
+#define XRS_TIMED(name, st, ...) do { xrsh_log.push_back(name); __VA_ARGS__; } while (0)
+template <typename... P, typename... A>
+static void xrsh_launch(dim3 grid, dim3 block, size_t, cudaStream_t, void (*kernel)(P...), A... args) {
+    const std::tuple<P...> params(args...);
+    const unsigned threads = block.x * block.y * block.z;
+    assert(threads % 32 == 0);
+    pthread_barrier_init(&xrsh_warp_bar, nullptr, 32);
+    std::vector<std::thread> lanes;
+    for (int lane = 0; lane < 32; ++lane)
+        lanes.emplace_back([&, lane] {
+            xrsh_lane = lane;
+            gridDim = grid;
+            blockDim = block;
+            for (unsigned bz = 0; bz < grid.z; ++bz)
+                for (unsigned by = 0; by < grid.y; ++by)
+                    for (unsigned bx = 0; bx < grid.x; ++bx)
+                        for (unsigned t = static_cast<unsigned>(lane); t < threads; t += 32) {
+                            blockIdx = dim3(bx, by, bz);
+                            threadIdx = dim3(t % block.x, (t / block.x) % block.y, t / (block.x * block.y));
+                            std::apply(kernel, params);
+                        }
+        });
+    for (auto &l : lanes) l.join();
+    pthread_barrier_destroy(&xrsh_warp_bar);
+}
+"""
+
+RSK_EXPORT = r"""
+// k5_u8x4_reduce launched directly, as launch_affine_fast would for F = 2 / 4 / 8: its median / mode branches are
+// kept for layouts k5_u8x2_sort declines, which the present dispatch never produces
+extern "C" int xrsh_u8x4(const uint8_t *src, void *dst, int f, long n, long h, long w, long pitch, long sstride, int agg) {
+    xrs::FastGeom g = {};
+    g.n_slices = n; g.src_h = h; g.src_w = w; g.src_pitch = pitch; g.src_slice_stride = sstride;
+    g.dst_h = h / f; g.dst_w = w / f; g.agg = agg; g.vec = 1;
+    switch (f) {
+    case 2: return xrs::launch_u8x4<2>(src, dst, g, nullptr);
+    case 4: return xrs::launch_u8x4<4>(src, dst, g, nullptr);
+    case 8: return xrs::launch_u8x4<8>(src, dst, g, nullptr);
+    }
+    return 1;
+}
+// kernel names launched since the last call (';'-separated), misaligned loads, last error message; resets all three
+extern "C" long xrsh_take_log(char *names, long cap, char *err, long err_cap) {
+    std::string s;
+    for (const auto &n : xrsh_log) s += (s.empty() ? "" : ";") + n;
+    std::snprintf(names, static_cast<size_t>(cap), "%s", s.c_str());
+    std::snprintf(err, static_cast<size_t>(err_cap), "%s", xrsh_error.c_str());
+    const long m = xrsh_misaligned;
+    xrsh_log.clear(); xrsh_error.clear(); xrsh_misaligned = 0;
+    return m;
+}
+// the SIMD intrinsics on word arrays: op 0 byte_perm(a, b, c), 1 vminu4, 2 vmaxu4, 3 vminu2, 4 vmaxu2, 5 vhaddu4,
+// 6 vadd4, 7 vcmpeq4, 8 vcmpne4, 9 vcmpgtu4, 10 dp4a(a, b, c)
+extern "C" int xrsh_simd(int op, const uint32_t *a, const uint32_t *b, const uint32_t *c, uint32_t *out, long n) {
+    for (long k = 0; k < n; ++k) {
+        switch (op) {
+        case 0: out[k] = __byte_perm(a[k], b[k], c[k]); break;
+        case 1: out[k] = __vminu4(a[k], b[k]); break;
+        case 2: out[k] = __vmaxu4(a[k], b[k]); break;
+        case 3: out[k] = __vminu2(a[k], b[k]); break;
+        case 4: out[k] = __vmaxu2(a[k], b[k]); break;
+        case 5: out[k] = __vhaddu4(a[k], b[k]); break;
+        case 6: out[k] = __vadd4(a[k], b[k]); break;
+        case 7: out[k] = __vcmpeq4(a[k], b[k]); break;
+        case 8: out[k] = __vcmpne4(a[k], b[k]); break;
+        case 9: out[k] = __vcmpgtu4(a[k], b[k]); break;
+        case 10: out[k] = __dp4a(a[k], b[k], c[k]); break;
+        default: return 1;
+        }
+    }
+    return 0;
+}
+"""
+
+SIMD_OPS = ("byte_perm", "vminu4", "vmaxu4", "vminu2", "vmaxu2", "vhaddu4", "vadd4", "vcmpeq4", "vcmpne4", "vcmpgtu4",
+            "dp4a")
+
+
+def _without_include(text: str, inc: str, what: str) -> str:
+    text, n = re.subn(r"#include " + re.escape(inc) + r"\n", "", text)
+    assert n == 1, f"{what} no longer includes {inc} exactly once"
+    return text
+
+
+def build_resample_kernels(out_dir: str) -> str:
+    """Host build of resample_common.cuh + resample_fast.cu + resample.cu, kernels, launch code and the C ABI
+    functions xrs_affine / xrs_coarsen / xrs_affine_recover / xrs_has_nan."""
+    gxx = shutil.which("g++")
+    if gxx is None:
+        raise RuntimeError("g++ not available")
+    common = _without_include(open(os.path.join(CSRC, "common.cuh")).read(), '"xrs.h"', "common.cuh")
+    m = re.search(r"#define XRS_DISPATCH_DTYPE\(.*?\n    }\n", common, re.S)
+    assert m, "XRS_DISPATCH_DTYPE moved"
+    dispatch = m.group(0)
+    rc = _without_include(open(os.path.join(CSRC, "resample_common.cuh")).read(), '"common.cuh"', "resample_common.cuh")
+    rc = rc.replace("#pragma once\n", "")
+    units = []
+    for name in ("resample_fast.cu", "resample.cu"):
+        text = _without_include(open(os.path.join(CSRC, name)).read(), '"resample_common.cuh"', name)
+        text, n = re.subn(r"([A-Za-z_]\w*(?:<[^<>;()]*>)?)<<<([^<>;]*?)>>>\(\s*", r"xrsh_launch(\2, &\1, ", text)
+        assert n > 0 and "<<<" not in text, f"launch syntax of {name} changed"
+        units.append(text)
+    src = os.path.join(out_dir, "resample_kernels_host.cpp")
+    with open(src, "w") as fh:
+        fh.write(RSK_SHIM + dispatch + "\n" + rc + "".join(units) + RSK_EXPORT)
+    so = os.path.join(out_dir, "libxrs_rskhost.so")
+    cmd = [gxx, "-O2", "-std=c++17", "-shared", "-fPIC", "-pthread", "-ffp-contract=off", "-Wl,-Bsymbolic",
+           f"-I{os.path.join(ROOT, 'include')}", src, "-o", so]
+    res = subprocess.run(cmd, capture_output=True, text=True)
+    if res.returncode != 0:
+        raise RuntimeError("host build of resample.cu / resample_fast.cu failed:\n" + res.stderr[-6000:])
+    return so
+
+
+def aligned_view(a, pitch: int, slice_stride: int, elem_off: int, base_align: int = 256):
+    """(n, h, w) copy of ``a`` in a fresh buffer whose first element sits ``elem_off`` elements past a
+    ``base_align``-byte boundary, rows ``pitch`` and slices ``slice_stride`` elements apart."""
+    a = np.asarray(a)
+    n, h, w = a.shape
+    es = a.dtype.itemsize
+    nbytes = (elem_off + (n - 1) * slice_stride + (h - 1) * pitch + w) * es
+    raw = np.zeros(nbytes + base_align, dtype=np.uint8)
+    start = (-raw.ctypes.data) % base_align
+    flat = raw[start:start + nbytes].view(a.dtype)
+    view = np.lib.stride_tricks.as_strided(flat[elem_off:], (n, h, w), (slice_stride * es, pitch * es, es))
+    view[...] = a
+    return view
+
+
+class ResampleKernels:
+    """The C ABI of the affine / coarsen family on host buffers through :func:`build_resample_kernels`.  Every call
+    returns ``(out, kernels, misaligned)``: the kernel names launched and the number of misaligned loads."""
+
+    def __init__(self, so_path: str):
+        self.lib = ctypes.CDLL(so_path)
+        c_d, c_i, c_l, c_p, c_64 = ctypes.c_double, ctypes.c_int32, ctypes.c_long, ctypes.c_void_p, ctypes.c_int64
+        self.lib.xrs_affine.restype = ctypes.c_int
+        self.lib.xrs_affine.argtypes = [c_p, c_p, c_i] + [c_64] * 7 + [c_d] * 4 + [c_i, c_d, c_i, c_i, c_i, c_i, c_p]
+        self.lib.xrs_affine_recover.restype = ctypes.c_int
+        self.lib.xrs_affine_recover.argtypes = [c_p, c_p, c_i] + [c_64] * 7 + [c_d] * 5 + [c_i, c_i, c_i, c_i, c_p]
+        self.lib.xrs_coarsen.restype = ctypes.c_int
+        self.lib.xrs_coarsen.argtypes = [c_p, c_p, c_i] + [c_64] * 5 + [c_i, c_i, c_i, c_p]
+        self.lib.xrs_has_nan.restype = ctypes.c_int
+        self.lib.xrs_has_nan.argtypes = [c_p, c_i] + [c_64] * 5 + [c_p, c_p]
+        self.lib.xrsh_take_log.restype = c_l
+        self.lib.xrsh_take_log.argtypes = [c_p, c_l, c_p, c_l]
+        self.lib.xrsh_u8x4.restype = ctypes.c_int
+        self.lib.xrsh_u8x4.argtypes = [c_p, c_p, c_i] + [c_l] * 5 + [c_i]
+        self.lib.xrsh_simd.restype = ctypes.c_int
+        self.lib.xrsh_simd.argtypes = [ctypes.c_int, c_p, c_p, c_p, c_p, c_l]
+        self.take()
+
+    def take(self):
+        names, err = ctypes.create_string_buffer(1 << 16), ctypes.create_string_buffer(1024)
+        mis = self.lib.xrsh_take_log(names, 1 << 16, err, 1024)
+        kernels = [k for k in names.value.decode().split(";") if k]
+        return kernels, int(mis), err.value.decode()
+
+    def _finish(self, rc, out, what):
+        kernels, mis, err = self.take()
+        if rc:
+            raise RuntimeError(f"{what} failed: {err}")
+        return out, kernels, mis
+
+    @staticmethod
+    def _geom(view):
+        """What the Python layer passes (affine.py): row pitch, and the slice stride (h * pitch for one slice)."""
+        n, h, w = view.shape
+        es = view.dtype.itemsize
+        pitch = view.strides[1] // es
+        return n, h, w, pitch, (view.strides[0] // es if n > 1 else h * pitch)
+
+    def affine(self, view, scale_ji, offset_ji, out_hw, order, cval, agg="mean", factors=(1, 1), slice_blend=False):
+        from xcube_resampling_b200.constants import AGG_CODES, DTYPE_CODES
+
+        n, h, w, pitch, sstride = self._geom(view)
+        f_j, f_i = int(factors[0]), int(factors[1])
+        is_float = view.dtype.kind == "f"
+        i64 = f_j * f_i > 1 and (agg in ("mode", "count") or (not is_float and agg in ("sum", "prod")))
+        out = aligned_view(np.zeros((n, int(out_hw[0]), int(out_hw[1])), np.int64 if i64 else view.dtype),
+                           int(out_hw[1]), int(out_hw[0]) * int(out_hw[1]), 0)
+        rc = self.lib.xrs_affine(view.ctypes.data, out.ctypes.data, DTYPE_CODES[view.dtype], n, h, w, pitch, sstride,
+                                 int(out_hw[0]), int(out_hw[1]), float(scale_ji[0]), float(offset_ji[0]),
+                                 float(scale_ji[1]), float(offset_ji[1]), int(order), float(cval), AGG_CODES[agg], f_j, f_i,
+                                 int(bool(slice_blend)), None)
+        return self._finish(rc, out, "xrs_affine")
+
+    def affine_recover(self, view, scale_ji, offset_ji, out_hw, cval, agg="mean", factors=(1, 1), slice_blend=False):
+        from xcube_resampling_b200.constants import AGG_CODES, DTYPE_CODES
+
+        n, h, w, pitch, sstride = self._geom(view)
+        out = aligned_view(np.zeros((n, int(out_hw[0]), int(out_hw[1]))), int(out_hw[1]), int(out_hw[0]) * int(out_hw[1]), 0)
+        rc = self.lib.xrs_affine_recover(view.ctypes.data, out.ctypes.data, DTYPE_CODES[view.dtype], n, h, w, pitch,
+                                         sstride, int(out_hw[0]), int(out_hw[1]), float(scale_ji[0]), float(offset_ji[0]),
+                                         float(scale_ji[1]), float(offset_ji[1]), float(cval), AGG_CODES[agg],
+                                         int(factors[0]), int(factors[1]), int(bool(slice_blend)), None)
+        return self._finish(rc, out, "xrs_affine_recover")
+
+    def coarsen(self, view, factors, agg):
+        from xcube_resampling_b200.constants import AGG_CODES, DTYPE_CODES
+
+        n, h, w, pitch, sstride = self._geom(view)
+        f_j, f_i = int(factors[0]), int(factors[1])
+        i64 = agg in ("mode", "count") or (view.dtype.kind != "f" and agg in ("sum", "prod"))
+        oh, ow = h // f_j, w // f_i
+        out = aligned_view(np.zeros((n, oh, ow), np.int64 if i64 else view.dtype), ow, oh * ow, 0)
+        rc = self.lib.xrs_coarsen(view.ctypes.data, out.ctypes.data, DTYPE_CODES[view.dtype], n, h, w, pitch, sstride,
+                                  AGG_CODES[agg], f_j, f_i, None)
+        return self._finish(rc, out, "xrs_coarsen")
+
+    def u8x4(self, view, f, agg):
+        """k5_u8x4_reduce on its own (every aggregation it implements, median and mode included)."""
+        from xcube_resampling_b200.constants import AGG_CODES
+
+        n, h, w, pitch, sstride = self._geom(view)
+        i64 = agg in ("mode", "count", "sum")
+        out = aligned_view(np.zeros((n, h // f, w // f), np.int64 if i64 else np.uint8), w // f, (h // f) * (w // f), 0)
+        rc = self.lib.xrsh_u8x4(view.ctypes.data, out.ctypes.data, int(f), n, h, w, pitch, sstride, AGG_CODES[agg])
+        return self._finish(rc, out, "k5_u8x4_reduce")
+
+    def has_nan(self, view):
+        from xcube_resampling_b200.constants import DTYPE_CODES
+
+        n, h, w, pitch, sstride = self._geom(view)
+        flag = np.full(1, 7, dtype=np.int32)
+        rc = self.lib.xrs_has_nan(view.ctypes.data, DTYPE_CODES[view.dtype], n, h, w, pitch, sstride, flag.ctypes.data, None)
+        return self._finish(rc, bool(flag[0]), "xrs_has_nan")
+
+    def simd(self, op: str, a, b, c=None) -> np.ndarray:
+        a = np.ascontiguousarray(a, dtype=np.uint32)
+        b = np.ascontiguousarray(b, dtype=np.uint32)
+        c = np.ascontiguousarray(np.zeros_like(a) if c is None else c, dtype=np.uint32)
+        out = np.empty_like(a)
+        rc = self.lib.xrsh_simd(SIMD_OPS.index(op), a.ctypes.data, b.ctypes.data, c.ctypes.data, out.ctypes.data, a.size)
+        assert rc == 0
+        return out

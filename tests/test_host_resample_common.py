@@ -48,17 +48,24 @@ def test_window_sums_follow_numpys_summation_order(lib, dtype, fn, f_j, f_i):
 
 
 def test_integer_output_conversion_is_scipys(lib):
+    """All nine dtypes, including what C leaves undefined and scipy on x86 defines: NaN, +-inf, 2^63 after the
+    +0.5 (INT64_MIN), beyond it (INT64_MAX), and values whose +0.5 rounds half to even in float64."""
     v = np.concatenate([np.linspace(-70000.0, 70000.0, 2801), np.arange(-6, 7) + 0.5, np.arange(-6, 7) - 0.5,
                         [0.0, -0.0, 0.49999999999999994, 254.5, 255.5, 32767.5, -32768.5, 65535.49, 65535.5, 2147483647.5,
-                         -2147483648.5, 4e9, -4e9]])
+                         -2147483648.5, 4e9, -4e9, 127.5, -128.5, 128.5, -129.5, 2.0 ** 31 - 0.5, 2.0 ** 31 + 0.5,
+                         2.0 ** 32 - 0.5, 2.0 ** 32 + 0.5, np.nan, -np.nan, np.inf, -np.inf, 1e300, -1e300, 2.0 ** 63,
+                         2.0 ** 63 - 1024, 2.0 ** 63 + 2048, 2.0 ** 64, -2.0 ** 63, -2.0 ** 63 - 4096, 2.0 ** 52 + 1,
+                         -2.0 ** 52 - 1, 2.0 ** 53 + 2, 1.7e18]])
     n = v.size
-    u8, i16 = np.empty(n, np.uint8), np.empty(n, np.int16)
-    i32, u16 = np.empty(n, np.int32), np.empty(n, np.uint16)
-    lib.xrsh_scipy_cast(_p(v), ctypes.c_long(n), _p(u8), _p(i16), _p(i32), _p(u16))
-    # scipy's own conversion: an identity affine_transform of the float64 values into an integer output
-    for got, dt in ((u8, np.uint8), (i16, np.int16), (i32, np.int32), (u16, np.uint16)):
+    dtypes = (np.float32, np.float64, np.uint8, np.int8, np.uint16, np.int16, np.int32, np.uint32, np.int64)
+    out = np.zeros(sum(np.dtype(d).itemsize for d in dtypes) * n, np.uint8)
+    lib.xrsh_scipy_cast(_p(v), ctypes.c_long(n), _p(out))
+    off = 0
+    for dt in dtypes:  # scipy's own conversion: an identity affine_transform of the float64 values
+        got = out[off:off + np.dtype(dt).itemsize * n].view(dt)
+        off += np.dtype(dt).itemsize * n
         want = ndimage.affine_transform(v, [1.0], output=dt, order=0, mode="constant")
-        assert np.array_equal(got, want), dt
+        assert np.array_equal(got, want, equal_nan=np.dtype(dt).kind == "f"), dt
 
 
 @pytest.mark.parametrize("length", [2, 3, 8, 100])

@@ -99,12 +99,24 @@ def affine_resample_dev(src: torch.Tensor, scale_ji, offset_ji, out_hw, order: i
 
 def coarsen_dev(src: torch.Tensor, factors, agg: str) -> torch.Tensor:
     """``dask.array.coarsen(agg, array, {y: f_j, x: f_i})`` on device buffers (``xrs_coarsen``)."""
+    lib = load()
     h, w = src.shape[-2:]
     f_j, f_i = int(factors[0]), int(factors[1])
     if h % f_j or w % f_i:
         raise ValueError("coarsening factors must divide the image size")
-    return affine_resample_dev(src, (1.0, 1.0), (0.0, 0.0), (h // f_j, w // f_i), 0, 0.0, agg, (f_j, f_i),
-                               slice_blend=False)
+    squeeze = src.dim() == 2
+    src3 = src.unsqueeze(0) if squeeze else src
+    if src3.stride(2) != 1:
+        src3 = src3.contiguous()
+    dt = _np_dtype(src3)
+    n = src3.shape[0]
+    out_int64 = f_j * f_i > 1 and (agg in _INT64_OUT_AGGS or (dt.kind != "f" and agg in ("sum", "prod")))
+    out = _dev.empty((n, h // f_j, w // f_i), np.dtype(np.int64) if out_int64 else dt, src3.device)
+    slice_stride = src3.stride(0) if n > 1 else h * src3.stride(1)
+    # xrs_coarsen, not xrs_affine: the values as stored, without scipy's float64 round trip
+    check(lib.xrs_coarsen(_dev.ptr(src3), _dev.ptr(out), DTYPE_CODES[dt], n, h, w, src3.stride(1), slice_stride,
+                          AGG_CODES[agg], f_j, f_i, _dev.stream_ptr(src3.device)), "xrs_coarsen")
+    return out[0] if squeeze else out
 
 
 def _resample_array_dev(src: torch.Tensor, affine_matrix, output_hw, interp_method: int, agg_method: str,

@@ -35,7 +35,12 @@ __device__ __forceinline__ T affine_sample(const T *__restrict__ sl, const T *__
         if (cj < 0.0 || cj > static_cast<double>(g.src_h - 1) || ci < 0.0 || ci > static_cast<double>(g.src_w - 1))
             return scipy_cast<T>(g.cval);
         const int64_t j = static_cast<int64_t>(floor(dadd(cj, 0.5))), i = static_cast<int64_t>(floor(dadd(ci, 0.5)));
-        return __ldg(sl + j * g.src_pitch + i);
+        const T v = __ldg(sl + j * g.src_pitch + i);
+        if constexpr (std::is_floating_point<T>::value || sizeof(T) == 8) {
+            // scipy adds every sample as a double to 0.0: -0.0 becomes +0.0, int64 beyond 2^53 is rounded
+            if (!g.exact_samples) return scipy_cast<T>(dadd(0.0, static_cast<double>(v)));
+        }
+        return v;
     }
     const Axis1 aj = axis_order1(cj, g.src_h), ai = axis_order1(ci, g.src_w);
     if (!aj.inside || !ai.inside) return scipy_cast<T>(g.cval);
@@ -157,11 +162,11 @@ __device__ __forceinline__ OutT reduce_window(T *w, int f_j, int f_i, int agg) {
             return OutT(0);
         }
         insertion_sort(w, m);
-        if (m & 1) return static_cast<OutT>(w[m / 2]);
-        const T a = w[m / 2 - 1], b = w[m / 2];
-        if constexpr (FLT) {  // np.mean of the two middle values in T
-            return static_cast<OutT>(static_cast<T>(static_cast<T>(a + b) * T(0.5)));
-        } else {  // float64 mean, then rint (half to even) and cast
+        const T b = w[m / 2], a = (m & 1) ? b : w[m / 2 - 1];
+        if constexpr (FLT) {  // np.nanmedian of small windows (np.ma.median): (low + high) / 2 in T, summed from +0.0
+            return static_cast<OutT>(static_cast<T>(static_cast<T>(static_cast<T>(a + b) + T(0)) * T(0.5)));
+        } else {  // float64 mean (np.median: of the middle value alone for odd counts), then rint (half to even), cast
+            if (m & 1) return static_cast<OutT>(static_cast<long long>(rint(static_cast<double>(b))));
             return static_cast<OutT>(static_cast<long long>(rint((static_cast<double>(a) + static_cast<double>(b)) / 2.0)));
         }
     }
@@ -228,10 +233,10 @@ __global__ void __launch_bounds__(256) k4_affine_generic(const T *__restrict__ s
     if (oi >= g.dst_w || oj >= g.dst_h) return;
     const T *cur = src + sl * g.src_slice_stride;
     const T *nx = nullptr;
-    if (g.slice_blend && g.order == 1 && std::is_floating_point<T>::value && g.n_slices > 1) {
+    if (g.slice_blend && g.order == 1 && std::is_floating_point<T>::value) {
         int64_t nsl = sl + 1;
-        if (nsl >= g.n_slices) nsl = g.n_slices > 2 ? g.n_slices - 2 : 0;  // mirrored tap
-        if (nsl != sl) nx = src + nsl * g.src_slice_stride;
+        if (nsl >= g.n_slices) nsl = g.n_slices > 2 ? g.n_slices - 2 : 0;  // mirrored tap; one slice: itself
+        nx = src + nsl * g.src_slice_stride;
     }
     OutT *out = dst + (sl * g.dst_h + oj) * g.dst_w + oi;
     const int n = g.f_j * g.f_i;
@@ -253,10 +258,10 @@ __global__ void __launch_bounds__(256) k4_affine_recover(const T *__restrict__ s
     if (oi >= g.dst_w || oj >= g.dst_h) return;
     const T *cur = src + sl * g.src_slice_stride;
     const T *nx = nullptr;
-    if (g.slice_blend && g.n_slices > 1) {
+    if (g.slice_blend) {
         int64_t nsl = sl + 1;
         if (nsl >= g.n_slices) nsl = g.n_slices > 2 ? g.n_slices - 2 : 0;
-        if (nsl != sl) nx = src + nsl * g.src_slice_stride;
+        nx = src + nsl * g.src_slice_stride;
     }
     double *out = dst + (sl * g.dst_h + oj) * g.dst_w + oi;
     const int n = g.f_j * g.f_i;
@@ -316,16 +321,10 @@ static int launch_affine(const void *src, void *dst, const AffineGeom &g, cudaSt
     return 0;
 }
 
-}  // namespace xrs
-
-using namespace xrs;
-
-extern "C" {
-
-int xrs_affine(const void *src, void *dst, int32_t dtype, int64_t n_slices, int64_t src_h, int64_t src_w,
-               int64_t src_pitch, int64_t src_slice_stride, int64_t dst_h, int64_t dst_w, double j_scale, double j_off,
-               double i_scale, double i_off, int32_t order, double cval, int32_t agg, int32_t f_j, int32_t f_i,
-               int32_t slice_blend, void *stream) {
+static int affine_entry(const void *src, void *dst, int32_t dtype, int64_t n_slices, int64_t src_h, int64_t src_w,
+                        int64_t src_pitch, int64_t src_slice_stride, int64_t dst_h, int64_t dst_w, double j_scale,
+                        double j_off, double i_scale, double i_off, int32_t order, double cval, int32_t agg, int32_t f_j,
+                        int32_t f_i, int32_t slice_blend, int exact_samples, void *stream) {
     if (!src || !dst) return fail("xrs_affine: null pointer");
     if (order != 0 && order != 1)
         return fail("interp_methods must be one of 0, 1, 'nearest', 'bilinear'. Higher order is not supported for 3D "
@@ -345,6 +344,7 @@ int xrs_affine(const void *src, void *dst, int32_t dtype, int64_t n_slices, int6
     g.dst_h = dst_h; g.dst_w = dst_w;
     g.j_scale = j_scale; g.j_off = j_off; g.i_scale = i_scale; g.i_off = i_off; g.cval = cval;
     g.order = order; g.agg = agg; g.f_j = f_j; g.f_i = f_i; g.slice_blend = slice_blend;
+    g.exact_samples = exact_samples;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (f_j * f_i > 1) {  // aligned integer-factor windows: streaming kernels (resample_fast.cu)
         bool handled = false;
@@ -355,12 +355,26 @@ int xrs_affine(const void *src, void *dst, int32_t dtype, int64_t n_slices, int6
     return 0;
 }
 
+}  // namespace xrs
+
+using namespace xrs;
+
+extern "C" {
+
+int xrs_affine(const void *src, void *dst, int32_t dtype, int64_t n_slices, int64_t src_h, int64_t src_w,
+               int64_t src_pitch, int64_t src_slice_stride, int64_t dst_h, int64_t dst_w, double j_scale, double j_off,
+               double i_scale, double i_off, int32_t order, double cval, int32_t agg, int32_t f_j, int32_t f_i,
+               int32_t slice_blend, void *stream) {
+    return affine_entry(src, dst, dtype, n_slices, src_h, src_w, src_pitch, src_slice_stride, dst_h, dst_w, j_scale, j_off,
+                        i_scale, i_off, order, cval, agg, f_j, f_i, slice_blend, 0, stream);
+}
+
 int xrs_coarsen(const void *src, void *dst, int32_t dtype, int64_t n_slices, int64_t src_h, int64_t src_w,
                 int64_t src_pitch, int64_t src_slice_stride, int32_t agg, int32_t f_j, int32_t f_i, void *stream) {
     if (f_j < 1 || f_i < 1 || src_h % f_j || src_w % f_i) return fail("xrs_coarsen: factors must divide the image size");
-    // identity nearest-neighbour "resample" + aggregation == dask.array.coarsen
-    return xrs_affine(src, dst, dtype, n_slices, src_h, src_w, src_pitch, src_slice_stride, src_h / f_j, src_w / f_i, 1.0,
-                      0.0, 1.0, 0.0, 0, 0.0, agg, f_j, f_i, 0, stream);
+    // identity nearest-neighbour "resample" of the values as stored + aggregation == dask.array.coarsen
+    return affine_entry(src, dst, dtype, n_slices, src_h, src_w, src_pitch, src_slice_stride, src_h / f_j, src_w / f_i, 1.0,
+                        0.0, 1.0, 0.0, 0, 0.0, agg, f_j, f_i, 0, 1, stream);
 }
 
 int xrs_has_nan(const void *src, int32_t dtype, int64_t n_slices, int64_t src_h, int64_t src_w, int64_t src_pitch,
@@ -396,6 +410,7 @@ int xrs_affine_recover(const void *src, double *dst, int32_t dtype, int64_t n_sl
     g.dst_h = dst_h; g.dst_w = dst_w;
     g.j_scale = j_scale; g.j_off = j_off; g.i_scale = i_scale; g.i_off = i_off; g.cval = cval;
     g.order = 1; g.agg = agg; g.f_j = f_j; g.f_i = f_i; g.slice_blend = slice_blend;
+    g.exact_samples = 0;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const dim3 block(32, 8);
     const dim3 grid(static_cast<unsigned>(ceil_div(dst_w, 32)), static_cast<unsigned>(ceil_div(dst_h, 8)), static_cast<unsigned>(n_slices));

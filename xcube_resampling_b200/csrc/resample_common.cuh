@@ -16,10 +16,16 @@ struct AffineGeom {
     double j_scale, j_off, i_scale, i_off;
     double cval;
     int order, agg, f_j, f_i, slice_blend;
+    // order-0 samples are the source values as stored (xrs_coarsen: dask's coarsen never converts); otherwise
+    // they take scipy's float64 round trip, which only 64-bit integers above 2^53 notice
+    int exact_samples;
 };
 
 // ---------------------------------------------------------------------------
-// scipy output conversion (CASE_INTERP_OUT*)
+// scipy output conversion (CASE_INTERP_OUT*) with the results scipy gets on x86 where C leaves the
+// conversion undefined: NaN -> INT32_MIN / INT64_MIN for 32- / 64-bit signed outputs (0 for narrower and
+// unsigned ones, whose conversion goes through a wider integer); 2^63 after the +0.5 -> INT64_MIN;
+// anything above -> INT64_MAX.  Written out so that the device and the host build agree.
 // ---------------------------------------------------------------------------
 template <typename T>
 __device__ __forceinline__ T scipy_cast(double t) {
@@ -33,10 +39,14 @@ __device__ __forceinline__ T scipy_cast(double t) {
         return static_cast<T>(static_cast<unsigned long long>(t));
     } else {
         t = t > 0 ? t + 0.5 : t - 0.5;
+        if (t != t) return sizeof(T) >= 4 ? std::numeric_limits<T>::min() : T(0);
         const double mx = static_cast<double>(std::numeric_limits<T>::max());
         const double mn = static_cast<double>(std::numeric_limits<T>::min());
-        t = t > mx ? mx : t;
-        t = t < mn ? mn : t;
+        if (t > mx) return std::numeric_limits<T>::max();
+        if (t < mn) return std::numeric_limits<T>::min();
+        if constexpr (sizeof(T) == 8) {
+            if (t == mx) return std::numeric_limits<T>::min();  // double(INT64_MAX) is 2^63
+        }
         return static_cast<T>(static_cast<long long>(t));
     }
 }

@@ -221,12 +221,12 @@ __device__ __forceinline__ OutT reduce_sort(T (&w)[F * F], int agg) {
             a = pick<N>(w, (m - 1) / 2);
             b = pick<N>(w, m / 2);
         }
-        if (m & 1) return static_cast<OutT>(b);
-        if constexpr (FLT) {
-            return static_cast<OutT>(static_cast<T>(static_cast<T>(a + b) * T(0.5)));
-        } else {
-            return static_cast<OutT>(static_cast<long long>(rint((static_cast<double>(a) + static_cast<double>(b)) / 2.0)));
+        if constexpr (FLT) {  // np.nanmedian of small windows (np.ma.median): (low + high) / 2 in T, summed from +0.0
+            if (m & 1) a = b;
+            return static_cast<OutT>(static_cast<T>(static_cast<T>(static_cast<T>(a + b) + T(0)) * T(0.5)));
         }
+        if (m & 1) return static_cast<OutT>(b);
+        return static_cast<OutT>(static_cast<long long>(rint((static_cast<double>(a) + static_cast<double>(b)) / 2.0)));
     }
     // mode (coarsen.py:138-155): most frequent value, lowest value wins ties
     bitonic_sort<N>(w);
@@ -776,7 +776,11 @@ int launch_affine_fast(const void *src, void *dst, int dtype, const AffineGeom &
     if (static_cast<int64_t>(a.j_off) + a.dst_h * a.f_j > a.src_h || static_cast<int64_t>(a.i_off) + a.dst_w * a.f_i > a.src_w)
         return 0;
     const bool is_float = dtype == XRS_F32 || dtype == XRS_F64;
-    if (a.order == 1 && is_float && a.slice_blend && a.n_slices > 1) return 0;  // next-slice taps: generic kernel
+    if (a.order == 1 && is_float && a.slice_blend) return 0;  // next-slice taps (one slice: its own): generic kernel
+    // samples scipy changes on the way through float64 -- int64 beyond 2^53 at order 0 and 1, -0.0 at order 0 --
+    // unless they come from xrs_coarsen: generic kernel
+    if (a.order == 0 && !a.exact_samples && (is_float || dtype == XRS_I64)) return 0;
+    if (a.order == 1 && dtype == XRS_I64) return 0;
     if (a.n_slices > 65535 || ceil_div(a.dst_h, 8) > 65535) return 0;
     XRS_DISPATCH_DTYPE(dtype, T, return launch_t<T>(src, dst, a, st, handled));
     return 0;
