@@ -194,8 +194,15 @@ int xrs_rectify_ij(const double *x, const double *y, int64_t src_h, int64_t src_
  *   dst_planes_host  HOST array of n_bands device pointers, each a
  *                    (dst_h, dst_w) plane of `dtype`, contiguous rows
  *   ij               (2, dst_h, dst_w) float64 from xrs_rectify_ij
- *   fill             value written where ij is NaN (cast to dtype with a C cast)
- * Arithmetic is float64 without FMA contraction, one C cast to dtype at the end. */
+ *   fill             value written where ij is NaN, converted to dtype like np.full(..., float(fill), dtype)
+ *                    on x86 (xrs_casts.h): NaN gives INT32_MIN / INT64_MIN for int32 / int64 and 0 for the
+ *                    other integer types, -1 gives 0xFFFFFFFF for uint32.  A double cannot hold every
+ *                    int64: fills beyond 2^53 arrive rounded to the nearest double (INT64_MAX as 2^63,
+ *                    which converts to INT64_MIN).
+ * Arithmetic is float64 without FMA contraction, one cast to dtype at the end with x86's results (an int64
+ * sample that rounds to 2^63 stores INT64_MIN).  Nearest samples take the reference's float64 round trip
+ * of the source window (rectify.py:628-630): int64 values beyond 2^53 are rounded, INT64_MAX reads back as
+ * INT64_MIN; every other dtype is copied unchanged. */
 int xrs_gather_ij(const void *const *src_planes_host, void *const *dst_planes_host, int32_t n_bands,
                   int32_t dtype, int64_t src_h, int64_t src_w, int64_t src_pitch, int64_t win_i0, int64_t win_j0,
                   int64_t win_w, int64_t win_h, const double *ij, int64_t dst_h, int64_t dst_w, int32_t method,
@@ -328,5 +335,6 @@ int xrs_coarsen(const void *src, void *dst, int32_t dtype, int64_t n_slices, int
 
 #ifdef __cplusplus
 }
+#include "xrs_casts.h" /* the conversions behind `fill` and the integer stores above, as C++ templates */
 #endif
 #endif /* XRS_H_ */

@@ -77,6 +77,16 @@ def rectify_ij_block(x_win, y_win, src_i_min, src_j_min, dst_h, dst_w, x_off, y_
     return out
 
 
+def _full(shape, fill_value, dtype) -> np.ndarray:
+    """rectify.py:618,621: ``np.full(shape, fill_value, dtype=src dtype)``.  numpy 2 refuses a Python int outside the
+    dtype's range -- the default integer fill -1 (utils.py:307-316) of a uint32 variable raises OverflowError -- where
+    numpy 1.x wrapped it modulo 2**bits (-1 -> 0xFFFFFFFF); this returns numpy 1.x's value."""
+    try:
+        return np.full(shape, fill_value, dtype=dtype)
+    except OverflowError:
+        return np.full(shape, np.array(fill_value).astype(dtype), dtype=dtype)
+
+
 def gather(src, ij, method, fill_value) -> np.ndarray:
     """rectify.py:579-734: (bands, h, w) or (h, w) source -> target via the ij image."""
     if method not in METHODS:
@@ -90,7 +100,7 @@ def gather(src, ij, method, fill_value) -> np.ndarray:
     ij = np.ascontiguousarray(ij, dtype=np.float64)
     bands, sh, sw = src3.shape
     _, dh, dw = ij.shape
-    out = np.full((bands, dh, dw), fill_value, dtype=src3.dtype)
+    out = _full((bands, dh, dw), fill_value, src3.dtype)
     rc = lib().xrso_gather_ij(ptr(src3), code, bands, sh, sw, ptr(ij), ptr(out), dh, dw, METHODS[method])
     assert rc == 0
     return out[0] if squeeze else out

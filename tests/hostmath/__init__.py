@@ -291,17 +291,11 @@ def resolve(so_path: str, x, y, tile_boxes, claims, g) -> np.ndarray:
 # ---------------------------------------------------------------------------
 # K2's per-pixel arithmetic (csrc/gather_common.cuh: make_taps / interp_value)
 # ---------------------------------------------------------------------------
+# cast_like_numpy / cast_fill come with "xrs.h" (include/xrs_casts.h), which every shim includes
 GATHER_SHIM = r"""
 #include <algorithm>
 #include <type_traits>
 using std::min; using std::max;
-namespace xrs {
-// common.cuh: float64 -> T with a C cast (what numba emits for `out[...] = float64_value`)
-template <typename T> static inline T cast_from_f64(double v) {
-    if constexpr (std::is_floating_point<T>::value) return static_cast<T>(v);
-    else return static_cast<T>(static_cast<long long>(v));
-}
-}
 """
 
 GATHER_EXPORT = r"""
@@ -316,8 +310,8 @@ static void gather_one(const T *src, long n_bands, long src_h, long src_w, const
                 const T *sp = src + b * src_h * src_w;
                 T out = fill;
                 if (t.valid) {
-                    if (METHOD == XRS_NEAREST) out = sp[t.j0 * src_w + t.i0];
-                    else out = xrs::cast_from_f64<T>(xrs::interp_value<METHOD>(
+                    if (METHOD == XRS_NEAREST) out = xrs::nearest_value(sp[t.j0 * src_w + t.i0]);
+                    else out = xrs::cast_like_numpy<T>(xrs::interp_value<METHOD>(
                         static_cast<double>(sp[t.j0 * src_w + t.i0]), static_cast<double>(sp[t.j0 * src_w + t.i1]),
                         static_cast<double>(sp[t.j1 * src_w + t.i0]), static_cast<double>(sp[t.j1 * src_w + t.i1]), t.u, t.v));
                 }
@@ -348,6 +342,8 @@ extern "C" int xrsh_gather(const void *src, int dtype, long n_bands, long src_h,
     case XRS_U16: return gather_t<uint16_t>(src, n_bands, src_h, src_w, ij, dst, dst_h, dst_w, method, fill);
     case XRS_I32: return gather_t<int32_t>(src, n_bands, src_h, src_w, ij, dst, dst_h, dst_w, method, fill);
     case XRS_I64: return gather_t<int64_t>(src, n_bands, src_h, src_w, ij, dst, dst_h, dst_w, method, fill);
+    case XRS_I8: return gather_t<int8_t>(src, n_bands, src_h, src_w, ij, dst, dst_h, dst_w, method, fill);
+    case XRS_U32: return gather_t<uint32_t>(src, n_bands, src_h, src_w, ij, dst, dst_h, dst_w, method, fill);
     }
     return 2;
 }
@@ -1433,7 +1429,23 @@ def lon_360(so_path: str, x, blocks: int = 2) -> np.ndarray:
 # memory" (elements outside the tensor read as zero, as the TMA unit fills them) and then completes the
 # mbarrier's phase; an mbarrier is a counter of completed phases whose parity `mbar_wait` polls; the fences are
 # no-ops; `elem_ptr` is pointer arithmetic.  A CTA is K2S_THREADS host threads.
-K2_SHIM = K0_SHIM + GATHER_SHIM.replace("#include <algorithm>\n", "").replace("using std::min; using std::max;\n", "") + r"""
+XRSH_DISPATCH = r"""
+// XRS_DISPATCH_DTYPE of common.cuh without its error path
+#define XRSH_DISPATCH_DTYPE(dtype, T, ...)                         \
+    switch (dtype) {                                               \
+    case XRS_F32: { using T = float; __VA_ARGS__; break; }         \
+    case XRS_F64: { using T = double; __VA_ARGS__; break; }        \
+    case XRS_U8: { using T = uint8_t; __VA_ARGS__; break; }        \
+    case XRS_I8: { using T = int8_t; __VA_ARGS__; break; }         \
+    case XRS_U16: { using T = uint16_t; __VA_ARGS__; break; }      \
+    case XRS_I16: { using T = int16_t; __VA_ARGS__; break; }       \
+    case XRS_I32: { using T = int32_t; __VA_ARGS__; break; }       \
+    case XRS_U32: { using T = uint32_t; __VA_ARGS__; break; }      \
+    case XRS_I64: { using T = int64_t; __VA_ARGS__; break; }       \
+    }
+"""
+
+K2_SHIM = XRSH_DISPATCH + K0_SHIM + GATHER_SHIM.replace("#include <algorithm>\n", "").replace("using std::min; using std::max;\n", "") + r"""
 #include <functional>
 #define __grid_constant__
 namespace xrs {
@@ -1607,12 +1619,7 @@ extern "C" int xrsh_k2_gather(const void *src, int dtype, long band_stride, int 
                               int method, double fill, int staged, long *stats) {
     xrs::xrsh_tma_boxes = xrs::xrsh_tma_oob = 0;
     int rc = 2;
-    switch (dtype) {
-    case XRS_F32: rc = xrsh_gather_t<float>(src, band_stride, n_bands, src_h, src_w, src_pitch, win_i0, win_j0, win_w, win_h, ij, dst, dst_h, dst_w, method, fill, staged != 0); break;
-    case XRS_F64: rc = xrsh_gather_t<double>(src, band_stride, n_bands, src_h, src_w, src_pitch, win_i0, win_j0, win_w, win_h, ij, dst, dst_h, dst_w, method, fill, staged != 0); break;
-    case XRS_U8: rc = xrsh_gather_t<uint8_t>(src, band_stride, n_bands, src_h, src_w, src_pitch, win_i0, win_j0, win_w, win_h, ij, dst, dst_h, dst_w, method, fill, staged != 0); break;
-    case XRS_I16: rc = xrsh_gather_t<int16_t>(src, band_stride, n_bands, src_h, src_w, src_pitch, win_i0, win_j0, win_w, win_h, ij, dst, dst_h, dst_w, method, fill, staged != 0); break;
-    }
+    XRSH_DISPATCH_DTYPE(dtype, T, rc = xrsh_gather_t<T>(src, band_stride, n_bands, src_h, src_w, src_pitch, win_i0, win_j0, win_w, win_h, ij, dst, dst_h, dst_w, method, fill, staged != 0));
     stats[0] = xrs::xrsh_tma_boxes; stats[1] = xrs::xrsh_tma_oob;
     return rc;
 }
@@ -1622,12 +1629,7 @@ extern "C" int xrsh_k2_gather_dual(const void *src, int dtype, long band_stride,
                                    long *stats) {
     xrs::xrsh_tma_boxes = xrs::xrsh_tma_oob = 0;
     int rc = 2;
-    switch (dtype) {
-    case XRS_F32: rc = xrsh_dual_t<float>(src, band_stride, n_bands, src_h, src_w, src_pitch, win_i0, win_j0, win_w, win_h, ij, dst_interp, dst_near, dst_h, dst_w, method, fill_interp, fill_near); break;
-    case XRS_F64: rc = xrsh_dual_t<double>(src, band_stride, n_bands, src_h, src_w, src_pitch, win_i0, win_j0, win_w, win_h, ij, dst_interp, dst_near, dst_h, dst_w, method, fill_interp, fill_near); break;
-    case XRS_U8: rc = xrsh_dual_t<uint8_t>(src, band_stride, n_bands, src_h, src_w, src_pitch, win_i0, win_j0, win_w, win_h, ij, dst_interp, dst_near, dst_h, dst_w, method, fill_interp, fill_near); break;
-    case XRS_I16: rc = xrsh_dual_t<int16_t>(src, band_stride, n_bands, src_h, src_w, src_pitch, win_i0, win_j0, win_w, win_h, ij, dst_interp, dst_near, dst_h, dst_w, method, fill_interp, fill_near); break;
-    }
+    XRSH_DISPATCH_DTYPE(dtype, T, rc = xrsh_dual_t<T>(src, band_stride, n_bands, src_h, src_w, src_pitch, win_i0, win_j0, win_w, win_h, ij, dst_interp, dst_near, dst_h, dst_w, method, fill_interp, fill_near));
     stats[0] = xrs::xrsh_tma_boxes; stats[1] = xrs::xrsh_tma_oob;
     return rc;
 }
@@ -1656,11 +1658,22 @@ void xrsh_fused_tm(const T *src, int n_bands, const xrs::IjGeom &geom, T *dst, d
     xrsh_launch(static_cast<unsigned>(ceil_div(dst_w, K2S_TW)), static_cast<unsigned>(ceil_div(dst_h, K2S_TH)), K2S_THREADS, false,
                 [&] { k2_gather_staged<T, METHOD, true>(sp, n_bands, geom.src_h, geom.src_w, geom.src_w, 0, 0, ijs, dst_h, dst_w, fill_t); });
 }
+template <typename T>
+int xrsh_fused_t(const void *src, int n_bands, const xrs::IjGeom &g, void *dst, int method, double fill) {
+    const T *s = static_cast<const T *>(src);
+    T *d = static_cast<T *>(dst);
+    switch (method) {
+    case XRS_NEAREST: xrsh_fused_tm<T, XRS_NEAREST>(s, n_bands, g, d, fill); return 0;
+    case XRS_BILINEAR: xrsh_fused_tm<T, XRS_BILINEAR>(s, n_bands, g, d, fill); return 0;
+    case XRS_TRIANGULAR: xrsh_fused_tm<T, XRS_TRIANGULAR>(s, n_bands, g, d, fill); return 0;
+    }
+    return 1;
 }
-extern "C" int xrsh_k2_gather_fused(const float *src, int n_bands, const double *x, const double *y, long src_h, long src_w,
+}
+extern "C" int xrsh_k2_gather_fused(const void *src, int dtype, int n_bands, const double *x, const double *y, long src_h, long src_w,
                                     const int64_t *tile_boxes, const uint32_t *claims, long dst_h, long dst_w, int tile_h,
                                     int tile_w, double x_min, double y_min, double y_max, double x_res, double y_res, int j_up,
-                                    long row_begin, long row_end, int method, double fill, float *dst) {
+                                    long row_begin, long row_end, int method, double fill, void *dst) {
     using namespace xrs;
     if (n_bands > K2_MAX_BANDS) return 3;
     IjGeom g = {};
@@ -1677,12 +1690,9 @@ extern "C" int xrsh_k2_gather_fused(const float *src, int n_bands, const double 
     g.magic_nqi = div_magic_of(static_cast<uint64_t>(src_w - 1));
     g.magic_tw = div_magic_of(static_cast<uint64_t>(g.tile_w));
     g.magic_th = div_magic_of(static_cast<uint64_t>(g.tile_h));
-    switch (method) {
-    case XRS_NEAREST: xrsh_fused_tm<float, XRS_NEAREST>(src, n_bands, g, dst, fill); return 0;
-    case XRS_BILINEAR: xrsh_fused_tm<float, XRS_BILINEAR>(src, n_bands, g, dst, fill); return 0;
-    case XRS_TRIANGULAR: xrsh_fused_tm<float, XRS_TRIANGULAR>(src, n_bands, g, dst, fill); return 0;
-    }
-    return 1;
+    int rc = 2;
+    XRSH_DISPATCH_DTYPE(dtype, T, rc = xrsh_fused_t<T>(src, n_bands, g, dst, method, fill));
+    return rc;
 }
 """
 
@@ -1731,8 +1741,9 @@ def _k2_codes():
         m = re.search(r"\b" + name + r"\s*=\s*(\d+)", hdr)
         assert m, name
         return int(m.group(1))
-    dt = {np.dtype(np.float32): code("XRS_F32"), np.dtype(np.float64): code("XRS_F64"), np.dtype(np.uint8): code("XRS_U8"),
-          np.dtype(np.int16): code("XRS_I16")}
+    dt = {np.dtype(t): code(name) for t, name in (
+        (np.float32, "XRS_F32"), (np.float64, "XRS_F64"), (np.uint8, "XRS_U8"), (np.int8, "XRS_I8"), (np.uint16, "XRS_U16"),
+        (np.int16, "XRS_I16"), (np.int32, "XRS_I32"), (np.uint32, "XRS_U32"), (np.int64, "XRS_I64"))}
     me = {"nearest": code("XRS_NEAREST"), "bilinear": code("XRS_BILINEAR"), "triangular": code("XRS_TRIANGULAR")}
     return dt, me
 
@@ -1792,23 +1803,23 @@ def k2_gather_dual(so_path: str, src, ij, method: str, fill_interp, fill_near, w
 
 
 def k2_gather_fused(so_path: str, src, x, y, tile_boxes, claims, g, method: str, fill, rows=None) -> np.ndarray:
-    """The gather half of ``xrs_rectify_gather`` (``k2_gather_staged<float, METHOD, FUSED = true>``): float32 bands
-    through K1's claim words (``claims``: (rows, W) uint32 of the row range ``rows``); ``g``: oracle RegularGrid."""
+    """The gather half of ``xrs_rectify_gather`` (``k2_gather_staged<T, METHOD, FUSED = true>``): the bands through K1's
+    claim words (``claims``: (rows, W) uint32 of the row range ``rows``); ``g``: oracle RegularGrid."""
     lib = ctypes.CDLL(so_path)
-    _, me = _k2_codes()
-    src = np.ascontiguousarray(src, dtype=np.float32)
+    dt, me = _k2_codes()
+    src = np.ascontiguousarray(src)
     x = np.ascontiguousarray(x, dtype=np.float64)
     y = np.ascontiguousarray(y, dtype=np.float64)
     boxes = np.ascontiguousarray(tile_boxes, dtype=np.int64)
     claims = np.ascontiguousarray(claims, dtype=np.uint32)
     r0, r1 = rows if rows is not None else (0, g.height)
     nb, h, w = src.shape
-    out = np.empty((nb, r1 - r0, g.width), dtype=np.float32)
+    out = np.empty((nb, r1 - r0, g.width), dtype=src.dtype)
     c_d, c_l, c_i, c_p = ctypes.c_double, ctypes.c_long, ctypes.c_int, ctypes.c_void_p
     lib.xrsh_k2_gather_fused.restype = c_i
-    lib.xrsh_k2_gather_fused.argtypes = [c_p, c_i, c_p, c_p, c_l, c_l, c_p, c_p, c_l, c_l, c_i, c_i, c_d, c_d, c_d, c_d, c_d, c_i,
+    lib.xrsh_k2_gather_fused.argtypes = [c_p, c_i, c_i, c_p, c_p, c_l, c_l, c_p, c_p, c_l, c_l, c_i, c_i, c_d, c_d, c_d, c_d, c_d, c_i,
                                          c_l, c_l, c_i, c_d, c_p]
-    rc = lib.xrsh_k2_gather_fused(src.ctypes.data, nb, x.ctypes.data, y.ctypes.data, h, w, boxes.ctypes.data, claims.ctypes.data,
+    rc = lib.xrsh_k2_gather_fused(src.ctypes.data, dt[src.dtype], nb, x.ctypes.data, y.ctypes.data, h, w, boxes.ctypes.data, claims.ctypes.data,
                                   g.height, g.width, g.tile_h, g.tile_w, float(g.x_min), float(g.y_min), float(g.y_max),
                                   float(g.x_res), float(g.y_res), int(g.is_j_axis_up), r0, r1, me[method], float(fill),
                                   out.ctypes.data)
@@ -1825,7 +1836,7 @@ def k2_gather_fused(so_path: str, src, x, y, tile_boxes, claims, g, method: str,
 # lattice pre-kernel, the tile logic, the separable / row-block / lattice / exact forms and the per-pixel blend
 # are the product's text.  Differences to the device build: libm instead of CUDA's math library and no FMA
 # contraction in proj.cuh (~1e-9 m in the source coordinates).
-K3K_SHIM = "#define _GNU_SOURCE 1\n#define XRS_K3_LD256 0\n" + K0_SHIM.replace("#define __shared__\n", "#define __shared__ static\n") + r"""
+K3K_SHIM = "#define _GNU_SOURCE 1\n#define XRS_K3_LD256 0\n" + XRSH_DISPATCH + K0_SHIM.replace("#define __shared__\n", "#define __shared__ static\n") + r"""
 #include <string>
 #include <type_traits>
 #include <math.h>
@@ -1843,10 +1854,6 @@ static inline double dsub(double a, double b) { return a - b; }
 static inline double dmul(double a, double b) { return a * b; }
 static inline double ddiv(double a, double b) { return a / b; }
 template <typename T> static inline void st_stream(T *p, T v) { *p = v; }
-template <typename T> static inline T cast_from_f64(double v) {
-    if constexpr (std::is_floating_point<T>::value) return static_cast<T>(v);
-    else return static_cast<T>(static_cast<long long>(v));
-}
 }
 template <typename T> static inline T __ldg(const T *p) { return *p; }
 template <typename T> static inline T __ldcs(const T *p) { return *p; }
@@ -1927,9 +1934,7 @@ int xrsh_launch_reproject(const xrs::K3Geom &g_in, const T *src, int64_t band_st
     g.lat_nodes = nullptr;
     const int64_t rows = g.row_end - g.row_begin;
     const unsigned gx = static_cast<unsigned>(ceil_div(g.dst_w, K3T_COLS)), gy = static_cast<unsigned>(ceil_div(g.row_end - g.row_tile0, K3T_ROWS));
-    T fill_t;
-    if constexpr (std::is_floating_point<T>::value) fill_t = static_cast<T>(fill);
-    else fill_t = static_cast<T>(static_cast<long long>(fill));
+    const T fill_t = cast_fill<T>(fill);
     const int plan = choose_plan(g.from, g.to) | (exact_only ? K3_PLAN_EXACT_ONLY : 0);
     const bool axis_only = (g.from.kind == XRS_PROJ_GEOGRAPHIC || g.from.kind == XRS_PROJ_WEBMERC) &&
                            (g.to.kind == XRS_PROJ_GEOGRAPHIC || g.to.kind == XRS_PROJ_WEBMERC);
@@ -1957,9 +1962,25 @@ int xrsh_launch_reproject(const xrs::K3Geom &g_in, const T *src, int64_t band_st
 }
 }
 
-// xrs_reproject for float32 sources: out_f64 = 1 writes float64 (bilinear as the reference returns it).  src points at
-// the resident window's origin (win_i0, win_j0).
-extern "C" int xrsh_reproject(const float *src, long band_stride, int n_bands, int out_f64, long src_h, long src_w, long src_pitch,
+template <typename T>
+int xrsh_reproject_t(const xrs::K3Geom &g, const void *src_v, long band_stride, int n_bands, int out_f64, int method,
+                     double fill, int exact_only, int use_nodes, void *dst, long *stats) {
+    const T *src = static_cast<const T *>(src_v);
+    switch (method) {
+    case XRS_NEAREST:
+        return xrsh_launch_reproject<T, T, XRS_NEAREST>(g, src, band_stride, static_cast<T *>(dst), n_bands, fill, exact_only, use_nodes, stats);
+    case XRS_TRIANGULAR:
+        return xrsh_launch_reproject<T, T, XRS_TRIANGULAR>(g, src, band_stride, static_cast<T *>(dst), n_bands, fill, exact_only, use_nodes, stats);
+    case XRS_BILINEAR:
+        if (out_f64) return xrsh_launch_reproject<T, double, XRS_BILINEAR>(g, src, band_stride, static_cast<double *>(dst), n_bands, fill, exact_only, use_nodes, stats);
+        return xrsh_launch_reproject<T, T, XRS_BILINEAR>(g, src, band_stride, static_cast<T *>(dst), n_bands, fill, exact_only, use_nodes, stats);
+    }
+    return 2;
+}
+
+// xrs_reproject: out_f64 = 1 writes float64 (bilinear as the reference returns it), otherwise the source dtype.  src
+// points at the resident window's origin (win_i0, win_j0).
+extern "C" int xrsh_reproject(const void *src, int dtype, long band_stride, int n_bands, int out_f64, long src_h, long src_w, long src_pitch,
                               long win_i0, long win_j0, long win_w, long win_h, const xrs_proj *src_crs, const xrs_proj *dst_crs,
                               const double *dst_x, const double *dst_y, long dst_h, long dst_w, int tile_h, int tile_w,
                               const double *tile_x0, const double *tile_y0, const int32_t *tile_i0, const int32_t *tile_j0,
@@ -1982,16 +2003,9 @@ extern "C" int xrsh_reproject(const float *src, long band_stride, int n_bands, i
     g.inv_x_res = 1.0 / src_x_res; g.inv_y_res = 1.0 / src_y_res;
     g.src_h = src_h; g.src_w = src_w; g.src_pitch = src_pitch;
     g.win_i0 = win_i0; g.win_j0 = win_j0; g.win_w = win_w; g.win_h = win_h;
-    switch (method) {
-    case XRS_NEAREST:
-        return xrsh_launch_reproject<float, float, XRS_NEAREST>(g, src, band_stride, static_cast<float *>(dst), n_bands, fill, exact_only, use_nodes, stats);
-    case XRS_TRIANGULAR:
-        return xrsh_launch_reproject<float, float, XRS_TRIANGULAR>(g, src, band_stride, static_cast<float *>(dst), n_bands, fill, exact_only, use_nodes, stats);
-    case XRS_BILINEAR:
-        if (out_f64) return xrsh_launch_reproject<float, double, XRS_BILINEAR>(g, src, band_stride, static_cast<double *>(dst), n_bands, fill, exact_only, use_nodes, stats);
-        return xrsh_launch_reproject<float, float, XRS_BILINEAR>(g, src, band_stride, static_cast<float *>(dst), n_bands, fill, exact_only, use_nodes, stats);
-    }
-    return 2;
+    int rc = 3;
+    XRSH_DISPATCH_DTYPE(dtype, T, rc = xrsh_reproject_t<T>(g, src, band_stride, n_bands, out_f64, method, fill, exact_only, use_nodes, dst, stats));
+    return rc;
 }
 """
 
@@ -2028,19 +2042,20 @@ def build_k3(out_dir: str) -> str:
 
 def k3_reproject(so_path: str, src, src_gm, tgt_gm, windows, method: str, fill, out_f64=None, rows=None, window=None,
                  exact_only: bool = False, use_nodes: bool = True):
-    """``xrs_reproject`` (float32 sources) through the host build: ``(out, (plan, separable kernel, lattice nodes))``.
+    """``xrs_reproject`` through the host build: ``(out, (plan, separable kernel, lattice nodes))``; the output has the
+    source's dtype, or float64 with ``out_f64`` (default: bilinear, as the reference returns it).
     ``src_gm`` / ``tgt_gm``: the product's GridMappings; ``windows``: ``reproject.SourceWindows``; ``window`` =
     (i0, j0, i1, j1) resident part of the source; arguments are prepared as ``ReprojectPlan`` does."""
     from xcube_resampling_b200._lib import XrsProj
 
     lib = ctypes.CDLL(so_path)
-    _, me = _k2_codes()
-    src = np.ascontiguousarray(src, dtype=np.float32)
+    dt, me = _k2_codes()
+    src = np.ascontiguousarray(src)
     nb, h, w = src.shape
     if out_f64 is None:
         out_f64 = method == "bilinear"
     r0, r1 = rows if rows is not None else (0, tgt_gm.height)
-    out = np.empty((nb, r1 - r0, tgt_gm.width), dtype=np.float64 if out_f64 else np.float32)
+    out = np.empty((nb, r1 - r0, tgt_gm.width), dtype=np.float64 if out_f64 else src.dtype)
     base, bstride, pitch, i0, j0, ww, wh = _k2_window(src, window)
     sp, dp = XrsProj.from_crs(src_gm.crs), XrsProj.from_crs(tgt_gm.crs)
     dst_x = np.ascontiguousarray(tgt_gm.x_values, dtype=np.float64)
@@ -2052,9 +2067,9 @@ def k3_reproject(so_path: str, src, src_gm, tgt_gm, windows, method: str, fill, 
     stats = np.zeros(3, dtype=np.int64)
     c_d, c_l, c_i, c_p = ctypes.c_double, ctypes.c_long, ctypes.c_int, ctypes.c_void_p
     lib.xrsh_reproject.restype = c_i
-    lib.xrsh_reproject.argtypes = [c_p, c_l, c_i, c_i, c_l, c_l, c_l, c_l, c_l, c_l, c_l, c_p, c_p, c_p, c_p, c_l, c_l, c_i, c_i,
+    lib.xrsh_reproject.argtypes = [c_p, c_i, c_l, c_i, c_i, c_l, c_l, c_l, c_l, c_l, c_l, c_l, c_p, c_p, c_p, c_p, c_l, c_l, c_i, c_i,
                                    c_p, c_p, c_p, c_p, c_i, c_i, c_d, c_d, c_i, c_d, c_l, c_l, c_i, c_i, c_p, c_p]
-    rc = lib.xrsh_reproject(base, bstride, nb, int(out_f64), src_gm.height, src_gm.width, pitch, i0, j0, ww, wh,
+    rc = lib.xrsh_reproject(base, dt[src.dtype], bstride, nb, int(out_f64), src_gm.height, src_gm.width, pitch, i0, j0, ww, wh,
                             ctypes.addressof(sp), ctypes.addressof(dp), dst_x.ctypes.data, dst_y.ctypes.data, tgt_gm.height,
                             tgt_gm.width, tgt_gm.tile_height, tgt_gm.tile_width, x0.ctypes.data, y0.ctypes.data,
                             ti0.ctypes.data, tj0.ctypes.data, int(windows.win_w), int(windows.win_h), float(src_gm.x_res),

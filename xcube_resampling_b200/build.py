@@ -49,7 +49,7 @@ def _nvcc() -> str:
 def _stamp(src: str, flags) -> str:
     h = hashlib.sha256()
     h.update(" ".join(flags).encode())
-    for path in [src, os.path.join(INCLUDE, "xrs.h")] + sorted(
+    for path in [src] + sorted(os.path.join(INCLUDE, f) for f in os.listdir(INCLUDE) if f.endswith(".h")) + sorted(
         os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cuh", ".h"))
     ):
         with open(path, "rb") as fh:

@@ -144,16 +144,6 @@ static inline int dtype_size(int dtype) {
     }
 }
 
-// float64 -> T with a C cast (what numba emits for `out[...] = float64_value`)
-template <typename T>
-__device__ __forceinline__ T cast_from_f64(double v) {
-    if constexpr (std::is_floating_point<T>::value) {
-        return static_cast<T>(v);
-    } else {
-        return static_cast<T>(static_cast<long long>(v));
-    }
-}
-
 #define XRS_DISPATCH_DTYPE(dtype, T, ...)                                   \
     switch (dtype) {                                                        \
     case XRS_F32: { using T = float; __VA_ARGS__; break; }                  \

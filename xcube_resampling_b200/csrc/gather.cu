@@ -2,7 +2,8 @@
 //
 //   xrs_gather_ij   rectify.py:579-734 (_compute_var_image* / _for_dest_line)
 //
-// Two kernels share the per-pixel arithmetic (fp64, no FMA contraction, one C cast):
+// Two kernels share the per-pixel arithmetic (fp64, no FMA contraction, one cast with x86's results,
+// xrs_casts.h):
 //   * k2_gather_staged: one CTA per 32x32 target tile.  The CTA reduces the bounding box of the
 //     source pixels its ij values reach and pulls that box of every band into shared memory with
 //     TMA tensor copies (cp.async.bulk.tensor.2d, one 64x48 box per band, 4-stage mbarrier ring),
@@ -65,7 +66,7 @@ k2_gather_direct(PlaneTable<T> planes, int n_bands, int64_t src_h, int64_t src_w
     const int64_t o10 = o00 + (t.j1 - t.j0) * src_pitch, o11 = o10 + (t.i1 - t.i0);
     if (METHOD == XRS_NEAREST) {
 #pragma unroll 8
-        for (int b = 0; b < n_bands; ++b) st_stream(planes.dst[b] + o, __ldg(planes.src[b] + o00));
+        for (int b = 0; b < n_bands; ++b) st_stream(planes.dst[b] + o, nearest_value(__ldg(planes.src[b] + o00)));
         return;
     }
 #pragma unroll 4
@@ -73,7 +74,7 @@ k2_gather_direct(PlaneTable<T> planes, int n_bands, int64_t src_h, int64_t src_w
         const T *sp = planes.src[b];
         const double val = interp_value<METHOD>(ld_f64(sp + o00), ld_f64(sp + o01), ld_f64(sp + o10), ld_f64(sp + o11),
                                                 t.u, t.v);
-        st_stream(planes.dst[b] + o, cast_from_f64<T>(val));
+        st_stream(planes.dst[b] + o, cast_like_numpy<T>(val));
     }
 }
 
@@ -206,13 +207,13 @@ k2_gather_staged(const __grid_constant__ StagedParams<T> p, int n_bands, int64_t
 #pragma unroll
                 for (int k = 0; k < K2S_PX; ++k) {
                     if (METHOD == XRS_NEAREST) {
-                        out[k] = t00[k][s * STAGE_ELEMS];
+                        out[k] = nearest_value(t00[k][s * STAGE_ELEMS]);
                     } else {
                         const double v00 = static_cast<double>(t00[k][s * STAGE_ELEMS]);
                         const double v01 = static_cast<double>(t01[k][s * STAGE_ELEMS]);
                         const double v10 = static_cast<double>(t10[k][s * STAGE_ELEMS]);
                         const double v11 = static_cast<double>(t11[k][s * STAGE_ELEMS]);
-                        out[k] = cast_from_f64<T>(interp_value<METHOD>(v00, v01, v10, v11, t[k].u, t[k].v));
+                        out[k] = cast_like_numpy<T>(interp_value<METHOD>(v00, v01, v10, v11, t[k].u, t[k].v));
                     }
                     out[k] = t[k].valid ? out[k] : fill;
                 }
@@ -248,11 +249,11 @@ k2_gather_staged(const __grid_constant__ StagedParams<T> p, int n_bands, int64_t
             if (!t[k].valid) {
                 out[k] = fill;
             } else if (METHOD == XRS_NEAREST) {
-                out[k] = __ldg(sp + o00[k]);
+                out[k] = nearest_value(__ldg(sp + o00[k]));
             } else {
-                out[k] = cast_from_f64<T>(interp_value<METHOD>(ld_f64(sp + o00[k]), ld_f64(sp + o00[k] + od[k]),
-                                                               ld_f64(sp + o00[k] + oj[k]),
-                                                               ld_f64(sp + o00[k] + oj[k] + od[k]), t[k].u, t[k].v));
+                out[k] = cast_like_numpy<T>(interp_value<METHOD>(ld_f64(sp + o00[k]), ld_f64(sp + o00[k] + od[k]),
+                                                                ld_f64(sp + o00[k] + oj[k]),
+                                                                ld_f64(sp + o00[k] + oj[k] + od[k]), t[k].u, t[k].v));
             }
         }
 #pragma unroll

@@ -67,10 +67,13 @@ constexpr int K2S_ROW_STEP = K2S_THREADS / K2S_TW;
 constexpr int K2S_BOX_W = 64, K2S_BOX_H = 48;
 constexpr int K2S_STAGES = 4;
 
+// A nearest sample as the reference stores it: it casts the source window to float64 (rectify.py:628-630) and
+// assigns the float64 value back (rectify.py:734).  The round trip is the identity for every type but int64,
+// whose values beyond 2^53 it rounds (and INT64_MAX, rounded up to 2^63, turns into INT64_MIN).
 template <typename T>
-static T cast_fill(double fill) {
-    if (std::is_floating_point<T>::value) return static_cast<T>(fill);
-    return static_cast<T>(static_cast<long long>(fill));
+__device__ __forceinline__ T nearest_value(T v) {
+    if constexpr (std::is_same<T, int64_t>::value) return cast_like_numpy<T>(static_cast<double>(v));
+    else return v;
 }
 
 }  // namespace xrs

@@ -161,8 +161,8 @@ k2_gather_dual(const __grid_constant__ DualParams<T> p, int n_bands, int64_t src
                 for (int k = 0; k < K2S_PX; ++k) {
                     const T r00 = t00[k][s * STAGE_ELEMS], r01 = t01[k][s * STAGE_ELEMS];
                     const T r10 = t10[k][s * STAGE_ELEMS], r11 = t11[k][s * STAGE_ELEMS];
-                    const T near = pick_tap(r00, r01, r10, r11, (near_sel >> (2 * k)) & 1u, (near_sel >> (2 * k + 1)) & 1u);
-                    const T val = cast_from_f64<T>(interp_value<METHOD>(
+                    const T near = nearest_value(pick_tap(r00, r01, r10, r11, (near_sel >> (2 * k)) & 1u, (near_sel >> (2 * k + 1)) & 1u));
+                    const T val = cast_like_numpy<T>(interp_value<METHOD>(
                         static_cast<double>(r00), static_cast<double>(r01), static_cast<double>(r10),
                         static_cast<double>(r11), t[k].u, t[k].v));
                     out_i[k] = t[k].valid ? val : fill_interp;
@@ -205,8 +205,8 @@ k2_gather_dual(const __grid_constant__ DualParams<T> p, int n_bands, int64_t src
             if (t[k].valid) {
                 const T r00 = __ldg(sp + o00[k]), r01 = __ldg(sp + o00[k] + od[k]);
                 const T r10 = __ldg(sp + o00[k] + oj[k]), r11 = __ldg(sp + o00[k] + oj[k] + od[k]);
-                out_n[k] = pick_tap(r00, r01, r10, r11, (near_sel >> (2 * k)) & 1u, (near_sel >> (2 * k + 1)) & 1u);
-                out_i[k] = cast_from_f64<T>(interp_value<METHOD>(
+                out_n[k] = nearest_value(pick_tap(r00, r01, r10, r11, (near_sel >> (2 * k)) & 1u, (near_sel >> (2 * k + 1)) & 1u));
+                out_i[k] = cast_like_numpy<T>(interp_value<METHOD>(
                     static_cast<double>(r00), static_cast<double>(r01), static_cast<double>(r10),
                     static_cast<double>(r11), t[k].u, t[k].v));
             }

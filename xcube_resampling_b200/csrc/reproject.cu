@@ -216,25 +216,8 @@ __device__ __forceinline__ double diff_as_f64(T a, T b) {
     }
 }
 
-// float64 -> integer the way numpy's astype does it on x86-64 (reproject.py:299-300 assigns float64
-// results into an array of the source dtype): types up to 32 bits go through a 32-bit cvttsd2si
-// (uint32 through the 64-bit one), whose out-of-range / NaN result is the "integer indefinite"
-// value 0x80000000 (0x8000000000000000), and are then truncated to the destination width.
-template <typename OUT>
-__device__ __forceinline__ OUT cast_like_numpy(double v) {
-    if constexpr (std::is_floating_point<OUT>::value) {
-        return static_cast<OUT>(v);
-    } else if constexpr (sizeof(OUT) == 8 || std::is_same<OUT, uint32_t>::value) {
-        const bool ok = v > -9223372036854775809.0 && v < 9223372036854775808.0;
-        const long long w = ok ? static_cast<long long>(v) : static_cast<long long>(0x8000000000000000ull);
-        return static_cast<OUT>(w);
-    } else {
-        const bool ok = v > -2147483649.0 && v < 2147483648.0;
-        const int w = ok ? static_cast<int>(v) : static_cast<int>(0x80000000u);
-        return static_cast<OUT>(w);
-    }
-}
-
+// (reproject.py:299-300 assigns the float64 results into an array of the source dtype: cast_like_numpy,
+// xrs_casts.h)
 template <typename T, typename OUT>
 __device__ __forceinline__ OUT k3_store_cast(double v) {
     if constexpr (std::is_same<OUT, double>::value) return v;
@@ -1272,9 +1255,7 @@ int launch_reproject(const K3Geom &g_in, const void *const *src_planes, void *co
     const dim3 grid(static_cast<unsigned>(ceil_div(g.dst_w, K3T_COLS)),
                     static_cast<unsigned>(ceil_div(g.row_end - g.row_tile0, K3T_ROWS)));
     if (grid.y > 65535) return fail("xrs_reproject: more than 2097120 target rows per call");
-    T fill_t;
-    if constexpr (std::is_floating_point<T>::value) fill_t = static_cast<T>(fill);
-    else fill_t = static_cast<T>(static_cast<long long>(fill));
+    const T fill_t = cast_fill<T>(fill);
     // XRS_K3_EXACT=1 makes every pixel evaluate the full projection formulas (the tests compare the
     // lattice form with it)
     const char *exact_env = getenv("XRS_K3_EXACT");
