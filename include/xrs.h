@@ -333,6 +333,75 @@ int xrs_affine_recover(const void *src, double *dst, int32_t dtype, int64_t n_sl
 int xrs_coarsen(const void *src, void *dst, int32_t dtype, int64_t n_slices, int64_t src_h, int64_t src_w,
                 int64_t src_pitch, int64_t src_slice_stride, int32_t agg, int32_t f_j, int32_t f_i, void *stream);
 
+/* ------------------------------------------------------------------------
+ * Compressed Zarr-v2 chunks decoded on the device (io.py, the I/O edge)
+ * --------------------------------------------------------------------- */
+
+/* codec of one chunk file: missing (the array's fill value), a Blosc-1 frame with an LZ4 / LZ4HC inner
+ * codec (numcodecs Blosc, byte shuffle or none, or a frame stored whole), or numcodecs' lz4 (int32 decoded
+ * size, then one LZ4 block) */
+enum xrs_chunk_codec { XRS_CHUNK_MISSING = 0, XRS_CHUNK_BLOSC = 1, XRS_CHUNK_LZ4 = 2 };
+
+/* One chunk file of a xrs_zarr_decode call (80 bytes). */
+typedef struct xrs_zarr_chunk {
+    int64_t offset;       /* first byte of the file in `data` */
+    int64_t length;       /* bytes of the file (0 when missing) */
+    int64_t band, row, col; /* array index of the chunk's element (0, 0, 0); band 0 for 2-D arrays */
+    int32_t codec;        /* enum xrs_chunk_codec */
+    int32_t n_streams;    /* filled by the call */
+    int64_t stream_base;  /* filled by the call */
+    int64_t scratch;      /* filled by the call: where the decoded chunk goes in the workspace, -1 when missing */
+    uint8_t header[16];   /* the first 16 bytes of the file (Blosc header; lz4: the size prefix) */
+} xrs_zarr_chunk;
+
+/* CF mask-and-scale of the decoded values (io.DecodedSource): the stored value is converted to out_dtype,
+ * values equal to one of `fills` become NaN, then * scale (if has_scale), then + offset (if has_offset), each
+ * rounded once in out_dtype -- numpy's steps in numpy's order. */
+#define XRS_ZARR_CF_MAX_FILLS 16
+typedef struct xrs_zarr_cf {
+    int32_t out_dtype;    /* XRS_F32 or XRS_F64 */
+    int32_t n_fills;      /* <= XRS_ZARR_CF_MAX_FILLS */
+    int32_t has_scale, has_offset;
+    double scale, offset;
+    uint64_t fills[XRS_ZARR_CF_MAX_FILLS]; /* stored-dtype values, native byte order, in the low bytes */
+} xrs_zarr_cf;
+
+/* reasons in bits 24-31 of the error word; bits 0-23 hold 1 + the index of the bad chunk in the table */
+enum xrs_decode_error {
+    XRS_DECODE_BAD_LAYOUT = 1,          /* a block offset or stream size points outside the file */
+    XRS_DECODE_OFFSET_ZERO = 2,         /* an LZ4 match offset of 0 */
+    XRS_DECODE_OFFSET_BEFORE_START = 3, /* a match reaching before the stream's first decoded byte */
+    XRS_DECODE_LITERALS_OVERRUN = 4,    /* literals past the decoded size or past the input */
+    XRS_DECODE_MATCH_OVERRUN = 5,       /* a match past the decoded size */
+    XRS_DECODE_INPUT_OVERRUN = 6,       /* length extension, offset or next token past the input */
+    XRS_DECODE_SHORT = 7                /* the stream ends short of its decoded size */
+};
+
+/* Decode whole chunk files and place their elements into a pitched (bands, rows, width) slot.
+ *   data, data_bytes   the chunk files, concatenated as read from the store
+ *   chunks_host        HOST table of n_chunks < 2^24 files (page-locked memory keeps the call asynchronous); the
+ *                      call checks each header and fills stream_base / n_streams / scratch, then copies the table to the
+ *                      workspace on `stream`: it must stay unchanged until the stream has passed the call
+ *   chunk_bands/h/w    chunk shape (chunk_bands 1 for 2-D arrays); dtype: the stored type, big_endian 1 for
+ *                      ">" dtypes (values are byte-swapped to native order)
+ *   fill_bits          the stored value of a missing chunk, native byte order in the low bytes
+ *   cf_host            NULL (values as stored, dst of `dtype`) or CF decoding (dst of cf_host->out_dtype)
+ *   img_h, img_w       array height and width: ragged edge chunks are clipped to them
+ *   dst                element (band b0, row win_j0, column 0) of the slot; pitch and band stride in elements;
+ *                      only rows [win_j0, win_j1) and bands [b0, b0 + nb) are written
+ *   workspace          xrs_zarr_decode_workspace_bytes(...) bytes, 256-byte aligned: the table, 32 bytes a stream and
+ *                      one decoded chunk per file present
+ *   error_word         device uint32, 0 before the first call; a malformed stream stores its reason and
+ *                      chunk there (the first one recorded wins) and the call's results are undefined.  A file
+ *                      the call can reject from its header alone fails the call itself, naming the chunk. */
+int64_t xrs_zarr_decode_workspace_bytes(xrs_zarr_chunk *chunks_host, int64_t n_chunks, int64_t chunk_bands,
+                                        int64_t chunk_h, int64_t chunk_w, int32_t dtype);
+int xrs_zarr_decode(const void *data, int64_t data_bytes, xrs_zarr_chunk *chunks_host, int64_t n_chunks,
+                    int64_t chunk_bands, int64_t chunk_h, int64_t chunk_w, int32_t dtype, int32_t big_endian,
+                    uint64_t fill_bits, const xrs_zarr_cf *cf_host, int64_t img_h, int64_t img_w, void *dst,
+                    int64_t dst_pitch, int64_t dst_band_stride, int64_t win_j0, int64_t win_j1, int64_t b0, int64_t nb,
+                    void *workspace, int64_t workspace_bytes, uint32_t *error_word, void *stream);
+
 #ifdef __cplusplus
 }
 #include "xrs_casts.h" /* the conversions behind `fill` and the integer stores above, as C++ templates */

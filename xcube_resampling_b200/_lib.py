@@ -37,6 +37,22 @@ class XrsProj(ctypes.Structure):
         return cls(kind, 0, a, inv_f, lon0, lat0, k0, fe, fn)
 
 
+class XrsZarrCF(ctypes.Structure):
+    """``struct xrs_zarr_cf`` of include/xrs.h."""
+
+    MAX_FILLS = 16
+    _fields_ = [("out_dtype", c_i32), ("n_fills", c_i32), ("has_scale", c_i32), ("has_offset", c_i32),
+                ("scale", c_f64), ("offset", c_f64), ("fills", ctypes.c_uint64 * MAX_FILLS)]
+
+    @classmethod
+    def from_params(cls, out_dtype: int, fills, scale, offset) -> "XrsZarrCF":
+        """``fills``: numpy array of the stored type; ``scale`` / ``offset``: ``None`` when absent."""
+        cf = cls(out_dtype, len(fills), scale is not None, offset is not None, scale or 0.0, offset or 0.0)
+        for k, f in enumerate(fills):
+            cf.fills[k] = int.from_bytes(f.tobytes(), "little")
+        return cf
+
+
 # name -> (restype, argtypes); must list every symbol of include/xrs.h
 SIGNATURES = {
     "xrs_version": (c_int, []),
@@ -78,6 +94,9 @@ SIGNATURES = {
     "xrs_affine_recover": (c_int, [c_p, c_p, c_i32, c_i64, c_i64, c_i64, c_i64, c_i64, c_i64, c_i64, c_f64, c_f64, c_f64,
                                    c_f64, c_f64, c_i32, c_i32, c_i32, c_i32, c_p]),
     "xrs_coarsen": (c_int, [c_p, c_p, c_i32, c_i64, c_i64, c_i64, c_i64, c_i64, c_i32, c_i32, c_i32, c_p]),
+    "xrs_zarr_decode_workspace_bytes": (c_i64, [c_p, c_i64, c_i64, c_i64, c_i64, c_i32]),
+    "xrs_zarr_decode": (c_int, [c_p, c_i64, c_p, c_i64, c_i64, c_i64, c_i64, c_i32, c_i32, ctypes.c_uint64, c_p, c_i64,
+                                c_i64, c_p, c_i64, c_i64, c_i64, c_i64, c_i64, c_i64, c_p, c_i64, c_p, c_p]),
 }
 
 _lock = threading.Lock()

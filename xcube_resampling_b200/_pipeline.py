@@ -29,7 +29,7 @@ import numpy as np
 import torch
 
 from . import _dev
-from ._lib import check, load
+from ._lib import XrsError, check, load
 
 
 @dataclass
@@ -124,6 +124,59 @@ def copy2d(dst_addr: int, dst_pitch: int, dst_slice: int, src_addr: int, src_pit
           "xrs_copy2d_slices")
 
 
+def _zarr_geometry(source):
+    """(stored ZarrV2Source, chunk (bands, h, w), dtype code, big-endian flag, CF struct or None) of a source with a
+    device read (``io.ZarrV2Source`` or ``io.DecodedSource`` over one)."""
+    from .constants import DTYPE_CODES
+    from ._lib import XrsZarrCF
+
+    stored = getattr(source, "source", source)
+    raw = np.dtype(stored.dtype)
+    chunk = tuple(stored.chunks) if len(stored.chunks) == 3 else (1,) + tuple(stored.chunks)
+    cf = None
+    if stored is not source:
+        p = source.device_cf()
+        cf = XrsZarrCF.from_params(DTYPE_CODES[np.dtype(p["out_dtype"])], p["fills"], p["scale"], p["offset"])
+    return stored, chunk, DTYPE_CODES[raw.newbyteorder("=")], int(raw.byteorder == ">"), cf
+
+
+def zarr_workspace_bytes(lib, source, table) -> int:
+    """``xrs_zarr_decode_workspace_bytes`` for the chunk table of a device read of ``source``."""
+    _, (cb, ch, cw), code, _, _ = _zarr_geometry(source)
+    n = lib.xrs_zarr_decode_workspace_bytes(ctypes.c_void_p(table.ctypes.data), len(table), cb, ch, cw, code)
+    if n < 0:
+        check(1, "xrs_zarr_decode_workspace_bytes")
+    return int(n)
+
+
+def zarr_decode(lib, source, data_addr: int, n_bytes: int, table, dst_addr: int, pitch: int, band_stride: int,
+                window, b0: int, nb: int, ws_addr: int, ws_bytes: int, err_addr: int, stream) -> int:
+    """``xrs_zarr_decode`` of a device read of ``source`` (``lib``: libxrs or a host build with the same ABI);
+    returns the status."""
+    stored, (cb, ch, cw), code, big, cf = _zarr_geometry(source)
+    h, w = stored.shape[-2:]
+    return lib.xrs_zarr_decode(ctypes.c_void_p(data_addr), n_bytes, ctypes.c_void_p(table.ctypes.data), len(table),
+                               cb, ch, cw, code, big, stored.device_fill_bits(),
+                               None if cf is None else ctypes.byref(cf), h, w, ctypes.c_void_p(dst_addr), pitch,
+                               band_stride, int(window[0]), int(window[1]), b0, nb, ctypes.c_void_p(ws_addr), ws_bytes,
+                               ctypes.c_void_p(err_addr), stream)
+
+
+DECODE_ERRORS = {1: "a block offset or stream size points outside the file", 2: "an LZ4 match offset of 0",
+                 3: "an LZ4 match reaching before the stream's start", 4: "LZ4 literals past the decoded size",
+                 5: "an LZ4 match past the decoded size", 6: "the LZ4 stream ends inside a sequence",
+                 7: "the LZ4 stream ends short of its decoded size"}
+
+
+def decode_error(word: int, paths) -> str | None:
+    """The message for an ``xrs_zarr_decode`` error word (``paths``: the chunk files of that call)."""
+    if word == 0:
+        return None
+    chunk = (word & 0xFFFFFF) - 1
+    where = paths[chunk] if 0 <= chunk < len(paths) else f"chunk {chunk}"
+    return f"{where}: malformed chunk file: {DECODE_ERRORS.get(word >> 24, f'error {word >> 24}')}"
+
+
 class GatherPipeline:
     """Three-stream pipeline over the band chunks of a list of :class:`SourceGroup`.
 
@@ -150,6 +203,7 @@ class GatherPipeline:
         self.d2h_bytes = 0
         self._pending = None
         self._keep = None
+        self._decode_checks = []  # (error words, chunk file paths per band chunk) of device-decoded sources
 
     def _slots(self, cache, key, shape, dtype, n=2):
         if key not in cache or len(cache[key]) < n:
@@ -161,8 +215,14 @@ class GatherPipeline:
         if self._pending is not None:
             s_out, main = self._pending
             s_out.synchronize()
-            main.synchronize()
+            main.synchronize()  # main waited for every decode on s_in
             self._pending = None
+        checks, self._decode_checks = self._decode_checks, []
+        for errs, paths_of in checks:
+            for word, paths in zip(errs.cpu().tolist(), paths_of):
+                msg = decode_error(word & 0xFFFFFFFF, paths)
+                if msg:
+                    raise XrsError(msg)
 
     def run(self, groups: list[SourceGroup], process, wait: bool = True, process_pair=None) -> None:
         """Enqueue uploads, kernels and downloads of every band chunk; ``wait=False`` returns as soon as
@@ -190,7 +250,8 @@ class GatherPipeline:
         for grp in groups:
             v = grp.values
             lazy = hasattr(v, "read_bands")
-            dtype = np.dtype(v.dtype)
+            on_device = lazy and getattr(v, "device_decodable", False)  # compressed chunks decode on the device
+            dtype = np.dtype(v.dtype).newbyteorder("=") if on_device else np.dtype(v.dtype)
             bands = (1 if v.ndim == 2 else v.shape[0]) if lazy else v.shape[0]
             h, w = v.shape[-2:]
             if (h, w) != (self.h, self.w):
@@ -201,7 +262,23 @@ class GatherPipeline:
             chunk = max(1, min(self.chunk, bands))
             in_slots = self._slots(self._in_slots, (dtype.str, chunk), (chunk, win_h, wp), dtype)
             schedule = chunk_schedule(bands, chunk)
-            if lazy:
+            if on_device:
+                # the chunk files of band chunk k+1 are read into one of two page-locked byte buffers on a reader
+                # thread while chunk k's files are uploaded and decoded into its slot (xrs_zarr_decode)
+                from concurrent.futures import ThreadPoolExecutor
+
+                lib = load()
+                files = [None, None]
+                stage_done = [None, None]
+                reader = ThreadPoolExecutor(max_workers=1)
+                pending = reader.submit(v.device_read, schedule[0][0], schedule[0][1], self.segments, self.win)
+                with torch.cuda.stream(s_in):
+                    errs = torch.zeros(len(schedule), dtype=torch.int32, device=dev)
+                dev_bytes = ws = None
+                paths_of = []
+                self._decode_checks.append((errs, paths_of))
+                keep.append(files)
+            elif lazy:
                 # the I/O edge: band chunk k+1 is read from the store into one of two page-locked staging
                 # buffers on a reader thread while chunk k is copied to the device
                 from concurrent.futures import ThreadPoolExecutor
@@ -215,7 +292,17 @@ class GatherPipeline:
                 base = v.__array_interface__["data"][0]
                 sb, sr = v.strides[0], v.strides[1]
             for ci, (b0, nb) in enumerate(schedule):
-                if lazy:
+                if on_device:
+                    files[ci % 2] = pending.result()
+                    buf, n_bytes, table, paths = files[ci % 2]
+                    paths_of.append(paths)
+                    if ci + 1 < len(schedule):
+                        if stage_done[(ci + 1) % 2] is not None:
+                            stage_done[(ci + 1) % 2].synchronize()  # its previous decode has left the buffer
+                        prev = files[(ci + 1) % 2]
+                        pending = reader.submit(v.device_read, schedule[ci + 1][0], schedule[ci + 1][1], self.segments,
+                                                self.win, None if prev is None else prev[0])
+                elif lazy:
                     pending.result()
                     base, sb, sr = stage[ci % 2].__array_interface__["data"][0], h * w * isz, w * isz
                     if ci + 1 < len(schedule):
@@ -229,10 +316,26 @@ class GatherPipeline:
                 src_slot = in_slots[slot]
                 with torch.cuda.stream(s_in):
                     s_in.wait_event(in_free[slot])
-                    for (j0, j1, i0, i1) in self.segments:
-                        copy2d(src_slot.data_ptr() + ((j0 - self.win[0]) * wp + i0) * isz, wp * isz, win_h * wp * isz,
-                               base + b_off * sb + j0 * sr + i0 * isz, sr, sb, (i1 - i0) * isz, j1 - j0, nb, dev)
-                        self.h2d_bytes += (i1 - i0) * isz * (j1 - j0) * nb
+                    if on_device:
+                        ws_bytes = zarr_workspace_bytes(lib, v, table)
+                        if dev_bytes is None or dev_bytes.numel() < n_bytes:
+                            dev_bytes = torch.empty(max(n_bytes + (n_bytes >> 3), 1 << 20), dtype=torch.uint8, device=dev)
+                        if ws is None or ws.numel() < ws_bytes:
+                            ws = torch.empty(max(ws_bytes + (ws_bytes >> 3), 1 << 20), dtype=torch.uint8, device=dev)
+                        if n_bytes:
+                            copy2d(dev_bytes.data_ptr(), n_bytes, n_bytes, buf.ctypes.data, n_bytes, n_bytes, n_bytes, 1,
+                                   1, dev)
+                        check(zarr_decode(lib, v, dev_bytes.data_ptr(), n_bytes, table, src_slot.data_ptr(), wp,
+                                          win_h * wp, self.win, b0, nb, ws.data_ptr(), ws.numel(),
+                                          errs.data_ptr() + 4 * ci, _dev.stream_ptr(dev)), "xrs_zarr_decode")
+                        self.h2d_bytes += n_bytes
+                        keep.append((dev_bytes, ws))
+                    else:
+                        for (j0, j1, i0, i1) in self.segments:
+                            copy2d(src_slot.data_ptr() + ((j0 - self.win[0]) * wp + i0) * isz, wp * isz,
+                                   win_h * wp * isz, base + b_off * sb + j0 * sr + i0 * isz, sr, sb, (i1 - i0) * isz,
+                                   j1 - j0, nb, dev)
+                            self.h2d_bytes += (i1 - i0) * isz * (j1 - j0) * nb
                     ready = torch.cuda.Event()
                     ready.record(s_in)
                 if lazy:

@@ -36,6 +36,7 @@ SOURCES = {
     "resample.cu": ["-fmad=false"],
     "resample_fast.cu": ["-fmad=false"],
     "reproject.cu": [],  # projection math may contract; the numpy-parity part uses _rn intrinsics
+    "decode.cu": [],  # CF scaling uses _rn intrinsics
 }
 
 

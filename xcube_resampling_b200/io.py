@@ -17,6 +17,10 @@ Stores understood without third-party packages:
   Zlib / Zstd inner codec, byte shuffle or none: :func:`blosc_decompress`), decoded on the reader thread.
   BloscLZ or bit-shuffled Blosc frames and Zarr filters need the ``zarr`` / ``numcodecs`` packages, which
   this build does not have; open such stores with xarray and pass the arrays instead.
+  Blosc-LZ4 / LZ4HC stores (byte shuffle or none) and numcodecs ``lz4`` stores are not decoded on the host in the
+  band pipeline: their chunk files are read as they are (:meth:`ZarrV2Source.device_read`), uploaded compressed and
+  decoded, unshuffled and CF-unpacked on the device (``xrs_zarr_decode``, ``csrc/decode.cu``).  ``read_bands`` stays
+  the host decode, for ``values`` / ``read_all`` and every other codec.
 * :class:`NpySource` -- a ``.npy`` file, memory-mapped.
 * :class:`NetCDF3Source` -- a variable of a NetCDF classic / 64-bit-offset file (CDF-1 / CDF-2), memory-mapped
   through ``scipy.io.netcdf_file``; its big-endian values are byte-swapped by the copy into the staging
@@ -257,9 +261,57 @@ class NetCDF3Source(LazySource):
         out[:nb] = (data[None] if data.ndim == 2 else data)[b0:b0 + nb]
 
 
+# one chunk file of a device read: ``struct xrs_zarr_chunk`` of include/xrs.h
+CHUNK_TABLE_DTYPE = np.dtype([("offset", "<i8"), ("length", "<i8"), ("band", "<i8"), ("row", "<i8"), ("col", "<i8"),
+                              ("codec", "<i4"), ("n_streams", "<i4"), ("stream_base", "<i8"), ("scratch", "<i8"),
+                              ("header", "u1", 16)])
+assert CHUNK_TABLE_DTYPE.itemsize == 80
+CHUNK_MISSING, CHUNK_BLOSC, CHUNK_LZ4 = 0, 1, 2  # enum xrs_chunk_codec
+
+
+def _device_codec(compressor: dict | None) -> int | None:
+    """The codec of ``xrs_zarr_decode`` a ``.zarray`` compressor maps to, ``None`` when chunks decode on the host."""
+    if not compressor:
+        return None
+    if compressor.get("id") == "lz4":
+        return CHUNK_LZ4
+    if compressor.get("id") == "blosc" and compressor.get("cname") in ("lz4", "lz4hc") and \
+            compressor.get("shuffle", 1) in (0, 1):
+        return CHUNK_BLOSC
+    return None
+
+
+def _check_device_header(path: str, codec: int, head: bytes, size: int, chunk_bytes: int) -> None:
+    """The checks :func:`blosc_decompress` / the numcodecs lz4 decoder make before decoding, on a file's header
+    only, with the same errors; the device decode checks the streams."""
+    if codec == CHUNK_LZ4:
+        if size < 4 or int.from_bytes(head[:4], "little", signed=True) != chunk_bytes:
+            raise ValueError(f"{path}: the lz4 chunk's size prefix does not match the chunk size {chunk_bytes}")
+        return
+    if size < 16:
+        raise ValueError(f"{path}: not a Blosc frame: shorter than its 16-byte header")
+    version, flags = head[0], head[2]
+    nbytes, blocksize, cbytes = (int.from_bytes(head[k:k + 4], "little") for k in (4, 8, 12))
+    if version != 2 or cbytes > size or (nbytes and blocksize == 0):
+        raise ValueError(f"{path}: not a Blosc-1 frame (version {version}, cbytes {cbytes} of {size} bytes)")
+    if nbytes != chunk_bytes:
+        raise ValueError(f"{path}: the Blosc frame holds {nbytes} bytes, the chunk {chunk_bytes}")
+    if flags & 0x2:
+        if 16 + nbytes > size:
+            raise ValueError(f"{path}: truncated Blosc frame")
+        return
+    if flags & 0x4:
+        raise NotImplementedError("bit-shuffled Blosc frames need the zarr / blosc packages, which this build does "
+                                  "not have")
+    if flags >> 5 != 1:
+        _blosc_stream_decoder(flags >> 5)  # BloscLZ: the host path's error
+        raise ValueError(f"{path}: the Blosc frame's inner codec ({flags >> 5}) is not the store's LZ4")
+
+
 class ZarrV2Source(LazySource):
     """One Zarr-v2 array of a directory store (2-D or 3-D, C order; uncompressed or with a codec of
-    :func:`chunk_decoder`)."""
+    :func:`chunk_decoder`).  Blosc-LZ4 / LZ4HC (byte shuffle or none) and numcodecs ``lz4`` stores can also be
+    read for the device (:meth:`device_read`): the band pipeline then decodes the chunks there."""
 
     def __init__(self, path: str):
         meta = json.load(open(os.path.join(path, ".zarray")))
@@ -284,6 +336,63 @@ class ZarrV2Source(LazySource):
         self.sep = meta.get("dimension_separator", ".")
         attrs_path = os.path.join(path, ".zattrs")
         self.attrs = json.load(open(attrs_path)) if os.path.isfile(attrs_path) else {}
+        self.device_codec = _device_codec(meta.get("compressor"))
+
+    @property
+    def device_decodable(self) -> bool:
+        """Whether :meth:`device_read` applies: the store's compressor is one ``xrs_zarr_decode`` decodes."""
+        return self.device_codec is not None
+
+    def device_fill_bits(self) -> int:
+        """The stored value of a missing chunk (what :meth:`_chunk` fills in), native byte order, as an integer."""
+        v = np.full(1, _fill_value(self.fill, self.dtype), dtype=self.dtype.newbyteorder("="))
+        return int.from_bytes(v.tobytes(), "little")
+
+    def device_read(self, b0: int, nb: int, segments, window, buffer=None):
+        """The chunk files behind bands ``b0 : b0 + nb`` of the (j0, j1, i0, i1) ``segments`` inside the row
+        ``window``, read as they are on disk into a page-locked byte buffer, followed by their chunk table
+        (:data:`CHUNK_TABLE_DTYPE`).  Only each file's header is checked here.  ``buffer`` (the previous
+        result's) is reused when it is large enough.  Returns ``(buffer, n_file_bytes, table, paths)``."""
+        from . import _dev
+
+        three_d = len(self.shape) == 3
+        cb = self.chunks[0] if three_d else 1
+        ch, cw = self.chunks[-2:]
+        chunk_bytes = int(np.prod(self.chunks)) * self.dtype.itemsize
+        tiles = set()
+        for (j0, j1, i0, i1) in segments:
+            j0, j1 = max(j0, window[0]), min(j1, window[1])
+            if j0 >= j1 or i0 >= i1:
+                continue
+            tiles.update((kj, ki) for kj in range(j0 // ch, -(-j1 // ch)) for ki in range(i0 // cw, -(-i1 // cw)))
+        keys = [(kb, kj, ki) for kb in range(b0 // cb, -(-(b0 + nb) // cb)) for (kj, ki) in sorted(tiles)]
+        paths = [os.path.join(self.path, self.sep.join(str(i) for i in ((kb, kj, ki) if three_d else (kj, ki))))
+                 for (kb, kj, ki) in keys]
+        sizes = [os.path.getsize(p) if os.path.isfile(p) else -1 for p in paths]
+        n_bytes = sum(max(s, 0) for s in sizes)
+        table_at = -(-n_bytes // 8) * 8
+        need = table_at + len(keys) * CHUNK_TABLE_DTYPE.itemsize
+        if buffer is None or buffer.nbytes < need:
+            buffer = _dev.pinned_empty((max(need, 1 << 20) + (need >> 3),), np.uint8)  # an eighth to grow into
+        table = buffer[table_at:need].view(CHUNK_TABLE_DTYPE)
+        table[...] = 0
+        pos = 0
+        for k, ((kb, kj, ki), p, size) in enumerate(zip(keys, paths, sizes)):
+            t = table[k]
+            t["band"], t["row"], t["col"] = kb * cb, kj * ch, ki * cw
+            if size < 0:  # a missing chunk is all fill value
+                t["codec"] = CHUNK_MISSING
+                continue
+            with open(p, "rb") as fh:
+                got = fh.readinto(memoryview(buffer[pos:pos + size]))
+            if got != size:
+                raise ValueError(f"{p}: short read ({got} of {size} bytes)")
+            head = buffer[pos:pos + min(size, 16)].tobytes()
+            _check_device_header(p, self.device_codec, head, size, chunk_bytes)
+            t["offset"], t["length"], t["codec"] = pos, size, self.device_codec
+            t["header"][:len(head)] = np.frombuffer(head, np.uint8)
+            pos += size
+        return buffer, n_bytes, table, paths
 
     def _chunk(self, idx):
         p = os.path.join(self.path, self.sep.join(str(i) for i in idx))
@@ -342,6 +451,30 @@ class DecodedSource(LazySource):
                 if f == f and (source.dtype.kind == "f" or float(f).is_integer()):
                     self._fills.append(f)
         self._scale, self._offset = attrs.get("scale_factor"), attrs.get("add_offset")
+
+    def _raw_fills(self) -> np.ndarray:
+        """The fill values :meth:`read_bands` masks, as values of the stored type (native byte order)."""
+        raw = np.dtype(self.source.dtype).newbyteorder("=")
+        keep = [f for f in self._fills if raw.kind == "f" or np.iinfo(raw).min <= f <= np.iinfo(raw).max]
+        with np.errstate(over="ignore"):
+            return np.array([raw.type(f) for f in keep], dtype=raw)
+
+    @property
+    def device_decodable(self) -> bool:
+        return bool(getattr(self.source, "device_decodable", False)) and len(self._raw_fills()) <= 16
+
+    def device_read(self, b0, nb, segments, window, buffer=None):
+        """The stored chunk files, as :meth:`ZarrV2Source.device_read`; :meth:`device_cf` gives the decoding."""
+        return self.source.device_read(b0, nb, segments, window, buffer)
+
+    def device_fill_bits(self) -> int:
+        return self.source.device_fill_bits()
+
+    def device_cf(self) -> dict:
+        """What ``xrs_zarr_decode`` needs to apply this decoding: decoded dtype, fills (stored type), scale, offset."""
+        return {"out_dtype": self.dtype, "fills": self._raw_fills(),
+                "scale": None if self._scale is None else float(self._scale),
+                "offset": None if self._offset is None else float(self._offset)}
 
     def read_bands(self, b0, nb, out):
         raw = np.empty((nb,) + self.shape[-2:], dtype=self.source.dtype)
