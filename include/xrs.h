@@ -337,10 +337,11 @@ int xrs_coarsen(const void *src, void *dst, int32_t dtype, int64_t n_slices, int
  * Compressed Zarr-v2 chunks decoded on the device (io.py, the I/O edge)
  * --------------------------------------------------------------------- */
 
-/* codec of one chunk file: missing (the array's fill value), a Blosc-1 frame with an LZ4 / LZ4HC inner
- * codec (numcodecs Blosc, byte shuffle or none, or a frame stored whole), or numcodecs' lz4 (int32 decoded
- * size, then one LZ4 block) */
-enum xrs_chunk_codec { XRS_CHUNK_MISSING = 0, XRS_CHUNK_BLOSC = 1, XRS_CHUNK_LZ4 = 2 };
+/* codec of one chunk file: missing (the array's fill value), a Blosc-1 frame with an LZ4 / LZ4HC or a Zstd inner
+ * codec (numcodecs Blosc, byte shuffle or none, or a frame stored whole; each stream of a Zstd frame is one zstd
+ * frame), numcodecs' lz4 (int32 decoded size, then one LZ4 block) or numcodecs' zstd (one zstd frame, RFC 8878,
+ * without a dictionary; skippable frames may follow it) */
+enum xrs_chunk_codec { XRS_CHUNK_MISSING = 0, XRS_CHUNK_BLOSC = 1, XRS_CHUNK_LZ4 = 2, XRS_CHUNK_ZSTD = 3 };
 
 /* One chunk file of a xrs_zarr_decode call (80 bytes). */
 typedef struct xrs_zarr_chunk {
@@ -351,7 +352,7 @@ typedef struct xrs_zarr_chunk {
     int32_t n_streams;    /* filled by the call */
     int64_t stream_base;  /* filled by the call */
     int64_t scratch;      /* filled by the call: where the decoded chunk goes in the workspace, -1 when missing */
-    uint8_t header[16];   /* the first 16 bytes of the file (Blosc header; lz4: the size prefix) */
+    uint8_t header[16];   /* the first 16 bytes of the file (Blosc header; lz4: the size prefix; zstd: the magic) */
 } xrs_zarr_chunk;
 
 /* CF mask-and-scale of the decoded values (io.DecodedSource): the stored value is converted to out_dtype,
@@ -373,8 +374,24 @@ enum xrs_decode_error {
     XRS_DECODE_OFFSET_BEFORE_START = 3, /* a match reaching before the stream's first decoded byte */
     XRS_DECODE_LITERALS_OVERRUN = 4,    /* literals past the decoded size or past the input */
     XRS_DECODE_MATCH_OVERRUN = 5,       /* a match past the decoded size */
-    XRS_DECODE_INPUT_OVERRUN = 6,       /* length extension, offset or next token past the input */
-    XRS_DECODE_SHORT = 7                /* the stream ends short of its decoded size */
+    XRS_DECODE_INPUT_OVERRUN = 6,       /* length extension, offset or next token past the input; zstd: a frame
+                                           header, block or checksum past the input */
+    XRS_DECODE_SHORT = 7,               /* the stream ends short of its decoded size */
+    /* zstd frames only (the reasons above apply to them too; an offset of 0 is a repeat offset of 0) */
+    XRS_DECODE_BAD_FRAME_HEADER = 8,    /* unknown magic, reserved bit set, a dictionary ID other than 0, a window
+                                           beyond 2^31 bytes, or a content size other than the stream's */
+    XRS_DECODE_BAD_BLOCK = 9,           /* reserved block type, or a compressed block above min(128 KiB, window) */
+    XRS_DECODE_BAD_LITERALS = 10,       /* a literals section past its block or above min(128 KiB, window),
+                                           treeless literals without a previous tree, or a Huffman stream that does
+                                           not decode to exactly its literals */
+    XRS_DECODE_BAD_HUFFMAN = 11,        /* a Huffman tree description that is truncated or does not form a tree */
+    XRS_DECODE_BAD_FSE = 12,            /* an FSE table description above the table's accuracy log or whose
+                                           probabilities do not sum */
+    XRS_DECODE_BAD_SEQUENCES = 13,      /* a sequences header past its block, reserved mode bits, a repeated table
+                                           without a previous one, an RLE code out of range, or a bitstream not
+                                           consumed exactly */
+    XRS_DECODE_TRAILING_BYTES = 14,     /* bytes after the frame that are not skippable frames */
+    XRS_DECODE_CHECKSUM = 15            /* the content checksum (XXH64, low 32 bits) does not match */
 };
 
 /* Decode whole chunk files and place their elements into a pitched (bands, rows, width) slot.
@@ -390,7 +407,10 @@ enum xrs_decode_error {
  *   dst                element (band b0, row win_j0, column 0) of the slot; pitch and band stride in elements;
  *                      only rows [win_j0, win_j1) and bands [b0, b0 + nb) are written
  *   workspace          xrs_zarr_decode_workspace_bytes(...) bytes, 256-byte aligned: the table, 32 bytes a stream and
- *                      one decoded chunk per file present
+ *                      one decoded chunk per file present; with Zstd streams also one literal buffer per Zstd
+ *                      stream of min(S, 128 KiB) bytes, S the largest decoded size of one Zstd stream in the call
+ *                      (a numcodecs zstd chunk; for Blosc-Zstd, blocksize / streams of a full block or the last,
+ *                      partial block), so a Blosc-Zstd call takes at most about twice the scratch of an LZ4 one
  *   error_word         device uint32, 0 before the first call; a malformed stream stores its reason and
  *                      chunk there (the first one recorded wins) and the call's results are undefined.  A file
  *                      the call can reject from its header alone fails the call itself, naming the chunk. */

@@ -1,8 +1,13 @@
-"""Store-fed rectify_dataset: Blosc-LZ4 chunks decoded on the host vs on the device (csrc/decode.cu).
+"""Store-fed rectify_dataset: compressed chunks decoded on the host vs on the device (csrc/decode.cu).
 
-Writes a seeded, OLCI-shaped scene (21 x 4091 x 4865 float32, compressible radiance-like values) as Blosc-LZ4,
-byte-shuffled Zarr-v2 stores with 32 KiB and 256 KiB blocks, plus a packed uint16 variant with CF attributes, into
-a temporary directory.  Then times one rectify_dataset call (nearest + bilinear of the same bands) three ways:
+Writes a seeded, OLCI-shaped scene (21 x 4091 x 4865 float32, compressible radiance-like values) as Zarr-v2 stores
+of the chosen ``--codec``, plus a packed uint16 variant with CF attributes, into a temporary directory:
+
+* ``blosc-lz4`` (default): Blosc-LZ4, byte-shuffled, with 32 KiB and 256 KiB blocks;
+* ``blosc-zstd``: the same with Zstd streams (``--zstd-level``);
+* ``zstd``: numcodecs ``zstd``, one frame per 1 MiB chunk (``--zstd-level``).
+
+  Then times one rectify_dataset call (nearest + bilinear of the same bands) three ways:
 
 * ``memory``: the bands as page-locked in-memory arrays;
 * ``host_decode``: the store through a plain LazySource that offers only ``read_bands`` (chunks decoded by
@@ -13,6 +18,7 @@ Also reports the decode kernels' time (CUDA events, one profiled call), GB/s of 
 the band bytes each path uploads (the band pipeline's ``h2d_bytes`` counter), the device name and power limit, and whether host- and device-decoded outputs are identical.
 
     python tools/zarr_decode_bench.py --steps 3 --out zarr_decode_bench.json
+    python tools/zarr_decode_bench.py --codec zstd --zstd-level 3 --steps 3
 """
 
 from __future__ import annotations
@@ -32,12 +38,21 @@ import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 
-def blosc_lz4_frame(raw: bytes, typesize: int, blocksize: int) -> bytes:
-    """A Blosc-1 frame (LZ4, byte shuffle, split streams) as numcodecs writes it, per io.blosc_decompress's layout."""
+def _compressor(codec: str, level: int):
+    """``bytes -> bytes`` of one Blosc stream or numcodecs chunk, and the Blosc inner codec number."""
     import pyarrow as pa
 
-    codec = pa.Codec("lz4_raw")
-    flags = (1 << 5) | 0x1
+    if codec == "blosc-lz4":
+        c = pa.Codec("lz4_raw")
+        return (lambda raw: c.compress(raw).to_pybytes()), 1
+    c = pa.Codec("zstd", compression_level=level)
+    return (lambda raw: c.compress(raw).to_pybytes()), 4
+
+
+def blosc_frame(raw: bytes, typesize: int, blocksize: int, codec: str = "blosc-lz4", level: int = 3) -> bytes:
+    """A Blosc-1 frame (byte shuffle, split streams) as numcodecs writes it, per io.blosc_decompress's layout."""
+    compress, fmt = _compressor(codec, level)
+    flags = (fmt << 5) | 0x1
     nblocks = -(-len(raw) // blocksize)
     parts, starts, pos = [], [], 16 + 4 * nblocks
     for b in range(nblocks):
@@ -50,7 +65,7 @@ def blosc_lz4_frame(raw: bytes, typesize: int, blocksize: int) -> bytes:
         starts.append(pos)
         for k in range(ns):
             part = block[k * ne:(k + 1) * ne].tobytes()
-            comp = codec.compress(part).to_pybytes()
+            comp = compress(part)
             if len(comp) >= ne:
                 comp = part
             parts.append(len(comp).to_bytes(4, "little") + comp)
@@ -59,10 +74,14 @@ def blosc_lz4_frame(raw: bytes, typesize: int, blocksize: int) -> bytes:
     return head + pos.to_bytes(4, "little") + b"".join(s.to_bytes(4, "little") for s in starts) + b"".join(parts)
 
 
-def write_store(path, array, chunks, blocksize, attrs=None):
+def write_store(path, array, chunks, blocksize, attrs=None, codec="blosc-lz4", level=3):
     os.makedirs(path, exist_ok=True)
-    meta = {"chunks": list(chunks), "compressor": {"id": "blosc", "cname": "lz4", "clevel": 5, "shuffle": 1,
-                                                    "blocksize": blocksize},
+    if codec == "zstd":
+        compressor = {"id": "zstd", "level": level}
+    else:
+        compressor = {"id": "blosc", "cname": "lz4" if codec == "blosc-lz4" else "zstd",
+                      "clevel": 5 if codec == "blosc-lz4" else level, "shuffle": 1, "blocksize": blocksize}
+    meta = {"chunks": list(chunks), "compressor": compressor,
             "dtype": array.dtype.str, "fill_value": None, "filters": None, "order": "C", "shape": list(array.shape),
             "zarr_format": 2}
     json.dump(meta, open(os.path.join(path, ".zarray"), "w"))
@@ -74,7 +93,10 @@ def write_store(path, array, chunks, blocksize, attrs=None):
         sl = tuple(slice(k * c, min(n, (k + 1) * c)) for k, c, n in zip(idx, chunks, array.shape))
         part = array[sl]
         block[tuple(slice(0, s) for s in part.shape)] = part
-        frame = blosc_lz4_frame(block.tobytes(), array.dtype.itemsize, blocksize)
+        if codec == "zstd":
+            frame = _compressor(codec, level)[0](block.tobytes())
+        else:
+            frame = blosc_frame(block.tobytes(), array.dtype.itemsize, blocksize, codec, level)
         with open(os.path.join(path, ".".join(str(k) for k in idx)), "wb") as fh:
             fh.write(frame)
         return len(frame)
@@ -110,6 +132,8 @@ def main():
     ap.add_argument("--steps", type=int, default=3)
     ap.add_argument("--scale", type=float, default=1.0, help="scene size relative to OLCI (1.0: 4865 x 4091)")
     ap.add_argument("--bands", type=int, default=21)
+    ap.add_argument("--codec", choices=("blosc-lz4", "blosc-zstd", "zstd"), default="blosc-lz4")
+    ap.add_argument("--zstd-level", type=int, default=3, help="zstd compression level (blosc-zstd, zstd)")
     ap.add_argument("--out", default=None, help="JSON result file (default: print only)")
     ap.add_argument("--dir", default=None, help="where the stores are written (default: a temporary directory)")
     args = ap.parse_args()
@@ -140,13 +164,16 @@ def main():
     chunks = (1, 512, 512)
     t0 = time.perf_counter()
     stores = {}
-    for label, bs in (("f32_block256k", 256 << 10), ("f32_block32k", 32 << 10)):
-        stores[label] = (os.path.join(root, label), write_store(os.path.join(root, label), rad, chunks, bs), None)
+    kw = dict(codec=args.codec, level=args.zstd_level)
+    blocks = (("f32", 0),) if args.codec == "zstd" else (("f32_block256k", 256 << 10), ("f32_block32k", 32 << 10))
+    for label, bs in blocks:
+        stores[label] = (os.path.join(root, label), write_store(os.path.join(root, label), rad, chunks, bs, **kw),
+                         None)
     packed = np.round((rad + 1.5) / 0.02).astype(np.uint16)
     packed[:, h // 3:h // 3 + 40, :] = 65535
     cf = {"scale_factor": 0.02, "add_offset": -1.5, "_FillValue": 65535}
-    stores["u16_cf_block256k"] = (os.path.join(root, "u16"), write_store(os.path.join(root, "u16"), packed, chunks,
-                                                                        256 << 10, cf), cf)
+    stores["u16_cf" if args.codec == "zstd" else "u16_cf_block256k"] = (
+        os.path.join(root, "u16"), write_store(os.path.join(root, "u16"), packed, chunks, 256 << 10, cf, **kw), cf)
     write_s = time.perf_counter() - t0
 
     class HostOnly(LazySource):
@@ -189,7 +216,8 @@ def main():
 
     result = {"tool": "tools/zarr_decode_bench.py", "device": torch.cuda.get_device_name(0),
               "power_limit": power_limit(), "scene": {"bands": nb, "height": h, "width": w, "chunks": list(chunks)},
-              "target": list(target_gm.size), "store_write_s": round(write_s, 1), "paths": {}}
+              "target": list(target_gm.size), "store_write_s": round(write_s, 1), "codec": args.codec,
+              "zstd_level": None if args.codec == "blosc-lz4" else args.zstd_level, "paths": {}}
     mem = _dev.pinned_empty(rad.shape, np.float32)
     mem[...] = rad
     _, t_mem, up_mem = timed(dataset(mem), args.steps)

@@ -1,10 +1,12 @@
-// decode.cu -- Zarr-v2 chunks compressed with Blosc-LZ4 / LZ4 (numcodecs) decoded on the device.
+// decode.cu -- Zarr-v2 chunks compressed with Blosc-LZ4 / Blosc-Zstd / LZ4 / Zstd (numcodecs) decoded on the device.
 //
-// The chunk files of a pipeline band chunk cross PCIe as they are on disk; three kernels turn them into the
+// The chunk files of a pipeline band chunk cross PCIe as they are on disk; four kernels turn them into the
 // pipeline's pitched (bands, win_h, wp) slot:
 //   k_zarr_index    one thread per Blosc block: walks the block's int32 stream-size prefixes and writes one
-//                   descriptor per stream (source range, destination range in the scratch, stored or LZ4);
-//   k_lz4_decode    one warp per stream: LZ4 block format into the scratch of decoded, still-shuffled blocks;
+//                   descriptor per stream (source range, destination range in the scratch, stored or compressed);
+//                   LZ4 streams come first in the descriptor array, Zstd streams after them;
+//   k_lz4_decode    one warp per LZ4 stream: LZ4 block format into the scratch of decoded, still-shuffled blocks;
+//   k_zstd_decode   one warp per Zstd stream: a Zstandard frame into the same scratch (decode_zstd.cuh);
 //   k_zarr_scatter  one thread per chunk element: gathers its bytes from the shuffled block, swaps big-endian
 //                   values, applies CF mask-and-scale, and stores it at its true position in the slot.
 // The container layout and the shuffle rule are those of io.blosc_decompress, which stays the reference.
@@ -19,8 +21,9 @@ namespace {
 
 constexpr int kBloscMaxSplits = 16, kBloscMinBufferSize = 128;
 constexpr int kMaxChunks = (1 << 24) - 1;  // the error word holds the chunk index in 24 bits
+constexpr int kZstdBlockMax = 128 << 10;  // a zstd block's largest decoded size, and its literals'
 
-// a stream of one Blosc block or of a numcodecs lz4 chunk (dsize 0: unused descriptor)
+// a stream of one Blosc block or of a numcodecs lz4 / zstd chunk (dsize 0: unused descriptor)
 struct StreamDesc {
     int64_t src;    // byte offset in `data`
     int64_t dst;    // byte offset in the scratch
@@ -76,6 +79,15 @@ __device__ inline void index_block(const uint8_t *data, const xrs_zarr_chunk *ch
         if (b != 0) return;
         d.src = ch.offset + 4;
         d.csize = static_cast<int32_t>(ch.length - 4);
+        d.dst = ch.scratch;
+        d.dsize = static_cast<int32_t>(chunk_bytes);
+        desc[ch.stream_base] = d;
+        return;
+    }
+    if (ch.codec == XRS_CHUNK_ZSTD) {  // numcodecs: one zstd frame
+        if (b != 0) return;
+        d.src = ch.offset;
+        d.csize = static_cast<int32_t>(ch.length);
         d.dst = ch.scratch;
         d.dsize = static_cast<int32_t>(chunk_bytes);
         desc[ch.stream_base] = d;
@@ -227,6 +239,13 @@ __global__ void __launch_bounds__(128) k_lz4_decode(const uint8_t *__restrict__ 
     if (reason && lane == 0) report(err, d.chunk, reason);
 }
 
+// The Zstd decoder (k_zstd_decode, launch_zstd) is compiled by nvcc; a host build of this file compiles it when it
+// defines XRS_HOST_ZSTD and leaves it out otherwise (a Zstd stream then fails the call).
+#if defined(__CUDACC__) || defined(XRS_HOST_ZSTD)
+#define XRS_ZSTD_DECODER 1
+#include "decode_zstd.cuh"
+#endif
+
 struct ScatterGeom {
     int64_t chunk_bytes, chunk_elems, cb, ch, cw;  // chunk shape (bands 1 for 2-D arrays)
     int64_t img_h, img_w, win_j0, win_j1, b0, nb;  // clip: image, slot rows, pipeline bands
@@ -339,57 +358,98 @@ int element_size(int dtype) {
     }
 }
 
-// Checks the table against the headers it carries and fills stream_base / n_streams / scratch; returns the stream
-// count (negative: an error, reported through fail()), the most blocks of one chunk and the scratch bytes (one decoded
-// chunk per file present).
-int64_t plan_streams(xrs_zarr_chunk *chunks, int64_t n_chunks, int64_t chunk_bytes, int64_t data_bytes,
-                     int64_t *max_blocks, int64_t *scratch_bytes) {
-    if (n_chunks < 0 || n_chunks > kMaxChunks) return fail("xrs_zarr_decode: bad chunk count"), -1;
+// Zstd streams: a numcodecs zstd chunk, or a Blosc frame with the Zstd inner codec that is not stored whole
+inline bool zstd_chunk(const xrs_zarr_chunk &ch) {
+    return ch.codec == XRS_CHUNK_ZSTD ||
+           (ch.codec == XRS_CHUNK_BLOSC && !(ch.header[2] & 0x2) && (ch.header[2] >> 5) == 4);
+}
+
+struct StreamPlan {
+    int64_t n;           // descriptors: [0, n_lz4) LZ4 or stored, [n_lz4, n) Zstd
+    int64_t n_lz4;
+    int64_t max_blocks;  // the most Blosc blocks of one chunk
+    int64_t scratch;     // bytes: one decoded chunk per file present
+    int64_t lit_stride;  // literal buffer of one Zstd stream: min(largest decoded Zstd stream, 128 KiB)
+};
+
+// Checks the table against the headers it carries and fills stream_base / n_streams / scratch; false on an error,
+// reported through fail().
+bool plan_streams(xrs_zarr_chunk *chunks, int64_t n_chunks, int64_t chunk_bytes, int64_t data_bytes, StreamPlan *plan) {
+    if (n_chunks < 0 || n_chunks > kMaxChunks) return fail("xrs_zarr_decode: bad chunk count"), false;
     if (chunk_bytes <= 0 || chunk_bytes > INT32_MAX)
-        return fail("xrs_zarr_decode: a chunk must hold 1 to 2^31 - 1 bytes"), -1;
-    int64_t n = 0;
-    *max_blocks = 1;
-    *scratch_bytes = 0;
+        return fail("xrs_zarr_decode: a chunk must hold 1 to 2^31 - 1 bytes"), false;
+    int64_t n_zstd = 0, largest = 0;
+    *plan = StreamPlan{0, 0, 1, 0, 0};
     for (int64_t c = 0; c < n_chunks; ++c) {
         xrs_zarr_chunk &ch = chunks[c];
         const std::string where = "xrs_zarr_decode: chunk " + std::to_string(c) + ": ";
-        ch.stream_base = n;
+        ch.stream_base = plan->n_lz4;
         ch.n_streams = 0;
         ch.scratch = -1;
         if (ch.codec == XRS_CHUNK_MISSING) continue;
         if (ch.offset < 0 || ch.length < 0 || (data_bytes >= 0 && ch.offset + ch.length > data_bytes))
-            return fail(where + "file bytes outside the data buffer"), -1;
+            return fail(where + "file bytes outside the data buffer"), false;
         if (ch.codec == XRS_CHUNK_LZ4) {
             if (ch.length < 4 || ch.length - 4 > INT32_MAX || static_cast<int32_t>(le32(ch.header)) != chunk_bytes)
-                return fail(where + "numcodecs lz4 size prefix does not match the chunk size"), -1;
+                return fail(where + "numcodecs lz4 size prefix does not match the chunk size"), false;
             ch.n_streams = 1;
+        } else if (ch.codec == XRS_CHUNK_ZSTD) {
+            if (ch.length < 6 || ch.length > INT32_MAX || le32(ch.header) != 0xFD2FB528u)
+                return fail(where + "not a zstd frame"), false;
+            ch.n_streams = 1;
+            largest = chunk_bytes > largest ? chunk_bytes : largest;
         } else if (ch.codec == XRS_CHUNK_BLOSC) {
             const BloscHeader h = blosc_header(ch.header);
             if (ch.length < 16 || ch.header[0] != 2 || h.nbytes != chunk_bytes || h.cbytes > ch.length)
-                return fail(where + "not a Blosc-1 frame of the chunk's size"), -1;
+                return fail(where + "not a Blosc-1 frame of the chunk's size"), false;
             if (h.flags & 0x2) {
-                if (16 + h.nbytes > ch.length) return fail(where + "truncated Blosc frame"), -1;
+                if (16 + h.nbytes > ch.length) return fail(where + "truncated Blosc frame"), false;
                 ch.n_streams = 1;
             } else {
-                if (h.flags & 0x4) return fail(where + "bit-shuffled Blosc frames are not decoded on the device"), -1;
-                if ((h.flags >> 5) != 1) return fail(where + "the Blosc frame's inner codec is not LZ4"), -1;
-                if (h.blocksize <= 0) return fail(where + "Blosc block size 0"), -1;
+                if (h.flags & 0x4) return fail(where + "bit-shuffled Blosc frames are not decoded on the device"), false;
+                if ((h.flags >> 5) != 1 && (h.flags >> 5) != 4)
+                    return fail(where + "the Blosc frame's inner codec is neither LZ4 nor Zstd"), false;
+                if (h.blocksize <= 0) return fail(where + "Blosc block size 0"), false;
                 const int64_t nblocks = ceil_div(h.nbytes, h.blocksize);
                 ch.n_streams = static_cast<int32_t>(nblocks * blosc_full_streams(h));
-                if (nblocks > *max_blocks) *max_blocks = nblocks;
+                if (nblocks > plan->max_blocks) plan->max_blocks = nblocks;
+                if ((h.flags >> 5) == 4) {  // a full block's streams, and the last, partial block (one stream)
+                    const int64_t full = h.nbytes >= h.blocksize ? h.blocksize / blosc_full_streams(h) : 0;
+                    const int64_t part = h.nbytes % h.blocksize;
+                    largest = full > largest ? full : largest;
+                    largest = part > largest ? part : largest;
+                }
             }
         } else {
-            return fail(where + "unknown codec " + std::to_string(ch.codec)), -1;
+            return fail(where + "unknown codec " + std::to_string(ch.codec)), false;
         }
-        n += ch.n_streams;
-        ch.scratch = *scratch_bytes;
-        *scratch_bytes += chunk_bytes;
+        int64_t &count = zstd_chunk(ch) ? n_zstd : plan->n_lz4;
+        ch.stream_base = count;
+        count += ch.n_streams;
+        ch.scratch = plan->scratch;
+        plan->scratch += chunk_bytes;
     }
-    if (ceil_div(n, 4) > INT32_MAX) return fail("xrs_zarr_decode: more LZ4 streams than one launch can take"), -1;
-    return n;
+    for (int64_t c = 0; c < n_chunks; ++c)
+        if (chunks[c].codec != XRS_CHUNK_MISSING && zstd_chunk(chunks[c])) chunks[c].stream_base += plan->n_lz4;
+    plan->n = plan->n_lz4 + n_zstd;
+    plan->lit_stride = largest < kZstdBlockMax ? largest : kZstdBlockMax;
+    if (ceil_div(plan->n_lz4, 4) > INT32_MAX) return fail("xrs_zarr_decode: more LZ4 streams than one launch can take"), false;
+    if (n_zstd > INT32_MAX) return fail("xrs_zarr_decode: more Zstd streams than one launch can take"), false;
+    return true;
 }
 
 int64_t align256(int64_t n) { return (n + 255) / 256 * 256; }
+
+// workspace: the chunk table, the descriptors, the scratch and, with Zstd streams, their literal buffers
+struct Workspace {
+    int64_t table, desc, scratch, lits;
+    Workspace(const StreamPlan &plan, int64_t n_chunks)
+        : table(align256(n_chunks * static_cast<int64_t>(sizeof(xrs_zarr_chunk)))),
+          desc(align256(plan.n * static_cast<int64_t>(sizeof(StreamDesc)))),
+          scratch(plan.n > plan.n_lz4 ? align256(plan.scratch) : plan.scratch),
+          lits((plan.n - plan.n_lz4) * plan.lit_stride) {}
+    int64_t total() const { return table + desc + scratch + lits; }
+};
 
 }  // namespace
 }  // namespace xrs
@@ -399,11 +459,9 @@ extern "C" {
 int64_t xrs_zarr_decode_workspace_bytes(xrs_zarr_chunk *chunks_host, int64_t n_chunks, int64_t chunk_bands,
                                         int64_t chunk_h, int64_t chunk_w, int32_t dtype) {
     const int64_t chunk_bytes = chunk_bands * chunk_h * chunk_w * xrs::element_size(dtype);
-    int64_t max_blocks, scratch_bytes;
-    const int64_t n_streams = xrs::plan_streams(chunks_host, n_chunks, chunk_bytes, -1, &max_blocks, &scratch_bytes);
-    if (n_streams < 0) return -1;
-    return xrs::align256(n_chunks * static_cast<int64_t>(sizeof(xrs_zarr_chunk))) +
-           xrs::align256(n_streams * static_cast<int64_t>(sizeof(xrs::StreamDesc))) + scratch_bytes;
+    xrs::StreamPlan plan;
+    if (!xrs::plan_streams(chunks_host, n_chunks, chunk_bytes, -1, &plan)) return -1;
+    return xrs::Workspace(plan, n_chunks).total();
 }
 
 int xrs_zarr_decode(const void *data, int64_t data_bytes, xrs_zarr_chunk *chunks_host, int64_t n_chunks,
@@ -418,30 +476,40 @@ int xrs_zarr_decode(const void *data, int64_t data_bytes, xrs_zarr_chunk *chunks
     if (!error_word || (n_chunks > 0 && (!data || !dst || !workspace)))
         return fail("xrs_zarr_decode: null buffer");
     const int64_t chunk_bytes = chunk_bands * chunk_h * chunk_w * isz;
-    int64_t max_blocks, scratch_bytes;
-    const int64_t n_streams = plan_streams(chunks_host, n_chunks, chunk_bytes, data_bytes, &max_blocks, &scratch_bytes);
-    if (n_streams < 0) return 1;
-    const int64_t table_bytes = align256(n_chunks * static_cast<int64_t>(sizeof(xrs_zarr_chunk)));
-    const int64_t desc_bytes = align256(n_streams * static_cast<int64_t>(sizeof(StreamDesc)));
-    if (workspace_bytes < table_bytes + desc_bytes + scratch_bytes)
+    StreamPlan plan;
+    if (!plan_streams(chunks_host, n_chunks, chunk_bytes, data_bytes, &plan)) return 1;
+    const int64_t n_streams = plan.n, n_zstd = plan.n - plan.n_lz4;
+    const Workspace ws(plan, n_chunks);
+    if (workspace_bytes < ws.total())
         return fail("xrs_zarr_decode: workspace smaller than xrs_zarr_decode_workspace_bytes");
     if (n_chunks == 0) return 0;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     auto *chunks = static_cast<xrs_zarr_chunk *>(workspace);
-    auto *desc = reinterpret_cast<StreamDesc *>(static_cast<uint8_t *>(workspace) + table_bytes);
-    uint8_t *scratch = static_cast<uint8_t *>(workspace) + table_bytes + desc_bytes;
+    auto *desc = reinterpret_cast<StreamDesc *>(static_cast<uint8_t *>(workspace) + ws.table);
+    uint8_t *scratch = static_cast<uint8_t *>(workspace) + ws.table + ws.desc;
     const auto *bytes = static_cast<const uint8_t *>(data);
     XRS_CUDA(cudaMemcpyAsync(chunks, chunks_host, n_chunks * sizeof(xrs_zarr_chunk), cudaMemcpyHostToDevice, st));
     if (n_streams > 0) {
-        const dim3 grid(static_cast<unsigned>(ceil_div(max_blocks, 128)),
+        const dim3 grid(static_cast<unsigned>(ceil_div(plan.max_blocks, 128)),
                         static_cast<unsigned>(n_chunks < 65535 ? n_chunks : 65535));  // the kernel strides over y
         XRS_TIMED("zarr_index", st,
                   k_zarr_index<<<grid, 128, 0, st>>>(bytes, chunks, n_chunks, chunk_bytes, desc, error_word));
         XRS_LAUNCH_CHECK("k_zarr_index");
-        const unsigned warps4 = static_cast<unsigned>(ceil_div(n_streams, 4));  // 4 warps of 32 per block
+    }
+    if (plan.n_lz4 > 0) {
+        const unsigned warps4 = static_cast<unsigned>(ceil_div(plan.n_lz4, 4));  // 4 warps of 32 per block
         XRS_TIMED("zarr_lz4_decode", st,
-                  k_lz4_decode<<<warps4, 128, 0, st>>>(bytes, desc, n_streams, scratch, error_word));
+                  k_lz4_decode<<<warps4, 128, 0, st>>>(bytes, desc, plan.n_lz4, scratch, error_word));
         XRS_LAUNCH_CHECK("k_lz4_decode");
+    }
+    if (n_zstd > 0) {
+#ifdef XRS_ZSTD_DECODER
+        const int rc = launch_zstd(bytes, desc + plan.n_lz4, n_zstd, scratch, scratch + ws.scratch, plan.lit_stride,
+                                   error_word, st);
+        if (rc) return rc;
+#else
+        return fail("xrs_zarr_decode: this build has no Zstd decoder");
+#endif
     }
     ScatterGeom g;
     g.chunk_bytes = chunk_bytes;

@@ -17,8 +17,8 @@ Stores understood without third-party packages:
   Zlib / Zstd inner codec, byte shuffle or none: :func:`blosc_decompress`), decoded on the reader thread.
   BloscLZ or bit-shuffled Blosc frames and Zarr filters need the ``zarr`` / ``numcodecs`` packages, which
   this build does not have; open such stores with xarray and pass the arrays instead.
-  Blosc-LZ4 / LZ4HC stores (byte shuffle or none) and numcodecs ``lz4`` stores are not decoded on the host in the
-  band pipeline: their chunk files are read as they are (:meth:`ZarrV2Source.device_read`), uploaded compressed and
+  Blosc-LZ4 / LZ4HC / Zstd stores (byte shuffle or none) and numcodecs ``lz4`` / ``zstd`` stores are not decoded on
+  the host in the band pipeline: their chunk files are read as they are (:meth:`ZarrV2Source.device_read`), uploaded compressed and
   decoded, unshuffled and CF-unpacked on the device (``xrs_zarr_decode``, ``csrc/decode.cu``).  ``read_bands`` stays
   the host decode, for ``values`` / ``read_all`` and every other codec.
 * :class:`NpySource` -- a ``.npy`` file, memory-mapped.
@@ -266,7 +266,9 @@ CHUNK_TABLE_DTYPE = np.dtype([("offset", "<i8"), ("length", "<i8"), ("band", "<i
                               ("codec", "<i4"), ("n_streams", "<i4"), ("stream_base", "<i8"), ("scratch", "<i8"),
                               ("header", "u1", 16)])
 assert CHUNK_TABLE_DTYPE.itemsize == 80
-CHUNK_MISSING, CHUNK_BLOSC, CHUNK_LZ4 = 0, 1, 2  # enum xrs_chunk_codec
+CHUNK_MISSING, CHUNK_BLOSC, CHUNK_LZ4, CHUNK_ZSTD = 0, 1, 2, 3  # enum xrs_chunk_codec
+_BLOSC_INNER = {"lz4": 1, "lz4hc": 1, "zstd": 4}  # Blosc flags bits 5-7 of a store's cname
+_ZSTD_HEADER_MAX = 18  # magic, descriptor, window, dictionary ID (4), content size (8)
 
 
 def _device_codec(compressor: dict | None) -> int | None:
@@ -275,18 +277,28 @@ def _device_codec(compressor: dict | None) -> int | None:
         return None
     if compressor.get("id") == "lz4":
         return CHUNK_LZ4
-    if compressor.get("id") == "blosc" and compressor.get("cname") in ("lz4", "lz4hc") and \
+    if compressor.get("id") == "zstd":
+        return CHUNK_ZSTD
+    if compressor.get("id") == "blosc" and compressor.get("cname") in _BLOSC_INNER and \
             compressor.get("shuffle", 1) in (0, 1):
         return CHUNK_BLOSC
     return None
 
 
-def _check_device_header(path: str, codec: int, head: bytes, size: int, chunk_bytes: int) -> None:
-    """The checks :func:`blosc_decompress` / the numcodecs lz4 decoder make before decoding, on a file's header
-    only, with the same errors; the device decode checks the streams."""
+def _check_device_header(path: str, codec: int, head: bytes, size: int, chunk_bytes: int, inner: int = 1) -> None:
+    """The checks :func:`blosc_decompress` / the numcodecs lz4 and zstd decoders make before decoding, on a file's
+    header only, with the same errors; the device decode checks the streams.  ``inner``: the Blosc inner codec the
+    store's ``cname`` names (1 LZ4, 4 Zstd); ``head``: the first 16 bytes of the file, 18 for zstd."""
     if codec == CHUNK_LZ4:
         if size < 4 or int.from_bytes(head[:4], "little", signed=True) != chunk_bytes:
             raise ValueError(f"{path}: the lz4 chunk's size prefix does not match the chunk size {chunk_bytes}")
+        return
+    if codec == CHUNK_ZSTD:
+        content = _zstd_content_size(head)
+        if content is None:
+            raise NotImplementedError("zstd frame without a content size")
+        if content != chunk_bytes:
+            raise ValueError(f"{path}: the zstd frame holds {content} bytes, the chunk {chunk_bytes}")
         return
     if size < 16:
         raise ValueError(f"{path}: not a Blosc frame: shorter than its 16-byte header")
@@ -303,15 +315,16 @@ def _check_device_header(path: str, codec: int, head: bytes, size: int, chunk_by
     if flags & 0x4:
         raise NotImplementedError("bit-shuffled Blosc frames need the zarr / blosc packages, which this build does "
                                   "not have")
-    if flags >> 5 != 1:
+    if flags >> 5 != inner:
         _blosc_stream_decoder(flags >> 5)  # BloscLZ: the host path's error
-        raise ValueError(f"{path}: the Blosc frame's inner codec ({flags >> 5}) is not the store's LZ4")
+        raise ValueError(f"{path}: the Blosc frame's inner codec ({flags >> 5}) is not the store's "
+                         f"{'Zstd' if inner == 4 else 'LZ4'}")
 
 
 class ZarrV2Source(LazySource):
     """One Zarr-v2 array of a directory store (2-D or 3-D, C order; uncompressed or with a codec of
-    :func:`chunk_decoder`).  Blosc-LZ4 / LZ4HC (byte shuffle or none) and numcodecs ``lz4`` stores can also be
-    read for the device (:meth:`device_read`): the band pipeline then decodes the chunks there."""
+    :func:`chunk_decoder`).  Blosc-LZ4 / LZ4HC / Zstd (byte shuffle or none) and numcodecs ``lz4`` / ``zstd`` stores
+    can also be read for the device (:meth:`device_read`): the band pipeline then decodes the chunks there."""
 
     def __init__(self, path: str):
         meta = json.load(open(os.path.join(path, ".zarray")))
@@ -337,6 +350,7 @@ class ZarrV2Source(LazySource):
         attrs_path = os.path.join(path, ".zattrs")
         self.attrs = json.load(open(attrs_path)) if os.path.isfile(attrs_path) else {}
         self.device_codec = _device_codec(meta.get("compressor"))
+        self._device_inner = _BLOSC_INNER.get((meta.get("compressor") or {}).get("cname"), 1)
 
     @property
     def device_decodable(self) -> bool:
@@ -387,10 +401,10 @@ class ZarrV2Source(LazySource):
                 got = fh.readinto(memoryview(buffer[pos:pos + size]))
             if got != size:
                 raise ValueError(f"{p}: short read ({got} of {size} bytes)")
-            head = buffer[pos:pos + min(size, 16)].tobytes()
-            _check_device_header(p, self.device_codec, head, size, chunk_bytes)
+            head = buffer[pos:pos + min(size, _ZSTD_HEADER_MAX if self.device_codec == CHUNK_ZSTD else 16)].tobytes()
+            _check_device_header(p, self.device_codec, head, size, chunk_bytes, self._device_inner)
             t["offset"], t["length"], t["codec"] = pos, size, self.device_codec
-            t["header"][:len(head)] = np.frombuffer(head, np.uint8)
+            t["header"][:min(len(head), 16)] = np.frombuffer(head[:16], np.uint8)
             pos += size
         return buffer, n_bytes, table, paths
 
