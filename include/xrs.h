@@ -337,11 +337,16 @@ int xrs_coarsen(const void *src, void *dst, int32_t dtype, int64_t n_slices, int
  * Compressed Zarr-v2 chunks decoded on the device (io.py, the I/O edge)
  * --------------------------------------------------------------------- */
 
-/* codec of one chunk file: missing (the array's fill value), a Blosc-1 frame with an LZ4 / LZ4HC or a Zstd inner
- * codec (numcodecs Blosc, byte shuffle or none, or a frame stored whole; each stream of a Zstd frame is one zstd
- * frame), numcodecs' lz4 (int32 decoded size, then one LZ4 block) or numcodecs' zstd (one zstd frame, RFC 8878,
- * without a dictionary; skippable frames may follow it) */
-enum xrs_chunk_codec { XRS_CHUNK_MISSING = 0, XRS_CHUNK_BLOSC = 1, XRS_CHUNK_LZ4 = 2, XRS_CHUNK_ZSTD = 3 };
+/* codec of one chunk file: missing (the array's fill value), a Blosc-1 frame with an LZ4 / LZ4HC, a Zstd or a Zlib
+ * inner codec (numcodecs Blosc, byte shuffle or none, or a frame stored whole; each stream of a Zstd frame is one
+ * zstd frame, each stream of a Zlib frame one zlib stream), numcodecs' lz4 (int32 decoded size, then one LZ4 block),
+ * numcodecs' zstd (one zstd frame, RFC 8878, without a dictionary; skippable frames may follow it), numcodecs' zlib
+ * (one zlib stream, RFC 1950, without a preset dictionary; bytes after its Adler-32 are ignored) or numcodecs' gzip
+ * (gzip members, RFC 1952, with NUL bytes between and after them allowed) */
+enum xrs_chunk_codec {
+    XRS_CHUNK_MISSING = 0, XRS_CHUNK_BLOSC = 1, XRS_CHUNK_LZ4 = 2, XRS_CHUNK_ZSTD = 3, XRS_CHUNK_ZLIB = 4,
+    XRS_CHUNK_GZIP = 5
+};
 
 /* One chunk file of a xrs_zarr_decode call (80 bytes). */
 typedef struct xrs_zarr_chunk {
@@ -371,15 +376,21 @@ typedef struct xrs_zarr_cf {
 enum xrs_decode_error {
     XRS_DECODE_BAD_LAYOUT = 1,          /* a block offset or stream size points outside the file */
     XRS_DECODE_OFFSET_ZERO = 2,         /* an LZ4 match offset of 0 */
-    XRS_DECODE_OFFSET_BEFORE_START = 3, /* a match reaching before the stream's first decoded byte */
-    XRS_DECODE_LITERALS_OVERRUN = 4,    /* literals past the decoded size or past the input */
+    XRS_DECODE_OFFSET_BEFORE_START = 3, /* a match reaching before the stream's first decoded byte (Deflate: before
+                                           the stream's or the gzip member's first byte) */
+    XRS_DECODE_LITERALS_OVERRUN = 4,    /* literals past the decoded size or past the input (Deflate: a literal or
+                                           stored block past the decoded size) */
     XRS_DECODE_MATCH_OVERRUN = 5,       /* a match past the decoded size */
     XRS_DECODE_INPUT_OVERRUN = 6,       /* length extension, offset or next token past the input; zstd: a frame
-                                           header, block or checksum past the input */
+                                           header, block or checksum past the input; Deflate: bits, a stored block,
+                                           a gzip header field or a trailer past the input */
     XRS_DECODE_SHORT = 7,               /* the stream ends short of its decoded size */
-    /* zstd frames only (the reasons above apply to them too; an offset of 0 is a repeat offset of 0) */
+    /* zstd frames (the reasons above apply to them too; an offset of 0 is a repeat offset of 0), and where noted
+     * zlib streams and gzip members */
     XRS_DECODE_BAD_FRAME_HEADER = 8,    /* unknown magic, reserved bit set, a dictionary ID other than 0, a window
-                                           beyond 2^31 bytes, or a content size other than the stream's */
+                                           beyond 2^31 bytes, or a content size other than the stream's; zlib: a
+                                           method other than 8, CINFO > 7, a bad FCHECK or FDICT set; gzip: a
+                                           member without the magic or with a method other than 8 */
     XRS_DECODE_BAD_BLOCK = 9,           /* reserved block type, or a compressed block above min(128 KiB, window) */
     XRS_DECODE_BAD_LITERALS = 10,       /* a literals section past its block or above min(128 KiB, window),
                                            treeless literals without a previous tree, or a Huffman stream that does
@@ -390,8 +401,19 @@ enum xrs_decode_error {
     XRS_DECODE_BAD_SEQUENCES = 13,      /* a sequences header past its block, reserved mode bits, a repeated table
                                            without a previous one, an RLE code out of range, or a bitstream not
                                            consumed exactly */
-    XRS_DECODE_TRAILING_BYTES = 14,     /* bytes after the frame that are not skippable frames */
-    XRS_DECODE_CHECKSUM = 15            /* the content checksum (XXH64, low 32 bits) does not match */
+    XRS_DECODE_TRAILING_BYTES = 14,     /* bytes after the frame that are not skippable frames; gzip: bytes after a
+                                           member that are neither NUL nor the next member */
+    XRS_DECODE_CHECKSUM = 15,           /* the content checksum (XXH64, low 32 bits) does not match; zlib: the
+                                           Adler-32; gzip: a member's CRC-32 or ISIZE (its size mod 2^32) */
+    /* Deflate streams only (RFC 1951) */
+    XRS_DECODE_BAD_DEFLATE_BLOCK = 16,  /* block type 3, or a stored block whose NLEN is not the complement of LEN */
+    XRS_DECODE_BAD_DEFLATE_CODES = 17,  /* a dynamic block's code description: more than 286 litlen or 30 distance
+                                           codes, an over-subscribed or incomplete set (a litlen or distance set may
+                                           be one code of length 1; a distance set may be empty), a repeat code 16
+                                           without a previous length or a repeat past the last length, or no
+                                           end-of-block code */
+    XRS_DECODE_BAD_DEFLATE_SYMBOL = 18  /* litlen symbol 286 / 287, distance symbol 30 / 31, or a code that an
+                                           incomplete set leaves unassigned (an empty distance set included) */
 };
 
 /* Decode whole chunk files and place their elements into a pitched (bands, rows, width) slot.
@@ -410,7 +432,8 @@ enum xrs_decode_error {
  *                      one decoded chunk per file present; with Zstd streams also one literal buffer per Zstd
  *                      stream of min(S, 128 KiB) bytes, S the largest decoded size of one Zstd stream in the call
  *                      (a numcodecs zstd chunk; for Blosc-Zstd, blocksize / streams of a full block or the last,
- *                      partial block), so a Blosc-Zstd call takes at most about twice the scratch of an LZ4 one
+ *                      partial block), so a Blosc-Zstd call takes at most about twice the scratch of an LZ4 one;
+ *                      Deflate streams (zlib, gzip, Blosc-Zlib) add nothing but their 32-byte descriptors
  *   error_word         device uint32, 0 before the first call; a malformed stream stores its reason and
  *                      chunk there (the first one recorded wins) and the call's results are undefined.  A file
  *                      the call can reject from its header alone fails the call itself, naming the chunk. */

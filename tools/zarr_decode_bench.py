@@ -5,13 +5,15 @@ of the chosen ``--codec``, plus a packed uint16 variant with CF attributes, into
 
 * ``blosc-lz4`` (default): Blosc-LZ4, byte-shuffled, with 32 KiB and 256 KiB blocks;
 * ``blosc-zstd``: the same with Zstd streams (``--zstd-level``);
-* ``zstd``: numcodecs ``zstd``, one frame per 1 MiB chunk (``--zstd-level``).
+* ``zstd``: numcodecs ``zstd``, one frame per 1 MiB chunk (``--zstd-level``);
+* ``blosc-zlib``: Blosc with Zlib streams (``--zlib-level``, default 1 as numcodecs');
+* ``zlib`` / ``gzip``: numcodecs ``zlib`` / ``gzip``, one stream or member per 1 MiB chunk (``--zlib-level``).
 
   Then times one rectify_dataset call (nearest + bilinear of the same bands) three ways:
 
 * ``memory``: the bands as page-locked in-memory arrays;
 * ``host_decode``: the store through a plain LazySource that offers only ``read_bands`` (chunks decoded by
-  ``io.blosc_decompress`` on the pipeline's reader thread);
+  the store's host decoder (``io.chunk_decoder``) on the pipeline's reader thread);
 * ``device_decode``: the store itself (chunk files uploaded compressed, decoded by xrs_zarr_decode).
 
 Also reports the decode kernels' time (CUDA events, one profiled call), GB/s of decoded and of compressed bytes,
@@ -19,6 +21,7 @@ the band bytes each path uploads (the band pipeline's ``h2d_bytes`` counter), th
 
     python tools/zarr_decode_bench.py --steps 3 --out zarr_decode_bench.json
     python tools/zarr_decode_bench.py --codec zstd --zstd-level 3 --steps 3
+    python tools/zarr_decode_bench.py --codec gzip --zlib-level 1 --steps 3
 """
 
 from __future__ import annotations
@@ -31,6 +34,7 @@ import subprocess
 import sys
 import tempfile
 import time
+import zlib
 from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
@@ -45,6 +49,12 @@ def _compressor(codec: str, level: int):
     if codec == "blosc-lz4":
         c = pa.Codec("lz4_raw")
         return (lambda raw: c.compress(raw).to_pybytes()), 1
+    if codec in ("blosc-zlib", "zlib"):
+        return (lambda raw: zlib.compress(raw, level)), 3
+    if codec == "gzip":
+        import gzip
+
+        return (lambda raw: gzip.compress(raw, level, mtime=0)), None
     c = pa.Codec("zstd", compression_level=level)
     return (lambda raw: c.compress(raw).to_pybytes()), 4
 
@@ -74,12 +84,15 @@ def blosc_frame(raw: bytes, typesize: int, blocksize: int, codec: str = "blosc-l
     return head + pos.to_bytes(4, "little") + b"".join(s.to_bytes(4, "little") for s in starts) + b"".join(parts)
 
 
+NUMCODECS = ("zstd", "zlib", "gzip")  # one compressed stream per chunk file, no Blosc container
+
+
 def write_store(path, array, chunks, blocksize, attrs=None, codec="blosc-lz4", level=3):
     os.makedirs(path, exist_ok=True)
-    if codec == "zstd":
-        compressor = {"id": "zstd", "level": level}
+    if codec in NUMCODECS:
+        compressor = {"id": codec, "level": level}
     else:
-        compressor = {"id": "blosc", "cname": "lz4" if codec == "blosc-lz4" else "zstd",
+        compressor = {"id": "blosc", "cname": codec[len("blosc-"):],
                       "clevel": 5 if codec == "blosc-lz4" else level, "shuffle": 1, "blocksize": blocksize}
     meta = {"chunks": list(chunks), "compressor": compressor,
             "dtype": array.dtype.str, "fill_value": None, "filters": None, "order": "C", "shape": list(array.shape),
@@ -93,7 +106,7 @@ def write_store(path, array, chunks, blocksize, attrs=None, codec="blosc-lz4", l
         sl = tuple(slice(k * c, min(n, (k + 1) * c)) for k, c, n in zip(idx, chunks, array.shape))
         part = array[sl]
         block[tuple(slice(0, s) for s in part.shape)] = part
-        if codec == "zstd":
+        if codec in NUMCODECS:
             frame = _compressor(codec, level)[0](block.tobytes())
         else:
             frame = blosc_frame(block.tobytes(), array.dtype.itemsize, blocksize, codec, level)
@@ -132,8 +145,10 @@ def main():
     ap.add_argument("--steps", type=int, default=3)
     ap.add_argument("--scale", type=float, default=1.0, help="scene size relative to OLCI (1.0: 4865 x 4091)")
     ap.add_argument("--bands", type=int, default=21)
-    ap.add_argument("--codec", choices=("blosc-lz4", "blosc-zstd", "zstd"), default="blosc-lz4")
+    ap.add_argument("--codec", choices=("blosc-lz4", "blosc-zstd", "zstd", "blosc-zlib", "zlib", "gzip"),
+                    default="blosc-lz4")
     ap.add_argument("--zstd-level", type=int, default=3, help="zstd compression level (blosc-zstd, zstd)")
+    ap.add_argument("--zlib-level", type=int, default=1, help="zlib compression level (blosc-zlib, zlib, gzip)")
     ap.add_argument("--out", default=None, help="JSON result file (default: print only)")
     ap.add_argument("--dir", default=None, help="where the stores are written (default: a temporary directory)")
     args = ap.parse_args()
@@ -164,15 +179,16 @@ def main():
     chunks = (1, 512, 512)
     t0 = time.perf_counter()
     stores = {}
-    kw = dict(codec=args.codec, level=args.zstd_level)
-    blocks = (("f32", 0),) if args.codec == "zstd" else (("f32_block256k", 256 << 10), ("f32_block32k", 32 << 10))
+    deflate = args.codec in ("blosc-zlib", "zlib", "gzip")
+    kw = dict(codec=args.codec, level=args.zlib_level if deflate else args.zstd_level)
+    blocks = (("f32", 0),) if args.codec in NUMCODECS else (("f32_block256k", 256 << 10), ("f32_block32k", 32 << 10))
     for label, bs in blocks:
         stores[label] = (os.path.join(root, label), write_store(os.path.join(root, label), rad, chunks, bs, **kw),
                          None)
     packed = np.round((rad + 1.5) / 0.02).astype(np.uint16)
     packed[:, h // 3:h // 3 + 40, :] = 65535
     cf = {"scale_factor": 0.02, "add_offset": -1.5, "_FillValue": 65535}
-    stores["u16_cf" if args.codec == "zstd" else "u16_cf_block256k"] = (
+    stores["u16_cf" if args.codec in NUMCODECS else "u16_cf_block256k"] = (
         os.path.join(root, "u16"), write_store(os.path.join(root, "u16"), packed, chunks, 256 << 10, cf, **kw), cf)
     write_s = time.perf_counter() - t0
 
@@ -217,7 +233,10 @@ def main():
     result = {"tool": "tools/zarr_decode_bench.py", "device": torch.cuda.get_device_name(0),
               "power_limit": power_limit(), "scene": {"bands": nb, "height": h, "width": w, "chunks": list(chunks)},
               "target": list(target_gm.size), "store_write_s": round(write_s, 1), "codec": args.codec,
-              "zstd_level": None if args.codec == "blosc-lz4" else args.zstd_level, "paths": {}}
+              "zstd_level": None if args.codec == "blosc-lz4" or deflate else args.zstd_level,
+              "paths": {}}
+    if deflate:
+        result["zlib_level"] = args.zlib_level
     mem = _dev.pinned_empty(rad.shape, np.float32)
     mem[...] = rad
     _, t_mem, up_mem = timed(dataset(mem), args.steps)

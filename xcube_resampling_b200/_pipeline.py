@@ -165,11 +165,14 @@ def zarr_decode(lib, source, data_addr: int, n_bytes: int, table, dst_addr: int,
 DECODE_ERRORS = {1: "a block offset or stream size points outside the file", 2: "a match offset of 0",
                  3: "a match reaching before the stream's start", 4: "literals past the decoded size",
                  5: "a match past the decoded size", 6: "the stream ends inside a sequence, header or block",
-                 7: "the stream ends short of its decoded size", 8: "a bad zstd frame header",
+                 7: "the stream ends short of its decoded size", 8: "a bad zstd frame, zlib or gzip header",
                  9: "a reserved zstd block type or a block above the block size limit",
                  10: "a bad zstd literals section", 11: "a bad zstd Huffman tree description",
                  12: "a bad zstd FSE table description", 13: "a bad zstd sequences section",
-                 14: "bytes after the zstd frame", 15: "a zstd content checksum mismatch"}
+                 14: "bytes after the zstd frame or gzip member",
+                 15: "a checksum mismatch (zstd content checksum, zlib Adler-32, gzip CRC-32 or size)",
+                 16: "a bad Deflate block type or stored block length",
+                 17: "a bad Deflate code description", 18: "an invalid Deflate litlen or distance code"}
 
 
 def decode_error(word: int, paths) -> str | None:

@@ -1,12 +1,14 @@
-// decode.cu -- Zarr-v2 chunks compressed with Blosc-LZ4 / Blosc-Zstd / LZ4 / Zstd (numcodecs) decoded on the device.
+// decode.cu -- Zarr-v2 chunks compressed with Blosc-LZ4 / Blosc-Zstd / Blosc-Zlib / LZ4 / Zstd / Zlib / GZip
+// (numcodecs) decoded on the device.
 //
-// The chunk files of a pipeline band chunk cross PCIe as they are on disk; four kernels turn them into the
+// The chunk files of a pipeline band chunk cross PCIe as they are on disk; five kernels turn them into the
 // pipeline's pitched (bands, win_h, wp) slot:
 //   k_zarr_index    one thread per Blosc block: walks the block's int32 stream-size prefixes and writes one
 //                   descriptor per stream (source range, destination range in the scratch, stored or compressed);
-//                   LZ4 streams come first in the descriptor array, Zstd streams after them;
+//                   LZ4 streams come first in the descriptor array, Zstd streams after them, Deflate streams last;
 //   k_lz4_decode    one warp per LZ4 stream: LZ4 block format into the scratch of decoded, still-shuffled blocks;
 //   k_zstd_decode   one warp per Zstd stream: a Zstandard frame into the same scratch (decode_zstd.cuh);
+//   k_inflate       one warp per Deflate stream: a zlib stream or gzip file into the same scratch (decode_deflate.cuh);
 //   k_zarr_scatter  one thread per chunk element: gathers its bytes from the shuffled block, swaps big-endian
 //                   values, applies CF mask-and-scale, and stores it at its true position in the slot.
 // The container layout and the shuffle rule are those of io.blosc_decompress, which stays the reference.
@@ -23,7 +25,7 @@ constexpr int kBloscMaxSplits = 16, kBloscMinBufferSize = 128;
 constexpr int kMaxChunks = (1 << 24) - 1;  // the error word holds the chunk index in 24 bits
 constexpr int kZstdBlockMax = 128 << 10;  // a zstd block's largest decoded size, and its literals'
 
-// a stream of one Blosc block or of a numcodecs lz4 / zstd chunk (dsize 0: unused descriptor)
+// a stream of one Blosc block or of a numcodecs lz4 / zstd / zlib / gzip chunk (dsize 0: unused descriptor)
 struct StreamDesc {
     int64_t src;    // byte offset in `data`
     int64_t dst;    // byte offset in the scratch
@@ -84,7 +86,7 @@ __device__ inline void index_block(const uint8_t *data, const xrs_zarr_chunk *ch
         desc[ch.stream_base] = d;
         return;
     }
-    if (ch.codec == XRS_CHUNK_ZSTD) {  // numcodecs: one zstd frame
+    if (ch.codec == XRS_CHUNK_ZSTD || ch.codec == XRS_CHUNK_ZLIB || ch.codec == XRS_CHUNK_GZIP) {  // the whole file
         if (b != 0) return;
         d.src = ch.offset;
         d.csize = static_cast<int32_t>(ch.length);
@@ -246,6 +248,12 @@ __global__ void __launch_bounds__(128) k_lz4_decode(const uint8_t *__restrict__ 
 #include "decode_zstd.cuh"
 #endif
 
+// The Deflate decoder (k_inflate, launch_inflate) likewise: a host build compiles it when it defines XRS_HOST_DEFLATE.
+#if defined(__CUDACC__) || defined(XRS_HOST_DEFLATE)
+#define XRS_DEFLATE_DECODER 1
+#include "decode_deflate.cuh"
+#endif
+
 struct ScatterGeom {
     int64_t chunk_bytes, chunk_elems, cb, ch, cw;  // chunk shape (bands 1 for 2-D arrays)
     int64_t img_h, img_w, win_j0, win_j1, b0, nb;  // clip: image, slot rows, pipeline bands
@@ -364,9 +372,15 @@ inline bool zstd_chunk(const xrs_zarr_chunk &ch) {
            (ch.codec == XRS_CHUNK_BLOSC && !(ch.header[2] & 0x2) && (ch.header[2] >> 5) == 4);
 }
 
+// Deflate streams: a numcodecs zlib or gzip chunk, or a Blosc frame with the Zlib inner codec not stored whole
+inline bool deflate_chunk(const xrs_zarr_chunk &ch) {
+    return ch.codec == XRS_CHUNK_ZLIB || ch.codec == XRS_CHUNK_GZIP ||
+           (ch.codec == XRS_CHUNK_BLOSC && !(ch.header[2] & 0x2) && (ch.header[2] >> 5) == 3);
+}
+
 struct StreamPlan {
-    int64_t n;           // descriptors: [0, n_lz4) LZ4 or stored, [n_lz4, n) Zstd
-    int64_t n_lz4;
+    int64_t n;           // descriptors: [0, n_lz4) LZ4 or stored, then n_zstd Zstd, then Deflate up to n
+    int64_t n_lz4, n_zstd;
     int64_t max_blocks;  // the most Blosc blocks of one chunk
     int64_t scratch;     // bytes: one decoded chunk per file present
     int64_t lit_stride;  // literal buffer of one Zstd stream: min(largest decoded Zstd stream, 128 KiB)
@@ -378,8 +392,8 @@ bool plan_streams(xrs_zarr_chunk *chunks, int64_t n_chunks, int64_t chunk_bytes,
     if (n_chunks < 0 || n_chunks > kMaxChunks) return fail("xrs_zarr_decode: bad chunk count"), false;
     if (chunk_bytes <= 0 || chunk_bytes > INT32_MAX)
         return fail("xrs_zarr_decode: a chunk must hold 1 to 2^31 - 1 bytes"), false;
-    int64_t n_zstd = 0, largest = 0;
-    *plan = StreamPlan{0, 0, 1, 0, 0};
+    int64_t n_zstd = 0, n_deflate = 0, largest = 0;
+    *plan = StreamPlan{0, 0, 0, 1, 0, 0};
     for (int64_t c = 0; c < n_chunks; ++c) {
         xrs_zarr_chunk &ch = chunks[c];
         const std::string where = "xrs_zarr_decode: chunk " + std::to_string(c) + ": ";
@@ -398,6 +412,17 @@ bool plan_streams(xrs_zarr_chunk *chunks, int64_t n_chunks, int64_t chunk_bytes,
                 return fail(where + "not a zstd frame"), false;
             ch.n_streams = 1;
             largest = chunk_bytes > largest ? chunk_bytes : largest;
+        } else if (ch.codec == XRS_CHUNK_ZLIB) {  // CMF, FLG, at least one byte of Deflate, Adler-32
+            const int cmf = ch.header[0], flg = ch.header[1];
+            if (ch.length < 7 || ch.length > INT32_MAX || (cmf & 15) != 8 || (cmf >> 4) > 7 ||
+                (cmf * 256 + flg) % 31 || (flg & 0x20))
+                return fail(where + "not a zlib stream without a preset dictionary"), false;
+            ch.n_streams = 1;
+        } else if (ch.codec == XRS_CHUNK_GZIP) {  // a 10-byte header, at least one byte of Deflate, CRC-32, ISIZE
+            if (ch.length < 19 || ch.length > INT32_MAX || ch.header[0] != 0x1f || ch.header[1] != 0x8b ||
+                ch.header[2] != 8)
+                return fail(where + "not a gzip member of method 8"), false;
+            ch.n_streams = 1;
         } else if (ch.codec == XRS_CHUNK_BLOSC) {
             const BloscHeader h = blosc_header(ch.header);
             if (ch.length < 16 || ch.header[0] != 2 || h.nbytes != chunk_bytes || h.cbytes > ch.length)
@@ -407,8 +432,8 @@ bool plan_streams(xrs_zarr_chunk *chunks, int64_t n_chunks, int64_t chunk_bytes,
                 ch.n_streams = 1;
             } else {
                 if (h.flags & 0x4) return fail(where + "bit-shuffled Blosc frames are not decoded on the device"), false;
-                if ((h.flags >> 5) != 1 && (h.flags >> 5) != 4)
-                    return fail(where + "the Blosc frame's inner codec is neither LZ4 nor Zstd"), false;
+                if ((h.flags >> 5) != 1 && (h.flags >> 5) != 3 && (h.flags >> 5) != 4)
+                    return fail(where + "the Blosc frame's inner codec is not LZ4, Zlib or Zstd"), false;
                 if (h.blocksize <= 0) return fail(where + "Blosc block size 0"), false;
                 const int64_t nblocks = ceil_div(h.nbytes, h.blocksize);
                 ch.n_streams = static_cast<int32_t>(nblocks * blosc_full_streams(h));
@@ -423,18 +448,24 @@ bool plan_streams(xrs_zarr_chunk *chunks, int64_t n_chunks, int64_t chunk_bytes,
         } else {
             return fail(where + "unknown codec " + std::to_string(ch.codec)), false;
         }
-        int64_t &count = zstd_chunk(ch) ? n_zstd : plan->n_lz4;
+        int64_t &count = zstd_chunk(ch) ? n_zstd : deflate_chunk(ch) ? n_deflate : plan->n_lz4;
         ch.stream_base = count;
         count += ch.n_streams;
         ch.scratch = plan->scratch;
         plan->scratch += chunk_bytes;
     }
-    for (int64_t c = 0; c < n_chunks; ++c)
-        if (chunks[c].codec != XRS_CHUNK_MISSING && zstd_chunk(chunks[c])) chunks[c].stream_base += plan->n_lz4;
-    plan->n = plan->n_lz4 + n_zstd;
+    for (int64_t c = 0; c < n_chunks; ++c) {
+        xrs_zarr_chunk &ch = chunks[c];
+        if (ch.codec == XRS_CHUNK_MISSING) continue;
+        if (zstd_chunk(ch)) ch.stream_base += plan->n_lz4;
+        else if (deflate_chunk(ch)) ch.stream_base += plan->n_lz4 + n_zstd;
+    }
+    plan->n_zstd = n_zstd;
+    plan->n = plan->n_lz4 + n_zstd + n_deflate;
     plan->lit_stride = largest < kZstdBlockMax ? largest : kZstdBlockMax;
     if (ceil_div(plan->n_lz4, 4) > INT32_MAX) return fail("xrs_zarr_decode: more LZ4 streams than one launch can take"), false;
     if (n_zstd > INT32_MAX) return fail("xrs_zarr_decode: more Zstd streams than one launch can take"), false;
+    if (n_deflate > INT32_MAX) return fail("xrs_zarr_decode: more Deflate streams than one launch can take"), false;
     return true;
 }
 
@@ -446,8 +477,8 @@ struct Workspace {
     Workspace(const StreamPlan &plan, int64_t n_chunks)
         : table(align256(n_chunks * static_cast<int64_t>(sizeof(xrs_zarr_chunk)))),
           desc(align256(plan.n * static_cast<int64_t>(sizeof(StreamDesc)))),
-          scratch(plan.n > plan.n_lz4 ? align256(plan.scratch) : plan.scratch),
-          lits((plan.n - plan.n_lz4) * plan.lit_stride) {}
+          scratch(plan.n_zstd > 0 ? align256(plan.scratch) : plan.scratch),
+          lits(plan.n_zstd * plan.lit_stride) {}
     int64_t total() const { return table + desc + scratch + lits; }
 };
 
@@ -478,7 +509,7 @@ int xrs_zarr_decode(const void *data, int64_t data_bytes, xrs_zarr_chunk *chunks
     const int64_t chunk_bytes = chunk_bands * chunk_h * chunk_w * isz;
     StreamPlan plan;
     if (!plan_streams(chunks_host, n_chunks, chunk_bytes, data_bytes, &plan)) return 1;
-    const int64_t n_streams = plan.n, n_zstd = plan.n - plan.n_lz4;
+    const int64_t n_streams = plan.n, n_zstd = plan.n_zstd, n_deflate = plan.n - plan.n_lz4 - plan.n_zstd;
     const Workspace ws(plan, n_chunks);
     if (workspace_bytes < ws.total())
         return fail("xrs_zarr_decode: workspace smaller than xrs_zarr_decode_workspace_bytes");
@@ -509,6 +540,14 @@ int xrs_zarr_decode(const void *data, int64_t data_bytes, xrs_zarr_chunk *chunks
         if (rc) return rc;
 #else
         return fail("xrs_zarr_decode: this build has no Zstd decoder");
+#endif
+    }
+    if (n_deflate > 0) {
+#ifdef XRS_DEFLATE_DECODER
+        const int rc = launch_inflate(bytes, chunks, desc + plan.n_lz4 + n_zstd, n_deflate, scratch, error_word, st);
+        if (rc) return rc;
+#else
+        return fail("xrs_zarr_decode: this build has no Deflate decoder");
 #endif
     }
     ScatterGeom g;

@@ -17,10 +17,11 @@ Stores understood without third-party packages:
   Zlib / Zstd inner codec, byte shuffle or none: :func:`blosc_decompress`), decoded on the reader thread.
   BloscLZ or bit-shuffled Blosc frames and Zarr filters need the ``zarr`` / ``numcodecs`` packages, which
   this build does not have; open such stores with xarray and pass the arrays instead.
-  Blosc-LZ4 / LZ4HC / Zstd stores (byte shuffle or none) and numcodecs ``lz4`` / ``zstd`` stores are not decoded on
-  the host in the band pipeline: their chunk files are read as they are (:meth:`ZarrV2Source.device_read`), uploaded compressed and
-  decoded, unshuffled and CF-unpacked on the device (``xrs_zarr_decode``, ``csrc/decode.cu``).  ``read_bands`` stays
-  the host decode, for ``values`` / ``read_all`` and every other codec.
+  Blosc-LZ4 / LZ4HC / Zstd / Zlib stores (byte shuffle or none) and numcodecs ``lz4`` / ``zstd`` / ``zlib`` / ``gzip``
+  stores are not decoded on the host in the band pipeline: their chunk files are read as they are
+  (:meth:`ZarrV2Source.device_read`), uploaded compressed and decoded, unshuffled and CF-unpacked on the device
+  (``xrs_zarr_decode``, ``csrc/decode.cu``).  ``read_bands`` stays the host decode, for ``values`` / ``read_all``
+  and every other codec.
 * :class:`NpySource` -- a ``.npy`` file, memory-mapped.
 * :class:`NetCDF3Source` -- a variable of a NetCDF classic / 64-bit-offset file (CDF-1 / CDF-2), memory-mapped
   through ``scipy.io.netcdf_file``; its big-endian values are byte-swapped by the copy into the staging
@@ -266,19 +267,20 @@ CHUNK_TABLE_DTYPE = np.dtype([("offset", "<i8"), ("length", "<i8"), ("band", "<i
                               ("codec", "<i4"), ("n_streams", "<i4"), ("stream_base", "<i8"), ("scratch", "<i8"),
                               ("header", "u1", 16)])
 assert CHUNK_TABLE_DTYPE.itemsize == 80
-CHUNK_MISSING, CHUNK_BLOSC, CHUNK_LZ4, CHUNK_ZSTD = 0, 1, 2, 3  # enum xrs_chunk_codec
-_BLOSC_INNER = {"lz4": 1, "lz4hc": 1, "zstd": 4}  # Blosc flags bits 5-7 of a store's cname
+CHUNK_MISSING, CHUNK_BLOSC, CHUNK_LZ4, CHUNK_ZSTD, CHUNK_ZLIB, CHUNK_GZIP = 0, 1, 2, 3, 4, 5  # enum xrs_chunk_codec
+_BLOSC_INNER = {"lz4": 1, "lz4hc": 1, "zlib": 3, "zstd": 4}  # Blosc flags bits 5-7 of a store's cname
+_BLOSC_INNER_NAMES = {1: "LZ4", 3: "Zlib", 4: "Zstd"}
+_NUMCODECS_DEVICE = {"lz4": CHUNK_LZ4, "zstd": CHUNK_ZSTD, "zlib": CHUNK_ZLIB, "gzip": CHUNK_GZIP}
 _ZSTD_HEADER_MAX = 18  # magic, descriptor, window, dictionary ID (4), content size (8)
+_GZIP_MIN = 19  # a gzip member's 10-byte header, one byte of Deflate, CRC-32 and ISIZE
 
 
 def _device_codec(compressor: dict | None) -> int | None:
     """The codec of ``xrs_zarr_decode`` a ``.zarray`` compressor maps to, ``None`` when chunks decode on the host."""
     if not compressor:
         return None
-    if compressor.get("id") == "lz4":
-        return CHUNK_LZ4
-    if compressor.get("id") == "zstd":
-        return CHUNK_ZSTD
+    if compressor.get("id") in _NUMCODECS_DEVICE:
+        return _NUMCODECS_DEVICE[compressor["id"]]
     if compressor.get("id") == "blosc" and compressor.get("cname") in _BLOSC_INNER and \
             compressor.get("shuffle", 1) in (0, 1):
         return CHUNK_BLOSC
@@ -286,9 +288,10 @@ def _device_codec(compressor: dict | None) -> int | None:
 
 
 def _check_device_header(path: str, codec: int, head: bytes, size: int, chunk_bytes: int, inner: int = 1) -> None:
-    """The checks :func:`blosc_decompress` / the numcodecs lz4 and zstd decoders make before decoding, on a file's
-    header only, with the same errors; the device decode checks the streams.  ``inner``: the Blosc inner codec the
-    store's ``cname`` names (1 LZ4, 4 Zstd); ``head``: the first 16 bytes of the file, 18 for zstd."""
+    """The checks :func:`blosc_decompress` / the numcodecs lz4, zstd, zlib and gzip decoders make before decoding, on
+    a file's header only, with the same errors; the device decode checks the streams.  ``inner``: the Blosc inner
+    codec the store's ``cname`` names (1 LZ4, 3 Zlib, 4 Zstd); ``head``: the first 16 bytes of the file, 18 for
+    zstd, 19 for gzip."""
     if codec == CHUNK_LZ4:
         if size < 4 or int.from_bytes(head[:4], "little", signed=True) != chunk_bytes:
             raise ValueError(f"{path}: the lz4 chunk's size prefix does not match the chunk size {chunk_bytes}")
@@ -299,6 +302,17 @@ def _check_device_header(path: str, codec: int, head: bytes, size: int, chunk_by
             raise NotImplementedError("zstd frame without a content size")
         if content != chunk_bytes:
             raise ValueError(f"{path}: the zstd frame holds {content} bytes, the chunk {chunk_bytes}")
+        return
+    if codec in (CHUNK_ZLIB, CHUNK_GZIP):
+        name = "zlib" if codec == CHUNK_ZLIB else "gzip"
+        if codec == CHUNK_ZLIB:  # CMF, FLG without FDICT, and room for one byte of Deflate and the Adler-32
+            ok = size >= 7 and (head[0] & 15) == 8 and head[0] >> 4 <= 7 and (head[0] * 256 + head[1]) % 31 == 0 \
+                and not head[1] & 0x20
+        else:  # magic and method 8, and room for one byte of Deflate, the CRC-32 and ISIZE
+            ok = size >= 19 and bytes(head[:3]) == b"\x1f\x8b\x08"
+        if not ok:  # the host decoder's own error for the file's start (all of it, when the file is that short)
+            chunk_decoder({"id": name})(bytes(head))
+            raise ValueError(f"{path}: a {name} chunk file of {size} bytes does not decode to {chunk_bytes} bytes")
         return
     if size < 16:
         raise ValueError(f"{path}: not a Blosc frame: shorter than its 16-byte header")
@@ -318,13 +332,14 @@ def _check_device_header(path: str, codec: int, head: bytes, size: int, chunk_by
     if flags >> 5 != inner:
         _blosc_stream_decoder(flags >> 5)  # BloscLZ: the host path's error
         raise ValueError(f"{path}: the Blosc frame's inner codec ({flags >> 5}) is not the store's "
-                         f"{'Zstd' if inner == 4 else 'LZ4'}")
+                         f"{_BLOSC_INNER_NAMES[inner]}")
 
 
 class ZarrV2Source(LazySource):
     """One Zarr-v2 array of a directory store (2-D or 3-D, C order; uncompressed or with a codec of
-    :func:`chunk_decoder`).  Blosc-LZ4 / LZ4HC / Zstd (byte shuffle or none) and numcodecs ``lz4`` / ``zstd`` stores
-    can also be read for the device (:meth:`device_read`): the band pipeline then decodes the chunks there."""
+    :func:`chunk_decoder`).  Blosc-LZ4 / LZ4HC / Zstd / Zlib (byte shuffle or none) and numcodecs ``lz4`` / ``zstd`` /
+    ``zlib`` / ``gzip`` stores can also be read for the device (:meth:`device_read`): the band pipeline then decodes
+    the chunks there."""
 
     def __init__(self, path: str):
         meta = json.load(open(os.path.join(path, ".zarray")))
@@ -401,7 +416,8 @@ class ZarrV2Source(LazySource):
                 got = fh.readinto(memoryview(buffer[pos:pos + size]))
             if got != size:
                 raise ValueError(f"{p}: short read ({got} of {size} bytes)")
-            head = buffer[pos:pos + min(size, _ZSTD_HEADER_MAX if self.device_codec == CHUNK_ZSTD else 16)].tobytes()
+            n_head = {CHUNK_ZSTD: _ZSTD_HEADER_MAX, CHUNK_GZIP: _GZIP_MIN}.get(self.device_codec, 16)
+            head = buffer[pos:pos + min(size, n_head)].tobytes()
             _check_device_header(p, self.device_codec, head, size, chunk_bytes, self._device_inner)
             t["offset"], t["length"], t["codec"] = pos, size, self.device_codec
             t["header"][:min(len(head), 16)] = np.frombuffer(head[:16], np.uint8)
