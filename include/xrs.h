@@ -334,7 +334,7 @@ int xrs_coarsen(const void *src, void *dst, int32_t dtype, int64_t n_slices, int
                 int64_t src_pitch, int64_t src_slice_stride, int32_t agg, int32_t f_j, int32_t f_i, void *stream);
 
 /* ------------------------------------------------------------------------
- * Compressed Zarr-v2 chunks decoded on the device (io.py, the I/O edge)
+ * Compressed Zarr v2 / v3 chunks decoded on the device (io.py, the I/O edge)
  * --------------------------------------------------------------------- */
 
 /* codec of one chunk file: missing (the array's fill value), a Blosc-1 frame with an LZ4 / LZ4HC, a Zstd or a Zlib
@@ -342,18 +342,27 @@ int xrs_coarsen(const void *src, void *dst, int32_t dtype, int64_t n_slices, int
  * zstd frame, each stream of a Zlib frame one zlib stream), numcodecs' lz4 (int32 decoded size, then one LZ4 block),
  * numcodecs' zstd (one zstd frame, RFC 8878, without a dictionary; skippable frames may follow it), numcodecs' zlib
  * (one zlib stream, RFC 1950, without a preset dictionary; bytes after its Adler-32 are ignored) or numcodecs' gzip
- * (gzip members, RFC 1952, with NUL bytes between and after them allowed) */
+ * (gzip members, RFC 1952, with NUL bytes between and after them allowed).  Zarr v3's zstd, gzip and blosc codecs
+ * write the same streams.
+ * XRS_CHUNK_CRC32C is a flag OR-ed into a codec other than XRS_CHUNK_MISSING (Zarr v3's crc32c codec after the
+ * compressor): the last 4 bytes of the file are the little-endian CRC-32C (Castagnoli, reflected polynomial
+ * 0x82F63B78) of the bytes in front of them, and the codec applies to the length - 4 bytes of that payload.  The
+ * call checks the trailer on the device (k_crc32c, before any decoder) and reports XRS_DECODE_CRC32C on a mismatch.
+ * `header` holds the payload's first 16 bytes, as for an unflagged file.  A table without the flag is decoded
+ * exactly as before. */
 enum xrs_chunk_codec {
     XRS_CHUNK_MISSING = 0, XRS_CHUNK_BLOSC = 1, XRS_CHUNK_LZ4 = 2, XRS_CHUNK_ZSTD = 3, XRS_CHUNK_ZLIB = 4,
-    XRS_CHUNK_GZIP = 5
+    XRS_CHUNK_GZIP = 5,
+    XRS_CHUNK_CRC32C = 0x100
 };
 
-/* One chunk file of a xrs_zarr_decode call (80 bytes). */
+/* One chunk file of a xrs_zarr_decode call (80 bytes); for a sharded Zarr v3 array, one inner chunk: offset / length
+ * cover exactly that chunk's bytes. */
 typedef struct xrs_zarr_chunk {
     int64_t offset;       /* first byte of the file in `data` */
     int64_t length;       /* bytes of the file (0 when missing) */
     int64_t band, row, col; /* array index of the chunk's element (0, 0, 0); band 0 for 2-D arrays */
-    int32_t codec;        /* enum xrs_chunk_codec */
+    int32_t codec;        /* enum xrs_chunk_codec, optionally | XRS_CHUNK_CRC32C */
     int32_t n_streams;    /* filled by the call */
     int64_t stream_base;  /* filled by the call */
     int64_t scratch;      /* filled by the call: where the decoded chunk goes in the workspace, -1 when missing */
@@ -412,8 +421,10 @@ enum xrs_decode_error {
                                            be one code of length 1; a distance set may be empty), a repeat code 16
                                            without a previous length or a repeat past the last length, or no
                                            end-of-block code */
-    XRS_DECODE_BAD_DEFLATE_SYMBOL = 18  /* litlen symbol 286 / 287, distance symbol 30 / 31, or a code that an
+    XRS_DECODE_BAD_DEFLATE_SYMBOL = 18, /* litlen symbol 286 / 287, distance symbol 30 / 31, or a code that an
                                            incomplete set leaves unassigned (an empty distance set included) */
+    /* files flagged XRS_CHUNK_CRC32C */
+    XRS_DECODE_CRC32C = 19              /* the CRC-32C trailer does not match the payload in front of it */
 };
 
 /* Decode whole chunk files and place their elements into a pitched (bands, rows, width) slot.

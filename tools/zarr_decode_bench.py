@@ -9,6 +9,12 @@ of the chosen ``--codec``, plus a packed uint16 variant with CF attributes, into
 * ``blosc-zlib``: Blosc with Zlib streams (``--zlib-level``, default 1 as numcodecs');
 * ``zlib`` / ``gzip``: numcodecs ``zlib`` / ``gzip``, one stream or member per 1 MiB chunk (``--zlib-level``).
 
+``--zarr-format 3`` writes the same scene as Zarr v3 arrays instead (``zarr.json``, ``c/...`` chunk keys, codecs
+``bytes`` then the compressor: ``zstd``, ``gzip``, ``blosc`` or ``numcodecs.zlib``); ``--crc32c`` appends the ``crc32c``
+codec; ``--shard BANDS,ROWS,COLS`` wraps the chunks into ``sharding_indexed`` shards of that shape (index at the end,
+followed by its CRC-32C, as zarr-python writes it).  The device decode then reports ``k_crc32c``'s time beside the
+decode kernels'.
+
   Then times one rectify_dataset call (nearest + bilinear of the same bands) three ways:
 
 * ``memory``: the bands as page-locked in-memory arrays;
@@ -22,6 +28,7 @@ the band bytes each path uploads (the band pipeline's ``h2d_bytes`` counter), th
     python tools/zarr_decode_bench.py --steps 3 --out zarr_decode_bench.json
     python tools/zarr_decode_bench.py --codec zstd --zstd-level 3 --steps 3
     python tools/zarr_decode_bench.py --codec gzip --zlib-level 1 --steps 3
+    python tools/zarr_decode_bench.py --codec zstd --zarr-format 3 --shard 1,2048,2048 --crc32c --steps 3
 """
 
 from __future__ import annotations
@@ -87,8 +94,25 @@ def blosc_frame(raw: bytes, typesize: int, blocksize: int, codec: str = "blosc-l
 NUMCODECS = ("zstd", "zlib", "gzip")  # one compressed stream per chunk file, no Blosc container
 
 
-def write_store(path, array, chunks, blocksize, attrs=None, codec="blosc-lz4", level=3):
+def _v3_codecs(codec: str, level: int, typesize: int, blocksize: int, crc: bool) -> list:
+    """The Zarr v3 codec chain of a store written with ``codec``."""
+    if codec == "zstd":
+        comp = {"name": "zstd", "configuration": {"level": level, "checksum": False}}
+    elif codec == "gzip":
+        comp = {"name": "gzip", "configuration": {"level": level}}
+    elif codec == "zlib":
+        comp = {"name": "numcodecs.zlib", "configuration": {"level": level}}
+    else:
+        comp = {"name": "blosc", "configuration": {"cname": codec[len("blosc-"):], "clevel": level, "shuffle": "shuffle",
+                                                   "typesize": typesize, "blocksize": blocksize}}
+    return [{"name": "bytes", "configuration": {"endian": "little"}}, comp] + ([{"name": "crc32c"}] if crc else [])
+
+
+def write_store(path, array, chunks, blocksize, attrs=None, codec="blosc-lz4", level=3, zarr_format=2, crc=False,
+                shard=None):
     os.makedirs(path, exist_ok=True)
+    if zarr_format == 3:
+        return _write_store_v3(path, array, chunks, blocksize, attrs, codec, level, crc, shard)
     if codec in NUMCODECS:
         compressor = {"id": codec, "level": level}
     else:
@@ -116,6 +140,68 @@ def write_store(path, array, chunks, blocksize, attrs=None, codec="blosc-lz4", l
 
     with ThreadPoolExecutor(os.cpu_count() or 4) as pool:
         return sum(pool.map(one, np.ndindex(*[len(g) for g in grid])))
+
+
+def _encode(array, chunks, idx, blocksize, codec, level) -> bytes:
+    """The compressed bytes of chunk ``idx`` (edge chunks padded with zeros)."""
+    block = np.zeros(chunks, dtype=array.dtype)
+    sl = tuple(slice(k * c, min(n, (k + 1) * c)) for k, c, n in zip(idx, chunks, array.shape))
+    part = array[sl]
+    block[tuple(slice(0, s) for s in part.shape)] = part
+    if codec in NUMCODECS:
+        return _compressor(codec, level)[0](block.tobytes())
+    return blosc_frame(block.tobytes(), array.dtype.itemsize, blocksize, codec, level)
+
+
+def _write_store_v3(path, array, chunks, blocksize, attrs, codec, level, crc, shard):
+    """A Zarr v3 array: chunks (inner chunks of ``shard``-shaped shards) under ``c/``, each followed by its CRC-32C
+    when ``crc``; a shard file ends in its index of (offset, nbytes) uint64 pairs and the index's CRC-32C."""
+    from xcube_resampling_b200.io import crc32c
+
+    def encode(idx):
+        data = _encode(array, chunks, idx, blocksize, codec, level)
+        return data + crc32c(data).to_bytes(4, "little") if crc else data
+
+    def put(idx, data):
+        p = os.path.join(path, "c", *[str(k) for k in idx])
+        os.makedirs(os.path.dirname(p), exist_ok=True)
+        with open(p, "wb") as fh:
+            fh.write(data)
+        return len(data)
+
+    inner = _v3_codecs(codec, level, array.dtype.itemsize, blocksize, crc)
+    if shard is None:
+        codecs, grid_chunks = inner, list(chunks)
+
+        def one(idx):
+            return put(idx, encode(idx))
+        units = np.ndindex(*[-(-n // c) for n, c in zip(array.shape, chunks)])
+    else:
+        per = tuple(s // c for s, c in zip(shard, chunks))
+        index_codecs = [{"name": "bytes", "configuration": {"endian": "little"}}, {"name": "crc32c"}]
+        codecs = [{"name": "sharding_indexed", "configuration": {
+            "chunk_shape": list(chunks), "codecs": inner, "index_codecs": index_codecs, "index_location": "end"}}]
+        grid_chunks = list(shard)
+
+        def one(sidx):
+            index = np.full((int(np.prod(per)), 2), 2 ** 64 - 1, np.uint64)
+            body = bytearray()
+            for k, local in enumerate(np.ndindex(*per)):
+                idx = tuple(s * p + q for s, p, q in zip(sidx, per, local))
+                if all(i * c < n for i, c, n in zip(idx, chunks, array.shape)):
+                    data = encode(idx)
+                    index[k] = (len(body), len(data))
+                    body += data
+            raw = index.astype("<u8").tobytes()
+            return put(sidx, bytes(body) + raw + crc32c(raw).to_bytes(4, "little"))
+        units = np.ndindex(*[-(-n // c) for n, c in zip(array.shape, shard)])
+    meta = {"zarr_format": 3, "node_type": "array", "shape": list(array.shape), "data_type": array.dtype.name,
+            "chunk_grid": {"name": "regular", "configuration": {"chunk_shape": grid_chunks}},
+            "chunk_key_encoding": {"name": "default", "configuration": {"separator": "/"}}, "fill_value": 0,
+            "codecs": codecs, "attributes": dict(attrs or {}), "dimension_names": ["band", "y", "x"]}
+    json.dump(meta, open(os.path.join(path, "zarr.json"), "w"))
+    with ThreadPoolExecutor(os.cpu_count() or 4) as pool:
+        return sum(pool.map(one, units))
 
 
 def radiance(nb, h, w, seed):
@@ -149,15 +235,21 @@ def main():
                     default="blosc-lz4")
     ap.add_argument("--zstd-level", type=int, default=3, help="zstd compression level (blosc-zstd, zstd)")
     ap.add_argument("--zlib-level", type=int, default=1, help="zlib compression level (blosc-zlib, zlib, gzip)")
+    ap.add_argument("--zarr-format", type=int, choices=(2, 3), default=2, help="write Zarr v2 or v3 stores")
+    ap.add_argument("--shard", default=None, help="BANDS,ROWS,COLS: v3 sharding_indexed shards of that shape")
+    ap.add_argument("--crc32c", action="store_true", help="v3: the crc32c codec after the compressor")
     ap.add_argument("--out", default=None, help="JSON result file (default: print only)")
     ap.add_argument("--dir", default=None, help="where the stores are written (default: a temporary directory)")
     args = ap.parse_args()
+    shard = tuple(int(v) for v in args.shard.split(",")) if args.shard else None
+    if args.zarr_format == 2 and (shard or args.crc32c):
+        ap.error("--shard and --crc32c need --zarr-format 3")
 
     import torch
 
     import xcube_resampling_b200 as xrs
     from xcube_resampling_b200 import _dev, _lib, _pipeline, synthetic as syn
-    from xcube_resampling_b200.io import DecodedSource, LazyDataArray, LazySource, ZarrV2Source
+    from xcube_resampling_b200.io import DecodedSource, LazyDataArray, LazySource, ZarrV2Source, ZarrV3Source
 
     if not torch.cuda.is_available():
         raise SystemExit("no CUDA device: this benchmark measures the GPU path and has no CPU fallback")
@@ -177,10 +269,13 @@ def main():
     root = args.dir or tempfile.mkdtemp(prefix="zarr_decode_bench_")
     rad = radiance(nb, h, w, seed=1)
     chunks = (1, 512, 512)
+    if shard and any(s % c for s, c in zip(shard, chunks)):
+        raise SystemExit(f"--shard {args.shard} is not a multiple of the chunks {chunks}")
     t0 = time.perf_counter()
     stores = {}
     deflate = args.codec in ("blosc-zlib", "zlib", "gzip")
-    kw = dict(codec=args.codec, level=args.zlib_level if deflate else args.zstd_level)
+    kw = dict(codec=args.codec, level=args.zlib_level if deflate else args.zstd_level, zarr_format=args.zarr_format,
+              crc=args.crc32c, shard=shard)
     blocks = (("f32", 0),) if args.codec in NUMCODECS else (("f32_block256k", 256 << 10), ("f32_block32k", 32 << 10))
     for label, bs in blocks:
         stores[label] = (os.path.join(root, label), write_store(os.path.join(root, label), rad, chunks, bs, **kw),
@@ -234,6 +329,7 @@ def main():
               "power_limit": power_limit(), "scene": {"bands": nb, "height": h, "width": w, "chunks": list(chunks)},
               "target": list(target_gm.size), "store_write_s": round(write_s, 1), "codec": args.codec,
               "zstd_level": None if args.codec == "blosc-lz4" or deflate else args.zstd_level,
+              "zarr_format": args.zarr_format, "shard": list(shard) if shard else None, "crc32c": args.crc32c,
               "paths": {}}
     if deflate:
         result["zlib_level"] = args.zlib_level
@@ -242,9 +338,10 @@ def main():
     _, t_mem, up_mem = timed(dataset(mem), args.steps)
     result["paths"]["memory_f32"] = {"ms": t_mem, "ms_median": float(np.median(t_mem)), "band_h2d_bytes": up_mem}
     for label, (path, file_bytes, attrs) in stores.items():
-        base = ZarrV2Source(path)
+        Source = ZarrV3Source if args.zarr_format == 3 else ZarrV2Source
+        base = Source(path)
         dev_src = DecodedSource(base, attrs) if attrs else base
-        host_src = HostOnly(DecodedSource(ZarrV2Source(path), attrs) if attrs else ZarrV2Source(path))
+        host_src = HostOnly(DecodedSource(Source(path), attrs) if attrs else Source(path))
         assert dev_src.device_decodable
         out_h, t_h, up_h = timed(dataset(host_src), args.steps)
         out_d, t_d, up_d = timed(dataset(dev_src), args.steps)
@@ -263,6 +360,8 @@ def main():
             "device_decode": {"ms": t_d, "ms_median": float(np.median(t_d)), "band_h2d_bytes": up_d,
                               "decode_kernels_ms": {k: {"ms": v[0], "launches": v[1]} for k, v in dec.items()},
                               "decode_ms": dec_ms,
+                              "crc32c_ms": dec.get("zarr_crc32c", (0.0,))[0],
+                              "crc32c_share_of_decode": dec.get("zarr_crc32c", (0.0,))[0] / dec_ms if dec_ms else None,
                               "decoded_GBps": decoded / dec_ms / 1e6 if dec_ms else None,
                               "compressed_GBps": up_d / dec_ms / 1e6 if dec_ms else None},
             "host_vs_device_outputs_identical": bool(same)}

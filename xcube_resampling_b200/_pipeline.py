@@ -172,7 +172,8 @@ DECODE_ERRORS = {1: "a block offset or stream size points outside the file", 2: 
                  14: "bytes after the zstd frame or gzip member",
                  15: "a checksum mismatch (zstd content checksum, zlib Adler-32, gzip CRC-32 or size)",
                  16: "a bad Deflate block type or stored block length",
-                 17: "a bad Deflate code description", 18: "an invalid Deflate litlen or distance code"}
+                 17: "a bad Deflate code description", 18: "an invalid Deflate litlen or distance code",
+                 19: "a CRC-32C trailer that does not match the chunk's bytes"}
 
 
 def decode_error(word: int, paths) -> str | None:

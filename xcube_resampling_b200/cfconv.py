@@ -156,7 +156,7 @@ def get_dataset_grid_mapping_proxies(dataset, *, missing_latitude_longitude_crs:
 
 def add_spatial_ref(store_path: str, crs: CRS, crs_var_name: str = "spatial_ref",
                     xy_dim_names: tuple[str, str] | None = None) -> None:
-    """``cfconv.py:320-358`` for a Zarr-v2 DIRECTORY store: add a scalar ``spatial_ref`` array that
+    """``cfconv.py:320-358`` for a Zarr v2 or v3 DIRECTORY store: add a scalar ``spatial_ref`` array that
     carries the CRS's CF attributes and point every array whose last two dimensions are (y, x) at it
     (``grid_mapping`` attribute); consolidated metadata, if present, is rewritten."""
     if not isinstance(store_path, str):
@@ -164,6 +164,9 @@ def add_spatial_ref(store_path: str, crs: CRS, crs_var_name: str = "spatial_ref"
     if not isinstance(crs_var_name, str):
         raise TypeError(f"crs_var_name must be an instance of {str}, was {type(crs_var_name)}")
     x_dim, y_dim = xy_dim_names or ("x", "y")
+    if os.path.isfile(os.path.join(store_path, "zarr.json")):
+        _add_spatial_ref_v3(store_path, crs, crs_var_name, x_dim, y_dim)
+        return
     var_dir = os.path.join(store_path, crs_var_name)
     os.makedirs(var_dir, exist_ok=True)
     with open(os.path.join(var_dir, ".zarray"), "w") as fh:
@@ -195,3 +198,50 @@ def add_spatial_ref(store_path: str, crs: CRS, crs_var_name: str = "spatial_ref"
                     entries[key] = json.load(open(os.path.join(root, f)))
         with open(consolidated, "w") as fh:
             json.dump({"metadata": entries, "zarr_consolidated_format": 1}, fh)
+
+
+def _add_spatial_ref_v3(store_path: str, crs: CRS, crs_var_name: str, x_dim: str, y_dim: str) -> None:
+    """:func:`add_spatial_ref` for a Zarr v3 group: a 0-D uint8 array (codecs ``[bytes]``, chunk key in the store's
+    encoding), ``grid_mapping`` in the ``attributes`` of the (y, x) arrays, and the root's ``consolidated_metadata``
+    entries rewritten when it has them."""
+    from .io import _v3_key, v3_dimension_names
+
+    root_path = os.path.join(store_path, "zarr.json")
+    root = json.load(open(root_path))
+    if root.get("zarr_format") != 3 or root.get("node_type") != "group":
+        raise ValueError(f"{store_path}: not a Zarr v3 group")
+    arrays = {}
+    for item in sorted(os.listdir(store_path)):
+        meta_path = os.path.join(store_path, item, "zarr.json")
+        if item != crs_var_name and os.path.isfile(meta_path):
+            meta = json.load(open(meta_path))
+            if meta.get("node_type") == "array":
+                arrays[item] = meta
+    encoding = next((m["chunk_key_encoding"] for m in arrays.values() if m.get("chunk_key_encoding")),
+                    {"name": "default", "configuration": {"separator": "/"}})
+    var_dir = os.path.join(store_path, crs_var_name)
+    os.makedirs(var_dir, exist_ok=True)
+    sr = {"zarr_format": 3, "node_type": "array", "shape": [], "data_type": "uint8",
+          "chunk_grid": {"name": "regular", "configuration": {"chunk_shape": []}}, "chunk_key_encoding": encoding,
+          "fill_value": 0, "codecs": [{"name": "bytes"}], "attributes": dict(crs.to_cf()), "dimension_names": [],
+          "storage_transformers": []}
+    with open(os.path.join(var_dir, "zarr.json"), "w") as fh:
+        json.dump(sr, fh)
+    with open(os.path.join(var_dir, _v3_key(encoding, ())), "wb") as fh:
+        fh.write(b"\x00")
+    for item, meta in arrays.items():
+        dims = v3_dimension_names(meta)
+        if len(dims) >= 2 and dims[-2] == y_dim and dims[-1] == x_dim:
+            meta["attributes"] = dict(meta.get("attributes") or {}, grid_mapping=crs_var_name)
+            with open(os.path.join(store_path, item, "zarr.json"), "w") as fh:
+                json.dump(meta, fh)
+    consolidated = root.get("consolidated_metadata")
+    if isinstance(consolidated, dict) and "metadata" in consolidated:
+        entries = {}
+        for dirpath, _dirs, files in os.walk(store_path):
+            if "zarr.json" in files and dirpath != store_path:
+                key = os.path.relpath(dirpath, store_path).replace(os.sep, "/")
+                entries[key] = json.load(open(os.path.join(dirpath, "zarr.json")))
+        consolidated["metadata"] = dict(sorted(entries.items()))
+        with open(root_path, "w") as fh:
+            json.dump(root, fh)

@@ -1,8 +1,10 @@
-// decode.cu -- Zarr-v2 chunks compressed with Blosc-LZ4 / Blosc-Zstd / Blosc-Zlib / LZ4 / Zstd / Zlib / GZip
-// (numcodecs) decoded on the device.
+// decode.cu -- Zarr chunks compressed with Blosc-LZ4 / Blosc-Zstd / Blosc-Zlib / LZ4 / Zstd / Zlib / GZip
+// (numcodecs, and the Zarr v3 codecs that write the same streams) decoded on the device.
 //
-// The chunk files of a pipeline band chunk cross PCIe as they are on disk; five kernels turn them into the
-// pipeline's pitched (bands, win_h, wp) slot:
+// The chunk files of a pipeline band chunk (Zarr v3: the inner chunks of a shard) cross PCIe as they are on disk;
+// six kernels turn them into the pipeline's pitched (bands, win_h, wp) slot:
+//   k_crc32c        one warp per file with a CRC-32C trailer (Zarr v3's crc32c codec): checks it, then drops it from
+//                   the device copy of the chunk table (decode_crc32c.cuh);
 //   k_zarr_index    one thread per Blosc block: walks the block's int32 stream-size prefixes and writes one
 //                   descriptor per stream (source range, destination range in the scratch, stored or compressed);
 //                   LZ4 streams come first in the descriptor array, Zstd streams after them, Deflate streams last;
@@ -241,6 +243,61 @@ __global__ void __launch_bounds__(128) k_lz4_decode(const uint8_t *__restrict__ 
     if (reason && lane == 0) report(err, d.chunk, reason);
 }
 
+// CRC arithmetic modulo a reflected polynomial (zlib's multmodp / x2nmodp): a * b, and x^(8n).  Poly 0xEDB88320 is
+// CRC-32 (gzip members), 0x82F63B78 CRC-32C (the crc32c codec of Zarr v3).
+template <uint32_t Poly>
+__device__ inline uint32_t crc_mul(uint32_t a, uint32_t b) {
+    uint32_t p = 0;
+    for (uint32_t m = 1u << 31; m != 0; m >>= 1) {
+        if (a & m) {
+            p ^= b;
+            if ((a & (m - 1)) == 0) break;
+        }
+        b = b & 1 ? (b >> 1) ^ Poly : b >> 1;
+    }
+    return p;
+}
+template <uint32_t Poly>
+__device__ inline uint32_t crc_shift(int64_t n) {
+    uint32_t p = 1u << 31, x = 1u << 23;  // x^0, x^8
+    for (; n; n >>= 1) {
+        if (n & 1) p = crc_mul<Poly>(x, p);
+        x = crc_mul<Poly>(x, x);
+    }
+    return p;
+}
+
+// The CRC of buf[0, n) by the whole warp: one contiguous segment a lane through a byte table, the segments' CRCs
+// combined as zlib's crc32_combine does.  `table` (256 words) and `part` (32 words) are the warp's shared memory.
+template <uint32_t Poly>
+__device__ inline uint32_t warp_crc(const uint8_t *buf, int64_t n, uint32_t *table, uint32_t *part, int lane) {
+    for (int i = lane; i < 256; i += 32) {
+        uint32_t c = static_cast<uint32_t>(i);
+        for (int k = 0; k < 8; ++k) c = c & 1 ? (c >> 1) ^ Poly : c >> 1;
+        table[i] = c;
+    }
+    __syncwarp();
+    const int64_t seg = (n + 31) / 32, lo = lane * seg < n ? lane * seg : n, hi = lo + seg < n ? lo + seg : n;
+    uint32_t c = 0xffffffffu;
+    for (int64_t k = lo; k < hi; ++k) c = table[(c ^ buf[k]) & 0xff] ^ (c >> 8);
+    part[lane] = ~c;
+    __syncwarp();
+    uint32_t crc = 0, shift = crc_shift<Poly>(seg);
+    for (int s = 0; s < 32; ++s) {
+        const int64_t l = s * seg < n ? (s * seg + seg < n ? seg : n - s * seg) : 0;
+        crc = crc_mul<Poly>(l == seg ? shift : crc_shift<Poly>(l), crc) ^ part[s];
+    }
+    __syncwarp();
+    return crc;
+}
+
+// The CRC-32C check (k_crc32c, launch_crc32c) is compiled by nvcc; a host build of this file compiles it when it
+// defines XRS_HOST_CRC32C and leaves it out otherwise (a chunk flagged XRS_CHUNK_CRC32C then fails the call).
+#if defined(__CUDACC__) || defined(XRS_HOST_CRC32C)
+#define XRS_CRC32C_CHECK 1
+#include "decode_crc32c.cuh"
+#endif
+
 // The Zstd decoder (k_zstd_decode, launch_zstd) is compiled by nvcc; a host build of this file compiles it when it
 // defines XRS_HOST_ZSTD and leaves it out otherwise (a Zstd stream then fails the call).
 #if defined(__CUDACC__) || defined(XRS_HOST_ZSTD)
@@ -366,16 +423,20 @@ int element_size(int dtype) {
     }
 }
 
+// the codec of a table entry without the XRS_CHUNK_CRC32C flag
+inline int base_codec(const xrs_zarr_chunk &ch) { return ch.codec & ~XRS_CHUNK_CRC32C; }
+
 // Zstd streams: a numcodecs zstd chunk, or a Blosc frame with the Zstd inner codec that is not stored whole
 inline bool zstd_chunk(const xrs_zarr_chunk &ch) {
-    return ch.codec == XRS_CHUNK_ZSTD ||
-           (ch.codec == XRS_CHUNK_BLOSC && !(ch.header[2] & 0x2) && (ch.header[2] >> 5) == 4);
+    const int codec = base_codec(ch);
+    return codec == XRS_CHUNK_ZSTD || (codec == XRS_CHUNK_BLOSC && !(ch.header[2] & 0x2) && (ch.header[2] >> 5) == 4);
 }
 
 // Deflate streams: a numcodecs zlib or gzip chunk, or a Blosc frame with the Zlib inner codec not stored whole
 inline bool deflate_chunk(const xrs_zarr_chunk &ch) {
-    return ch.codec == XRS_CHUNK_ZLIB || ch.codec == XRS_CHUNK_GZIP ||
-           (ch.codec == XRS_CHUNK_BLOSC && !(ch.header[2] & 0x2) && (ch.header[2] >> 5) == 3);
+    const int codec = base_codec(ch);
+    return codec == XRS_CHUNK_ZLIB || codec == XRS_CHUNK_GZIP ||
+           (codec == XRS_CHUNK_BLOSC && !(ch.header[2] & 0x2) && (ch.header[2] >> 5) == 3);
 }
 
 struct StreamPlan {
@@ -384,6 +445,7 @@ struct StreamPlan {
     int64_t max_blocks;  // the most Blosc blocks of one chunk
     int64_t scratch;     // bytes: one decoded chunk per file present
     int64_t lit_stride;  // literal buffer of one Zstd stream: min(largest decoded Zstd stream, 128 KiB)
+    int64_t n_crc;       // files flagged XRS_CHUNK_CRC32C
 };
 
 // Checks the table against the headers it carries and fills stream_base / n_streams / scratch; false on an error,
@@ -393,7 +455,7 @@ bool plan_streams(xrs_zarr_chunk *chunks, int64_t n_chunks, int64_t chunk_bytes,
     if (chunk_bytes <= 0 || chunk_bytes > INT32_MAX)
         return fail("xrs_zarr_decode: a chunk must hold 1 to 2^31 - 1 bytes"), false;
     int64_t n_zstd = 0, n_deflate = 0, largest = 0;
-    *plan = StreamPlan{0, 0, 0, 1, 0, 0};
+    *plan = StreamPlan{0, 0, 0, 1, 0, 0, 0};
     for (int64_t c = 0; c < n_chunks; ++c) {
         xrs_zarr_chunk &ch = chunks[c];
         const std::string where = "xrs_zarr_decode: chunk " + std::to_string(c) + ": ";
@@ -403,32 +465,39 @@ bool plan_streams(xrs_zarr_chunk *chunks, int64_t n_chunks, int64_t chunk_bytes,
         if (ch.codec == XRS_CHUNK_MISSING) continue;
         if (ch.offset < 0 || ch.length < 0 || (data_bytes >= 0 && ch.offset + ch.length > data_bytes))
             return fail(where + "file bytes outside the data buffer"), false;
-        if (ch.codec == XRS_CHUNK_LZ4) {
-            if (ch.length < 4 || ch.length - 4 > INT32_MAX || static_cast<int32_t>(le32(ch.header)) != chunk_bytes)
+        // a CRC-32C trailer: the codec applies to the payload in front of it (k_crc32c checks and drops it)
+        const int codec = base_codec(ch);
+        const bool crc = ch.codec & XRS_CHUNK_CRC32C;
+        if (crc && (codec == XRS_CHUNK_MISSING || ch.length < 4))
+            return fail(where + "a CRC-32C flag on a missing chunk or on a file shorter than its 4-byte trailer"), false;
+        const int64_t length = ch.length - (crc ? 4 : 0);
+        plan->n_crc += crc;
+        if (codec == XRS_CHUNK_LZ4) {
+            if (length < 4 || length - 4 > INT32_MAX || static_cast<int32_t>(le32(ch.header)) != chunk_bytes)
                 return fail(where + "numcodecs lz4 size prefix does not match the chunk size"), false;
             ch.n_streams = 1;
-        } else if (ch.codec == XRS_CHUNK_ZSTD) {
-            if (ch.length < 6 || ch.length > INT32_MAX || le32(ch.header) != 0xFD2FB528u)
+        } else if (codec == XRS_CHUNK_ZSTD) {
+            if (length < 6 || length > INT32_MAX || le32(ch.header) != 0xFD2FB528u)
                 return fail(where + "not a zstd frame"), false;
             ch.n_streams = 1;
             largest = chunk_bytes > largest ? chunk_bytes : largest;
-        } else if (ch.codec == XRS_CHUNK_ZLIB) {  // CMF, FLG, at least one byte of Deflate, Adler-32
+        } else if (codec == XRS_CHUNK_ZLIB) {  // CMF, FLG, at least one byte of Deflate, Adler-32
             const int cmf = ch.header[0], flg = ch.header[1];
-            if (ch.length < 7 || ch.length > INT32_MAX || (cmf & 15) != 8 || (cmf >> 4) > 7 ||
+            if (length < 7 || length > INT32_MAX || (cmf & 15) != 8 || (cmf >> 4) > 7 ||
                 (cmf * 256 + flg) % 31 || (flg & 0x20))
                 return fail(where + "not a zlib stream without a preset dictionary"), false;
             ch.n_streams = 1;
-        } else if (ch.codec == XRS_CHUNK_GZIP) {  // a 10-byte header, at least one byte of Deflate, CRC-32, ISIZE
-            if (ch.length < 19 || ch.length > INT32_MAX || ch.header[0] != 0x1f || ch.header[1] != 0x8b ||
+        } else if (codec == XRS_CHUNK_GZIP) {  // a 10-byte header, at least one byte of Deflate, CRC-32, ISIZE
+            if (length < 19 || length > INT32_MAX || ch.header[0] != 0x1f || ch.header[1] != 0x8b ||
                 ch.header[2] != 8)
                 return fail(where + "not a gzip member of method 8"), false;
             ch.n_streams = 1;
-        } else if (ch.codec == XRS_CHUNK_BLOSC) {
+        } else if (codec == XRS_CHUNK_BLOSC) {
             const BloscHeader h = blosc_header(ch.header);
-            if (ch.length < 16 || ch.header[0] != 2 || h.nbytes != chunk_bytes || h.cbytes > ch.length)
+            if (length < 16 || ch.header[0] != 2 || h.nbytes != chunk_bytes || h.cbytes > length)
                 return fail(where + "not a Blosc-1 frame of the chunk's size"), false;
             if (h.flags & 0x2) {
-                if (16 + h.nbytes > ch.length) return fail(where + "truncated Blosc frame"), false;
+                if (16 + h.nbytes > length) return fail(where + "truncated Blosc frame"), false;
                 ch.n_streams = 1;
             } else {
                 if (h.flags & 0x4) return fail(where + "bit-shuffled Blosc frames are not decoded on the device"), false;
@@ -520,6 +589,14 @@ int xrs_zarr_decode(const void *data, int64_t data_bytes, xrs_zarr_chunk *chunks
     uint8_t *scratch = static_cast<uint8_t *>(workspace) + ws.table + ws.desc;
     const auto *bytes = static_cast<const uint8_t *>(data);
     XRS_CUDA(cudaMemcpyAsync(chunks, chunks_host, n_chunks * sizeof(xrs_zarr_chunk), cudaMemcpyHostToDevice, st));
+    if (plan.n_crc > 0) {
+#ifdef XRS_CRC32C_CHECK
+        const int rc = launch_crc32c(bytes, chunks, n_chunks, error_word, st);
+        if (rc) return rc;
+#else
+        return fail("xrs_zarr_decode: this build has no CRC-32C check");
+#endif
+    }
     if (n_streams > 0) {
         const dim3 grid(static_cast<unsigned>(ceil_div(plan.max_blocks, 128)),
                         static_cast<unsigned>(n_chunks < 65535 ? n_chunks : 65535));  // the kernel strides over y

@@ -441,49 +441,6 @@ __device__ inline uint32_t inf_adler32(const uint8_t *buf, int64_t n, InflateSha
     return static_cast<uint32_t>(((sb % 65521) << 16) | (sa % 65521));
 }
 
-// CRC-32 arithmetic modulo the reflected polynomial (zlib's multmodp / x2nmodp): a * b, and x^(8n)
-__device__ inline uint32_t crc_mul(uint32_t a, uint32_t b) {
-    uint32_t p = 0;
-    for (uint32_t m = 1u << 31; m != 0; m >>= 1) {
-        if (a & m) {
-            p ^= b;
-            if ((a & (m - 1)) == 0) break;
-        }
-        b = b & 1 ? (b >> 1) ^ 0xEDB88320u : b >> 1;
-    }
-    return p;
-}
-__device__ inline uint32_t crc_shift(int64_t n) {
-    uint32_t p = 1u << 31, x = 1u << 23;  // x^0, x^8
-    for (; n; n >>= 1) {
-        if (n & 1) p = crc_mul(x, p);
-        x = crc_mul(x, x);
-    }
-    return p;
-}
-
-// CRC-32 of buf[0, n), one segment a lane, the segments' CRCs combined as zlib's crc32_combine does
-__device__ inline uint32_t inf_crc32(const uint8_t *buf, int64_t n, InflateShared &sm, int lane) {
-    for (int i = lane; i < 256; i += 32) {
-        uint32_t c = static_cast<uint32_t>(i);
-        for (int k = 0; k < 8; ++k) c = c & 1 ? (c >> 1) ^ 0xEDB88320u : c >> 1;
-        sm.crc[i] = c;
-    }
-    __syncwarp();
-    const int64_t seg = (n + 31) / 32, lo = lane * seg < n ? lane * seg : n, hi = lo + seg < n ? lo + seg : n;
-    uint32_t c = 0xffffffffu;
-    for (int64_t k = lo; k < hi; ++k) c = sm.crc[(c ^ buf[k]) & 0xff] ^ (c >> 8);
-    sm.part[lane] = ~c;
-    __syncwarp();
-    uint32_t crc = 0, shift = crc_shift(seg);
-    for (int s = 0; s < 32; ++s) {
-        const int64_t l = s * seg < n ? (s * seg + seg < n ? seg : n - s * seg) : 0;
-        crc = crc_mul(l == seg ? shift : crc_shift(l), crc) ^ sm.part[s];
-    }
-    __syncwarp();
-    return crc;
-}
-
 // The zlib stream or gzip file in[0, n) into out[0, dsize), by the whole warp; returns 0 or the reason.  Not inlined:
 // inlined, it changes how nvcc compiles k_zstd_decode in the same file.
 __device__ __noinline__ int inflate_file(const uint8_t *in, int64_t n, uint8_t *out, int64_t dsize, bool gzip,
@@ -537,7 +494,8 @@ __device__ __noinline__ int inflate_file(const uint8_t *in, int64_t n, uint8_t *
         const int reason = inflate_stream(in, n, &p, out, &op, m0, dsize, sm, lane);
         if (reason) return reason;
         if (n - p < 8) return XRS_DECODE_INPUT_OVERRUN;
-        if (inf_crc32(out + m0, op - m0, sm, lane) != le32(in + p) || le32(in + p + 4) != static_cast<uint32_t>(op - m0))
+        if (warp_crc<0xEDB88320u>(out + m0, op - m0, sm.crc, sm.part, lane) != le32(in + p) ||
+            le32(in + p + 4) != static_cast<uint32_t>(op - m0))
             return XRS_DECODE_CHECKSUM;
         p += 8;
     }

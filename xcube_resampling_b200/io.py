@@ -22,6 +22,14 @@ Stores understood without third-party packages:
   (:meth:`ZarrV2Source.device_read`), uploaded compressed and decoded, unshuffled and CF-unpacked on the device
   (``xrs_zarr_decode``, ``csrc/decode.cu``).  ``read_bands`` stays the host decode, for ``values`` / ``read_all``
   and every other codec.
+* :class:`ZarrV3Source` -- a Zarr v3 array in a directory store (``zarr.json``), sharded (``sharding_indexed``)
+  or not, with the ``bytes`` codec (either byte order), at most one compressor (``zstd``, ``gzip``, ``blosc``, or the
+  ``numcodecs.<id>`` twin of a :func:`chunk_decoder` codec) and optionally the ``crc32c`` checksum, checked by
+  :func:`crc32c` on the host path.  Written from the Zarr v3 core specification and its ``sharding_indexed`` and
+  ``crc32c`` codec specifications.  It shares the chunk loops of :class:`ZarrV2Source`; only where a chunk's bytes
+  are (a file, or a range of a shard file named by the shard's index) and how they are framed differ.  Stores whose
+  compressor the device decodes reach it the same way, one inner chunk at a time, their CRC-32C checked on the
+  device.
 * :class:`NpySource` -- a ``.npy`` file, memory-mapped.
 * :class:`NetCDF3Source` -- a variable of a NetCDF classic / 64-bit-offset file (CDF-1 / CDF-2), memory-mapped
   through ``scipy.io.netcdf_file``; its big-endian values are byte-swapped by the copy into the staging
@@ -29,7 +37,7 @@ Stores understood without third-party packages:
   have; open them with xarray and pass the arrays instead.
 
 :func:`open_zarr_dataset` / :func:`open_netcdf_dataset` assemble a :class:`~xcube_resampling_b200.dataset.Dataset` from a
-directory store: coordinate arrays (1-D, or 2-D named like coordinates) are read eagerly, every
+directory store (Zarr v2, or a Zarr v3 group): coordinate arrays (1-D, or 2-D named like coordinates) are read eagerly, every
 other array becomes a lazy variable.
 """
 
@@ -206,6 +214,95 @@ def _zstd_content_size(raw: bytes) -> int | None:
     return value + 256 if n == 2 else value
 
 
+_CRC32C_POLY = 0x82F63B78  # CRC-32C (Castagnoli), reflected
+_CRC_SEGMENT = 64  # bytes of one segment of crc32c's vectorised pass
+
+
+def _crc_mul(a: int, b, poly: int = _CRC32C_POLY):
+    """``a * b`` modulo the reflected polynomial ``poly`` (bit 31 is x^0; zlib's multmodp); ``b`` may be a uint32
+    array, multiplied element by element."""
+    p = b ^ b
+    for k in range(32):
+        if a & (0x80000000 >> k):
+            p = p ^ b
+        b = (b >> 1) ^ ((b & 1) * poly)
+    return p
+
+
+def _crc_shift(n: int, poly: int = _CRC32C_POLY) -> int:
+    """x^(8n) modulo ``poly``: the operator that runs a CRC register over ``n`` zero bytes (zlib's x2nmodp)."""
+    p, x = 0x80000000, 0x00800000  # x^0, x^8
+    while n:
+        if n & 1:
+            p = _crc_mul(x, p, poly)
+        x = _crc_mul(x, x, poly)
+        n >>= 1
+    return p
+
+
+_crc32c_tables: dict = {}
+
+
+def _crc32c_table(shift_bytes: int) -> np.ndarray:
+    """(4, 256) uint32: row k maps byte v to x^(8 * shift_bytes) * (v << 8k), so that a register ``c`` run over
+    ``shift_bytes`` zero bytes is the XOR of ``table[k][(c >> 8k) & 255]``; ``shift_bytes`` 0 gives the byte table of
+    CRC-32C itself (register ``c`` over one byte ``v`` is ``table0[(c ^ v) & 255] ^ (c >> 8)``)."""
+    if shift_bytes not in _crc32c_tables:
+        v = np.arange(256, dtype=np.uint32)
+        if shift_bytes == 0:
+            for _ in range(8):
+                v = (v >> 1) ^ ((v & 1) * np.uint32(_CRC32C_POLY))
+            _crc32c_tables[0] = v
+        else:
+            by = (v[None, :] << (8 * np.arange(4, dtype=np.uint32))[:, None]).astype(np.uint32)
+            _crc32c_tables[shift_bytes] = _crc_mul(_crc_shift(shift_bytes), by).astype(np.uint32)
+    return _crc32c_tables[shift_bytes]
+
+
+def crc32c(data) -> int:
+    """CRC-32C (Castagnoli, reflected polynomial 0x82F63B78, init and final XOR 0xFFFFFFFF) of ``data`` -- the
+    checksum of Zarr v3's ``crc32c`` codec and of its shard indexes.
+
+    The bytes are cut into segments of 64 bytes that are run through the byte table side by side (one numpy step per
+    byte position, over all segments at once); the segment registers are then combined pairwise, level by level,
+    with the GF(2) shift ``x^(8 * 64 * 2^level)`` (the linearity crc32_combine uses), and the tail of fewer than 64
+    bytes runs through the table last.  No Python loop runs per byte of the bulk."""
+    buf = np.frombuffer(memoryview(data).cast("B"), dtype=np.uint8)
+    n_seg = len(buf) // _CRC_SEGMENT
+    table = _crc32c_table(0)
+    reg = np.uint32(0xFFFFFFFF)
+    if n_seg:
+        levels = max(n_seg - 1, 0).bit_length()
+        # leading zero segments are free: with a zero register they leave it zero
+        segs = np.zeros((1 << levels, _CRC_SEGMENT), np.uint8)
+        segs[(1 << levels) - n_seg:] = buf[:n_seg * _CRC_SEGMENT].reshape(n_seg, _CRC_SEGMENT)
+        cols = np.ascontiguousarray(segs.T)
+        c = np.zeros(1 << levels, np.uint32)
+        c[(1 << levels) - n_seg] = reg
+        for col in cols:
+            c = table[(c ^ col) & 0xFF] ^ (c >> 8)
+        for level in range(levels):
+            t = _crc32c_table(_CRC_SEGMENT << level)
+            a, b = c[0::2], c[1::2]
+            c = t[0][a & 0xFF] ^ t[1][(a >> 8) & 0xFF] ^ t[2][(a >> 16) & 0xFF] ^ t[3][a >> 24] ^ b
+        reg = c[0]
+    reg = int(reg)
+    for v in buf[n_seg * _CRC_SEGMENT:].tolist():
+        reg = int(table[(reg ^ v) & 0xFF]) ^ (reg >> 8)
+    return reg ^ 0xFFFFFFFF
+
+
+def _check_crc32c(raw, where: str) -> memoryview:
+    """The payload of a chunk that ends in the crc32c codec's 4-byte little-endian CRC-32C; ``ValueError`` naming
+    ``where`` when the file is too short or the checksum does not match."""
+    raw = memoryview(raw)
+    if len(raw) < 4:
+        raise ValueError(f"{where}: shorter than its 4-byte CRC-32C")
+    if crc32c(raw[:-4]) != int.from_bytes(raw[-4:], "little"):
+        raise ValueError(f"{where}: CRC-32C mismatch")
+    return raw[:-4]
+
+
 class LazySource:
     """A (bands, h, w) or (h, w) array that can deliver whole bands into a caller's buffer."""
 
@@ -268,6 +365,7 @@ CHUNK_TABLE_DTYPE = np.dtype([("offset", "<i8"), ("length", "<i8"), ("band", "<i
                               ("header", "u1", 16)])
 assert CHUNK_TABLE_DTYPE.itemsize == 80
 CHUNK_MISSING, CHUNK_BLOSC, CHUNK_LZ4, CHUNK_ZSTD, CHUNK_ZLIB, CHUNK_GZIP = 0, 1, 2, 3, 4, 5  # enum xrs_chunk_codec
+CHUNK_CRC32C = 0x100  # flag: the file ends in a CRC-32C of its payload
 _BLOSC_INNER = {"lz4": 1, "lz4hc": 1, "zlib": 3, "zstd": 4}  # Blosc flags bits 5-7 of a store's cname
 _BLOSC_INNER_NAMES = {1: "LZ4", 3: "Zlib", 4: "Zstd"}
 _NUMCODECS_DEVICE = {"lz4": CHUNK_LZ4, "zstd": CHUNK_ZSTD, "zlib": CHUNK_ZLIB, "gzip": CHUNK_GZIP}
@@ -335,7 +433,119 @@ def _check_device_header(path: str, codec: int, head: bytes, size: int, chunk_by
                          f"{_BLOSC_INNER_NAMES[inner]}")
 
 
-class ZarrV2Source(LazySource):
+class _ZarrSource(LazySource):
+    """What Zarr v2 and v3 arrays share: the loops of :meth:`read_bands` and :meth:`device_read` over the chunk grid.
+    A subclass says where the bytes of one chunk are and how they are framed (:meth:`_locate`, :meth:`_payload`) and
+    sets ``path``, ``shape``, ``chunks`` (the unit of decoding), ``dtype``, ``device_codec``, ``_device_inner`` and
+    ``_fill`` (the value of a missing chunk)."""
+
+    _crc = False  # chunk files end in a CRC-32C of the bytes in front of it (Zarr v3's crc32c codec)
+
+    def _locate(self, idx) -> tuple[str, str, int, int] | None:  # pragma: no cover - interface
+        """(file, name for messages, offset, size) of chunk ``idx``'s bytes; ``None`` for a missing chunk."""
+        raise NotImplementedError
+
+    def _payload(self, raw, where: str) -> bytes:  # pragma: no cover - interface
+        """The decoded bytes of a chunk file ``raw``."""
+        raise NotImplementedError
+
+    @property
+    def device_decodable(self) -> bool:
+        """Whether :meth:`device_read` applies: the store's compressor is one ``xrs_zarr_decode`` decodes."""
+        return self.device_codec is not None
+
+    def device_fill_bits(self) -> int:
+        """The stored value of a missing chunk (what :meth:`_chunk` fills in), native byte order, as an integer."""
+        v = np.full(1, self._fill, dtype=self.dtype.newbyteorder("="))
+        return int.from_bytes(v.tobytes(), "little")
+
+    def device_read(self, b0: int, nb: int, segments, window, buffer=None):
+        """The chunk files behind bands ``b0 : b0 + nb`` of the (j0, j1, i0, i1) ``segments`` inside the row
+        ``window``, read as they are on disk into a page-locked byte buffer, followed by their chunk table
+        (:data:`CHUNK_TABLE_DTYPE`).  Only each file's header is checked here.  ``buffer`` (the previous
+        result's) is reused when it is large enough.  Returns ``(buffer, n_file_bytes, table, paths)``."""
+        from . import _dev
+
+        three_d = len(self.shape) == 3
+        cb = self.chunks[0] if three_d else 1
+        ch, cw = self.chunks[-2:]
+        chunk_bytes = int(np.prod(self.chunks)) * self.dtype.itemsize
+        tiles = set()
+        for (j0, j1, i0, i1) in segments:
+            j0, j1 = max(j0, window[0]), min(j1, window[1])
+            if j0 >= j1 or i0 >= i1:
+                continue
+            tiles.update((kj, ki) for kj in range(j0 // ch, -(-j1 // ch)) for ki in range(i0 // cw, -(-i1 // cw)))
+        keys = [(kb, kj, ki) for kb in range(b0 // cb, -(-(b0 + nb) // cb)) for (kj, ki) in sorted(tiles)]
+        locs = [self._locate((kb, kj, ki) if three_d else (kj, ki)) for (kb, kj, ki) in keys]
+        paths = [loc[1] if loc else self._missing_name((kb, kj, ki) if three_d else (kj, ki))
+                 for (kb, kj, ki), loc in zip(keys, locs)]
+        n_bytes = sum(loc[3] for loc in locs if loc)
+        table_at = -(-n_bytes // 8) * 8
+        need = table_at + len(keys) * CHUNK_TABLE_DTYPE.itemsize
+        if buffer is None or buffer.nbytes < need:
+            buffer = _dev.pinned_empty((max(need, 1 << 20) + (need >> 3),), np.uint8)  # an eighth to grow into
+        table = buffer[table_at:need].view(CHUNK_TABLE_DTYPE)
+        table[...] = 0
+        pos = 0
+        trailer = 4 if self._crc else 0
+        for k, ((kb, kj, ki), loc, p) in enumerate(zip(keys, locs, paths)):
+            t = table[k]
+            t["band"], t["row"], t["col"] = kb * cb, kj * ch, ki * cw
+            if loc is None:  # a missing chunk is all fill value
+                t["codec"] = CHUNK_MISSING
+                continue
+            file, _, offset, size = loc
+            with open(file, "rb") as fh:
+                fh.seek(offset)
+                got = fh.readinto(memoryview(buffer[pos:pos + size]))
+            if got != size:
+                raise ValueError(f"{p}: short read ({got} of {size} bytes)")
+            if size < trailer:
+                raise ValueError(f"{p}: shorter than its 4-byte CRC-32C")
+            n_head = {CHUNK_ZSTD: _ZSTD_HEADER_MAX, CHUNK_GZIP: _GZIP_MIN}.get(self.device_codec, 16)
+            head = buffer[pos:pos + min(size - trailer, n_head)].tobytes()  # of the payload: the trailer excluded
+            _check_device_header(p, self.device_codec, head, size - trailer, chunk_bytes, self._device_inner)
+            t["offset"], t["length"] = pos, size
+            t["codec"] = self.device_codec | (CHUNK_CRC32C if self._crc else 0)
+            t["header"][:min(len(head), 16)] = np.frombuffer(head[:16], np.uint8)
+            pos += size
+        return buffer, n_bytes, table, paths
+
+    def _missing_name(self, idx) -> str:  # pragma: no cover - interface
+        """Where chunk ``idx`` would be, for messages about a table that lists it as missing."""
+        raise NotImplementedError
+
+    def _chunk(self, idx):
+        loc = self._locate(idx)
+        if loc is None:  # a missing chunk is all fill value
+            return np.full(self.chunks, self._fill, dtype=self.dtype)
+        file, where, offset, size = loc
+        with open(file, "rb") as fh:
+            fh.seek(offset)
+            raw = fh.read(size)
+        if len(raw) != size:
+            raise ValueError(f"{where}: short read ({len(raw)} of {size} bytes)")
+        return np.frombuffer(self._payload(raw, where), dtype=self.dtype).reshape(self.chunks)
+
+    def read_bands(self, b0, nb, out):
+        three_d = len(self.shape) == 3
+        cb = self.chunks[0] if three_d else 1
+        ch, cw = self.chunks[-2:]
+        h, w = self.shape[-2:]
+        for kb in range(b0 // cb, -(-(b0 + nb) // cb)):
+            lo, hi = max(b0, kb * cb), min(b0 + nb, (kb + 1) * cb)
+            for kj in range(-(-h // ch)):
+                for ki in range(-(-w // cw)):
+                    block = self._chunk((kb, kj, ki) if three_d else (kj, ki))
+                    if not three_d:
+                        block = block[None]
+                    j0, i0 = kj * ch, ki * cw
+                    j1, i1 = min(h, j0 + ch), min(w, i0 + cw)
+                    out[lo - b0:hi - b0, j0:j1, i0:i1] = block[lo - kb * cb:hi - kb * cb, :j1 - j0, :i1 - i0]
+
+
+class ZarrV2Source(_ZarrSource):
     """One Zarr-v2 array of a directory store (2-D or 3-D, C order; uncompressed or with a codec of
     :func:`chunk_decoder`).  Blosc-LZ4 / LZ4HC / Zstd / Zlib (byte shuffle or none) and numcodecs ``lz4`` / ``zstd`` /
     ``zlib`` / ``gzip`` stores can also be read for the device (:meth:`device_read`): the band pipeline then decodes
@@ -361,93 +571,286 @@ class ZarrV2Source(LazySource):
         self.chunks = tuple(int(n) for n in meta["chunks"])
         self.dtype = np.dtype(meta["dtype"])
         self.fill = meta.get("fill_value")
+        self._fill = _fill_value(self.fill, self.dtype)
         self.sep = meta.get("dimension_separator", ".")
         attrs_path = os.path.join(path, ".zattrs")
         self.attrs = json.load(open(attrs_path)) if os.path.isfile(attrs_path) else {}
         self.device_codec = _device_codec(meta.get("compressor"))
         self._device_inner = _BLOSC_INNER.get((meta.get("compressor") or {}).get("cname"), 1)
 
-    @property
-    def device_decodable(self) -> bool:
-        """Whether :meth:`device_read` applies: the store's compressor is one ``xrs_zarr_decode`` decodes."""
-        return self.device_codec is not None
-
-    def device_fill_bits(self) -> int:
-        """The stored value of a missing chunk (what :meth:`_chunk` fills in), native byte order, as an integer."""
-        v = np.full(1, _fill_value(self.fill, self.dtype), dtype=self.dtype.newbyteorder("="))
-        return int.from_bytes(v.tobytes(), "little")
-
-    def device_read(self, b0: int, nb: int, segments, window, buffer=None):
-        """The chunk files behind bands ``b0 : b0 + nb`` of the (j0, j1, i0, i1) ``segments`` inside the row
-        ``window``, read as they are on disk into a page-locked byte buffer, followed by their chunk table
-        (:data:`CHUNK_TABLE_DTYPE`).  Only each file's header is checked here.  ``buffer`` (the previous
-        result's) is reused when it is large enough.  Returns ``(buffer, n_file_bytes, table, paths)``."""
-        from . import _dev
-
-        three_d = len(self.shape) == 3
-        cb = self.chunks[0] if three_d else 1
-        ch, cw = self.chunks[-2:]
-        chunk_bytes = int(np.prod(self.chunks)) * self.dtype.itemsize
-        tiles = set()
-        for (j0, j1, i0, i1) in segments:
-            j0, j1 = max(j0, window[0]), min(j1, window[1])
-            if j0 >= j1 or i0 >= i1:
-                continue
-            tiles.update((kj, ki) for kj in range(j0 // ch, -(-j1 // ch)) for ki in range(i0 // cw, -(-i1 // cw)))
-        keys = [(kb, kj, ki) for kb in range(b0 // cb, -(-(b0 + nb) // cb)) for (kj, ki) in sorted(tiles)]
-        paths = [os.path.join(self.path, self.sep.join(str(i) for i in ((kb, kj, ki) if three_d else (kj, ki))))
-                 for (kb, kj, ki) in keys]
-        sizes = [os.path.getsize(p) if os.path.isfile(p) else -1 for p in paths]
-        n_bytes = sum(max(s, 0) for s in sizes)
-        table_at = -(-n_bytes // 8) * 8
-        need = table_at + len(keys) * CHUNK_TABLE_DTYPE.itemsize
-        if buffer is None or buffer.nbytes < need:
-            buffer = _dev.pinned_empty((max(need, 1 << 20) + (need >> 3),), np.uint8)  # an eighth to grow into
-        table = buffer[table_at:need].view(CHUNK_TABLE_DTYPE)
-        table[...] = 0
-        pos = 0
-        for k, ((kb, kj, ki), p, size) in enumerate(zip(keys, paths, sizes)):
-            t = table[k]
-            t["band"], t["row"], t["col"] = kb * cb, kj * ch, ki * cw
-            if size < 0:  # a missing chunk is all fill value
-                t["codec"] = CHUNK_MISSING
-                continue
-            with open(p, "rb") as fh:
-                got = fh.readinto(memoryview(buffer[pos:pos + size]))
-            if got != size:
-                raise ValueError(f"{p}: short read ({got} of {size} bytes)")
-            n_head = {CHUNK_ZSTD: _ZSTD_HEADER_MAX, CHUNK_GZIP: _GZIP_MIN}.get(self.device_codec, 16)
-            head = buffer[pos:pos + min(size, n_head)].tobytes()
-            _check_device_header(p, self.device_codec, head, size, chunk_bytes, self._device_inner)
-            t["offset"], t["length"], t["codec"] = pos, size, self.device_codec
-            t["header"][:min(len(head), 16)] = np.frombuffer(head[:16], np.uint8)
-            pos += size
-        return buffer, n_bytes, table, paths
-
-    def _chunk(self, idx):
+    def _locate(self, idx):
         p = os.path.join(self.path, self.sep.join(str(i) for i in idx))
-        if not os.path.isfile(p):  # a missing chunk is all fill value
-            return np.full(self.chunks, _fill_value(self.fill, self.dtype), dtype=self.dtype)
-        if self._decode is None:
-            return np.fromfile(p, dtype=self.dtype).reshape(self.chunks)
-        with open(p, "rb") as fh:
-            return np.frombuffer(self._decode(fh.read()), dtype=self.dtype).reshape(self.chunks)
+        return (p, p, 0, os.path.getsize(p)) if os.path.isfile(p) else None
 
-    def read_bands(self, b0, nb, out):
-        three_d = len(self.shape) == 3
-        cb = self.chunks[0] if three_d else 1
-        ch, cw = self.chunks[-2:]
-        h, w = self.shape[-2:]
-        for kb in range(b0 // cb, -(-(b0 + nb) // cb)):
-            lo, hi = max(b0, kb * cb), min(b0 + nb, (kb + 1) * cb)
-            for kj in range(-(-h // ch)):
-                for ki in range(-(-w // cw)):
-                    block = self._chunk((kb, kj, ki) if three_d else (kj, ki))
-                    if not three_d:
-                        block = block[None]
-                    j0, i0 = kj * ch, ki * cw
-                    j1, i1 = min(h, j0 + ch), min(w, i0 + cw)
-                    out[lo - b0:hi - b0, j0:j1, i0:i1] = block[lo - kb * cb:hi - kb * cb, :j1 - j0, :i1 - i0]
+    def _missing_name(self, idx):
+        return os.path.join(self.path, self.sep.join(str(i) for i in idx))
+
+    def _payload(self, raw, where):
+        return raw if self._decode is None else self._decode(raw)
+
+
+_V3_TYPES = ("bool", "int8", "int16", "int32", "int64", "uint8", "uint16", "uint32", "uint64", "float16", "float32",
+             "float64", "complex64", "complex128")
+_V3_SHUFFLE = {"noshuffle": 0, "shuffle": 1}
+_MISSING = 2 ** 64 - 1  # offset and size of an inner chunk a shard does not hold
+
+
+def _v3_codec(entry) -> tuple[str, dict]:
+    """(name, configuration) of one entry of a v3 ``codecs`` list (a bare name stands for no configuration)."""
+    if isinstance(entry, str):
+        return entry, {}
+    return entry.get("name"), dict(entry.get("configuration") or {})
+
+
+def _v3_compressor(name: str, conf: dict) -> dict:
+    """The numcodecs configuration (what :func:`chunk_decoder` / :func:`_device_codec` take) of a v3 bytes -> bytes
+    compressor."""
+    if name == "zstd":
+        return {"id": "zstd", "level": conf.get("level", 0)}
+    if name == "gzip":
+        return {"id": "gzip", "level": conf.get("level", 5)}
+    if name == "blosc":
+        shuffle = conf.get("shuffle", "noshuffle")
+        if shuffle == "bitshuffle":
+            raise NotImplementedError("bit-shuffled Blosc frames need the zarr / blosc packages, which this build "
+                                      "does not have")
+        if shuffle not in _V3_SHUFFLE:
+            raise ValueError(f"unknown Blosc shuffle {shuffle!r}")
+        return {"id": "blosc", "cname": conf.get("cname", "lz4"), "clevel": conf.get("clevel", 5),
+                "shuffle": _V3_SHUFFLE[shuffle], "typesize": conf.get("typesize"), "blocksize": conf.get("blocksize", 0)}
+    if name.startswith("numcodecs.") and name[10:] in ("zlib", "gzip", "bz2", "lzma", "zstd", "lz4", "blosc"):
+        return dict(conf, id=name[10:])
+    if name in ("bitshuffle", "numcodecs.bitshuffle"):
+        raise NotImplementedError("bit-shuffled chunks need the zarr / numcodecs packages, which this build does not "
+                                  "have; open the store with xarray and pass the arrays instead")
+    raise NotImplementedError(f"Zarr v3 codec {name!r} needs the zarr package, which this build does not have; open "
+                              "the store with xarray and pass the arrays instead")
+
+
+def _v3_chain(codecs, data_type: str, ndim: int, nested: bool = False) -> dict:
+    """The rules of a v3 codec chain this build reads: an identity ``transpose`` at most, exactly one array -> bytes
+    codec (``bytes``, or ``sharding_indexed`` when not ``nested``), then at most one compressor, then ``crc32c``.
+    Returns ``{"endian", "compressor", "crc", "sharding"}``."""
+    out = {"endian": None, "compressor": None, "crc": False, "sharding": None}
+    stage = 0  # 0 before the array -> bytes codec, 1 after it, 2 after the compressor, 3 after crc32c
+    for entry in codecs or ():
+        name, conf = _v3_codec(entry)
+        if name == "transpose" and stage == 0:
+            if list(conf.get("order", ())) != list(range(ndim)):
+                raise NotImplementedError(f"a transpose codec of order {conf.get('order')} (only the identity order "
+                                          "is read)")
+        elif name in ("bytes", "sharding_indexed") and stage == 0:
+            if name == "sharding_indexed":
+                if nested:
+                    raise NotImplementedError("nested sharding_indexed codecs are not read")
+                out["sharding"] = conf
+            else:
+                endian = conf.get("endian")
+                if endian is None and np.dtype(data_type).itemsize > 1:
+                    raise ValueError(f"the bytes codec of a {data_type} array needs an endian")
+                if endian not in (None, "little", "big"):
+                    raise ValueError(f"unknown endian {endian!r} of the bytes codec")
+                out["endian"] = endian
+            stage = 1
+        elif name == "crc32c" and stage in (1, 2):
+            out["crc"] = True
+            stage = 3
+        elif stage == 1 and name not in ("transpose", "bytes", "sharding_indexed", "crc32c", "vlen-utf8",
+                                         "vlen-bytes"):
+            out["compressor"] = _v3_compressor(name, conf)
+            stage = 2
+        elif stage == 0 and name not in ("bytes", "sharding_indexed", "transpose"):
+            raise NotImplementedError(f"array -> array codec {name!r} (only an identity transpose is read)")
+        else:
+            raise NotImplementedError(f"codec {name!r} at this place of the chain (read: [transpose], bytes or "
+                                      "sharding_indexed, [one compressor], [crc32c])")
+    if stage == 0:
+        raise ValueError("the codec chain has no array -> bytes codec")
+    if out["sharding"] is not None and stage != 1:
+        raise NotImplementedError("codecs after sharding_indexed are not read")
+    return out
+
+
+def _v3_fill(fill, dtype: np.dtype):
+    """The value of a v3 ``fill_value``: a number, ``"NaN"`` / ``"Infinity"`` / ``"-Infinity"``, or ``"0x..."`` -- a
+    float's raw bits."""
+    if isinstance(fill, str) and fill.startswith("0x"):
+        bits = np.array([int(fill, 16)], dtype=f"u{dtype.itemsize}")
+        return bits.view(dtype.newbyteorder("="))[0]
+    if isinstance(fill, str):
+        special = {"NaN": np.nan, "Infinity": np.inf, "-Infinity": -np.inf}
+        if fill not in special:
+            raise ValueError(f"unknown fill_value {fill!r}")
+        return dtype.newbyteorder("=").type(special[fill])
+    if isinstance(fill, list) and dtype.kind == "c":
+        return dtype.newbyteorder("=").type(complex(_v3_fill(fill[0], np.dtype("f8")), _v3_fill(fill[1], np.dtype("f8"))))
+    return dtype.newbyteorder("=").type(0 if fill is None else fill)
+
+
+def _v3_key(encoding, idx) -> str:
+    """The key of chunk ``idx`` under a v3 ``chunk_key_encoding`` (``default``: ``c/1/2`` or ``c.1.2``, ``c`` for a
+    0-D array; ``v2``: ``1.2``, ``0`` for a 0-D array), as a relative path."""
+    name, conf = _v3_codec(encoding or {"name": "default"})
+    if name == "default":
+        sep = conf.get("separator", "/")
+        key = sep.join(["c"] + [str(i) for i in idx])
+    elif name == "v2":
+        sep = conf.get("separator", ".")
+        key = sep.join(str(i) for i in idx) if idx else "0"
+    else:
+        raise NotImplementedError(f"chunk_key_encoding {name!r}")
+    if sep not in ("/", "."):
+        raise ValueError(f"chunk key separator {sep!r}")
+    return key.replace("/", os.sep)
+
+
+def _v3_meta(path: str) -> dict:
+    meta = json.load(open(os.path.join(path, "zarr.json")))
+    if meta.get("zarr_format") != 3 or meta.get("node_type") != "array":
+        raise ValueError(f"{path}: not a Zarr v3 array")
+    return meta
+
+
+def v3_dimension_names(meta: dict) -> list:
+    """``dimension_names``, else ``attributes._ARRAY_DIMENSIONS``, else ``dim_k``; a null name becomes ``dim_k``."""
+    names = meta.get("dimension_names") or (meta.get("attributes") or {}).get("_ARRAY_DIMENSIONS")
+    ndim = len(meta["shape"])
+    if not names or len(names) != ndim:
+        names = [None] * ndim
+    return [n if n is not None else f"dim_{k}" for k, n in enumerate(names)]
+
+
+class _ZarrV3Array(_ZarrSource):
+    """A Zarr v3 array of a directory store of any rank (:class:`ZarrV3Source` is the 2-D / 3-D lazy source).
+    Written from the Zarr v3 core specification and its ``sharding_indexed`` and ``crc32c`` codec specifications.
+
+    * ``zarr.json``: ``shape``, a ``regular`` chunk grid, a numeric ``data_type``, ``fill_value``,
+      ``chunk_key_encoding`` (``default`` or ``v2``), ``attributes``, ``dimension_names``; no storage transformers.
+    * Codecs (:func:`_v3_chain`): [identity ``transpose``], ``bytes`` (its ``endian`` sets the byte order), at most one
+      compressor (``zstd``, ``gzip``, ``blosc`` or ``numcodecs.<id>`` of :func:`chunk_decoder`), [``crc32c``].
+    * ``sharding_indexed`` (not nested): a shard file holds inner chunks (``chunk_shape``, inner ``codecs``) and an
+      index of one little-endian uint64 (offset, nbytes) pair per inner chunk in C order, (2^64 - 1, 2^64 - 1) for
+      an absent one, at the ``end`` (default) or ``start`` of the file and optionally followed by its CRC-32C.  The
+      index of each shard is read once, with one ranged read, and kept; inner chunks are read with ranged reads.
+      A missing shard file is all fill value.
+
+    ``chunks`` is the unit of decoding: the inner chunk of a sharded array."""
+
+    def __init__(self, path: str):
+        meta = _v3_meta(path)
+        self.path = path
+        self.shape = tuple(int(n) for n in meta["shape"])
+        grid_name, grid = _v3_codec(meta.get("chunk_grid") or {})
+        if grid_name != "regular":
+            raise NotImplementedError(f"{path}: chunk grid {grid_name!r} (only regular grids are read)")
+        outer = tuple(int(n) for n in grid["chunk_shape"])
+        data_type = meta.get("data_type")
+        if data_type not in _V3_TYPES:
+            raise NotImplementedError(f"{path}: Zarr v3 data type {data_type!r} is not read (numeric types only)")
+        if meta.get("storage_transformers"):
+            raise NotImplementedError(f"{path}: storage transformers are not read")
+        self._encoding = meta.get("chunk_key_encoding")
+        self.attrs = dict(meta.get("attributes") or {})
+        self.dimension_names = v3_dimension_names(meta)
+        try:
+            _v3_key(self._encoding, (0,) * len(self.shape))
+            chain = _v3_chain(meta.get("codecs"), data_type, len(self.shape))
+            self._shard = None
+            if chain["sharding"] is not None:
+                conf = chain["sharding"]
+                inner = tuple(int(n) for n in conf["chunk_shape"])
+                if len(inner) != len(outer) or any(o % i for o, i in zip(outer, inner)):
+                    raise ValueError(f"inner chunks {inner} do not tile the shard {outer}")
+                index = _v3_chain(conf.get("index_codecs"), "uint64", len(outer) + 1, nested=True)
+                if index["compressor"] is not None or index["endian"] not in ("little", None):
+                    raise NotImplementedError("a shard index other than little-endian bytes [+ crc32c]")
+                location = conf.get("index_location", "end")
+                if location not in ("start", "end"):
+                    raise ValueError(f"unknown index_location {location!r}")
+                per = tuple(o // i for o, i in zip(outer, inner))
+                n_inner = int(np.prod(per, dtype=np.int64))
+                self._shard = {"per": per, "n": n_inner, "start": location == "start",
+                               "index_bytes": 16 * n_inner + (4 if index["crc"] else 0), "index_crc": index["crc"]}
+                self._indexes: dict = {}
+                chain = _v3_chain(conf.get("codecs"), data_type, len(outer), nested=True)
+                self.chunks = inner
+            else:
+                self.chunks = outer
+            self._decode = chunk_decoder(chain["compressor"])
+            dtype = np.dtype(data_type)
+            self.dtype = dtype.newbyteorder(">" if chain["endian"] == "big" else "<") if dtype.itemsize > 1 else dtype
+            self._fill = _v3_fill(meta.get("fill_value"), self.dtype)
+        except (NotImplementedError, ValueError) as e:
+            raise type(e)(f"{path}: {e}") from None
+        self._crc = chain["crc"]
+        self.device_codec = _device_codec(chain["compressor"])
+        self._device_inner = _BLOSC_INNER.get((chain["compressor"] or {}).get("cname"), 1)
+
+    def _key_path(self, idx) -> str:
+        return os.path.join(self.path, _v3_key(self._encoding, idx))
+
+    def _missing_name(self, idx):
+        if self._shard is None:
+            return self._key_path(idx)
+        shard = tuple(i // p for i, p in zip(idx, self._shard["per"]))
+        return f"{self._key_path(shard)} (inner chunk {tuple(int(i) for i in idx)})"
+
+    def _index(self, shard) -> tuple[str, np.ndarray | None]:
+        """(file, (n, 2) uint64 index) of a shard, ``None`` for a missing shard file; checked once and cached."""
+        if shard not in self._indexes:
+            p = self._key_path(shard)
+            if not os.path.isfile(p):
+                self._indexes[shard] = (p, None)
+                return self._indexes[shard]
+            sh = self._shard
+            size = os.path.getsize(p)
+            if size < sh["index_bytes"]:
+                raise ValueError(f"{p}: a shard of {size} bytes cannot hold its {sh['index_bytes']}-byte index")
+            with open(p, "rb") as fh:
+                fh.seek(0 if sh["start"] else size - sh["index_bytes"])
+                raw = fh.read(sh["index_bytes"])
+            if len(raw) != sh["index_bytes"]:
+                raise ValueError(f"{p}: short read of the shard index")
+            if sh["index_crc"]:
+                raw = _check_crc32c(raw, f"{p}: shard index")
+            index = np.frombuffer(raw, dtype="<u8").reshape(sh["n"], 2).astype(np.uint64)
+            present = ~((index[:, 0] == _MISSING) & (index[:, 1] == _MISSING))
+            off, nbytes = index[present, 0], index[present, 1]
+            if np.any(off > size) or np.any(nbytes > np.uint64(size) - off):
+                raise ValueError(f"{p}: a shard index entry points outside the file of {size} bytes")
+            self._indexes[shard] = (p, index)
+        return self._indexes[shard]
+
+    def _locate(self, idx):
+        if self._shard is None:
+            p = self._key_path(idx)
+            return (p, p, 0, os.path.getsize(p)) if os.path.isfile(p) else None
+        per = self._shard["per"]
+        p, index = self._index(tuple(i // q for i, q in zip(idx, per)))
+        if index is None:
+            return None
+        k = int(np.ravel_multi_index(tuple(i % q for i, q in zip(idx, per)), per)) if per else 0
+        off, nbytes = int(index[k, 0]), int(index[k, 1])
+        if off == _MISSING and nbytes == _MISSING:
+            return None
+        return p, f"{p} (inner chunk {tuple(int(i) for i in idx)})", off, nbytes
+
+    def _payload(self, raw, where):
+        if self._crc:
+            raw = _check_crc32c(raw, where)
+        return raw if self._decode is None else self._decode(bytes(raw))
+
+
+class ZarrV3Source(_ZarrV3Array):
+    """One 2-D or 3-D Zarr v3 array of a directory store (:class:`_ZarrV3Array`), sharded or not.  Chunks compressed
+    with a codec ``xrs_zarr_decode`` decodes (``zstd``, ``gzip``, ``blosc`` with an LZ4 / Zstd / Zlib inner codec and
+    byte shuffle or none, and their ``numcodecs.*`` twins) can be read for the device (:meth:`device_read`); a
+    ``crc32c`` trailer is then checked there too."""
+
+    def __init__(self, path: str):
+        super().__init__(path)
+        if len(self.shape) not in (2, 3):
+            raise ValueError(f"{self.path}: expected a 2-D or 3-D array, got shape {self.shape}")
 
 
 def cf_decoded_dtype(dtype: np.dtype, attrs: Mapping) -> np.dtype | None:
@@ -557,8 +960,16 @@ def _fill_value(fill, dtype: np.dtype):
 
 
 def _read_small_array(arr_dir: str, meta: dict) -> np.ndarray:
-    """A 0-D or 1-D Zarr-v2 array (``spatial_ref``, axis coordinates), chunks decoded like those of
-    :class:`ZarrV2Source`; missing chunks hold the fill value."""
+    """A 0-D or 1-D Zarr array (``spatial_ref``, axis coordinates), chunks decoded like those of
+    :class:`ZarrV2Source` / :class:`ZarrV3Source` (``meta``: its ``.zarray`` or ``zarr.json``); missing chunks hold the
+    fill value."""
+    if meta.get("zarr_format") == 3:
+        arr = _ZarrV3Array(arr_dir)
+        if not arr.shape:
+            return arr._chunk(())[()].copy()
+        n, c = arr.shape[0], arr.chunks[0]
+        parts = [arr._chunk((k,))[:min(c, n - k * c)] for k in range(-(-n // c))]
+        return np.concatenate(parts) if n else np.empty(0, arr.dtype)
     if meta.get("filters"):
         raise NotImplementedError(f"{arr_dir}: filtered Zarr arrays need the zarr package, which this build does not "
                                   "have; open the store with xarray and pass the arrays instead")
@@ -589,7 +1000,17 @@ def open_zarr_dataset(path: str, coord_names=("lon", "lat", "x", "y", "longitude
     now, every other 2-D / 3-D array becomes a :class:`LazyDataArray`.  By default values are delivered
     as stored (what ``xarray.open_zarr(..., mask_and_scale=False)`` gives): ``scale_factor`` /
     ``add_offset`` / ``_FillValue`` attributes are passed through, not applied.  ``mask_and_scale=True``
-    decodes the lazy variables that carry such attributes on the reader thread (:class:`DecodedSource`)."""
+    decodes the lazy variables that carry such attributes on the reader thread (:class:`DecodedSource`).
+
+    A Zarr v3 store (a root ``zarr.json`` of ``node_type`` group) is read the same way, each child array from its
+    own ``zarr.json`` (:class:`ZarrV3Source`); the group attributes come from the root, and consolidated metadata is
+    not used for reading."""
+    root = os.path.join(path, "zarr.json")
+    if os.path.isfile(root):
+        group = json.load(open(root))
+        if group.get("zarr_format") != 3 or group.get("node_type") != "group":
+            raise ValueError(f"{path}: not a Zarr v3 group")
+        return _open_zarr_v3(path, group, coord_names, mask_and_scale)
     data_vars, coords = {}, {}
     for item in sorted(os.listdir(path)):
         arr_dir = os.path.join(path, item)
@@ -610,6 +1031,32 @@ def open_zarr_dataset(path: str, coord_names=("lon", "lat", "x", "y", "longitude
                 data_vars[item] = _lazy_variable(src, dims, attrs, item, mask_and_scale)
     group_attrs = os.path.join(path, ".zattrs")
     return Dataset(data_vars=data_vars, coords=coords, attrs=json.load(open(group_attrs)) if os.path.isfile(group_attrs) else {})
+
+
+def _open_zarr_v3(path: str, group: dict, coord_names, mask_and_scale: bool) -> Dataset:
+    """:func:`open_zarr_dataset` for a Zarr v3 group: its child arrays, by the same rules as a v2 store."""
+    data_vars, coords = {}, {}
+    for item in sorted(os.listdir(path)):
+        arr_dir = os.path.join(path, item)
+        meta_path = os.path.join(arr_dir, "zarr.json")
+        if not os.path.isfile(meta_path):
+            continue
+        meta = json.load(open(meta_path))
+        if meta.get("zarr_format") != 3 or meta.get("node_type") != "array":
+            continue
+        dims = v3_dimension_names(meta)
+        attrs = dict(meta.get("attributes") or {})
+        attrs.pop("_ARRAY_DIMENSIONS", None)
+        shape = tuple(meta["shape"])
+        if len(shape) <= 1:
+            coords[item] = DataArray(_read_small_array(arr_dir, meta), dims=dims, attrs=attrs, name=item)
+        else:
+            src = ZarrV3Source(arr_dir)
+            if item in coord_names:
+                coords[item] = DataArray(src.read_all(), dims=dims, attrs=attrs, name=item)
+            else:
+                data_vars[item] = _lazy_variable(src, dims, attrs, item, mask_and_scale)
+    return Dataset(data_vars=data_vars, coords=coords, attrs=dict(group.get("attributes") or {}))
 
 
 def open_netcdf_dataset(path: str, coord_names=("lon", "lat", "x", "y", "longitude", "latitude",
